@@ -13,6 +13,9 @@ renders the same samples, so every step — at every N — must produce the same
 
 The reference is a Rust program and there is no Rust toolchain in this image, so the reference arm times the oracle —
 the C++ f64 restatement of the reference's algorithm (oracle/) — on all host cores, on a bounded sample of the same job.
+
+`--dump-outputs DIR` writes what the last timed step computed (see dump_outputs) as DIR/<name>.npy.  The job is fixed
+by the arguments and seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -141,6 +144,28 @@ def cpu_reference_run(wl, spp, steps, warmup, threads=0):
     return total[0] / secs / 1e6, 1e3 * secs / steps, cores, per_path
 
 
+DUMP_SAMPLE_PIXELS = 1 << 20  # 44 B per sampled pixel in the three files: 44 MB, under the 64 MB a dump may take
+
+
+def dump_outputs(out_dir, rgb, accum):
+    """Writes what the timed path hands its caller (distributed.render_sharded on rank 0) as float .npy files:
+    rgb.npy, the tonemapped 8-bit image as float32, and accum.npy, the radiance sums per pixel and channel as float64
+    (the int64 fixed-point sums times 2^-32: exact while a sum stays below 2^21).  Both are [H, W, 3] with row 0 at the
+    bottom.  An image of more than DUMP_SAMPLE_PIXELS pixels is reduced to the same fixed, seeded sample of pixels in both
+    files ([n, 3]), and pixel.npy holds the row-major index of each sampled pixel."""
+    from mu_lambda_raytracer_b200 import abi
+    H, W = rgb.shape[:2]
+    out = {"rgb": rgb.cpu().numpy().astype(np.float32),
+           "accum": accum.cpu().numpy().astype(np.float64) / abi.RT_ACCUM_FIXED_ONE}
+    if H * W > DUMP_SAMPLE_PIXELS:
+        pixel = np.sort(np.random.default_rng(SEED).choice(H * W, DUMP_SAMPLE_PIXELS, replace=False))
+        out = {name: a.reshape(H * W, 3)[pixel] for name, a in out.items()}
+        out["pixel"] = pixel.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_name(wl):
     return f"{'C5' if wl['width'] == 3840 else 'C4'} {wl['world']} {wl['width']}x{wl['height']} seed {SEED} max_depth {MAX_DEPTH}"
 
@@ -243,6 +268,8 @@ def run_b200(args, wl):
     ms_total = float(t.item())
     value = paths_per_step * args.steps / (ms_total / 1e3) / 1e6
     checksum = int(rgb.sum().item()) if rank == 0 else 0
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, rgb, accum)
 
     # ---- this rank's render region alone (CUDA events recorded by the library on the launching stream around the kernels of
     # the pipeline; no flush / reduce / tonemap): the numerator of the roofline figure
@@ -389,7 +416,10 @@ def main():
     ap.add_argument("--multi-steps", type=int, default=2, help="N > 1: timed steps of the one-process rt_render_multi leg (0 = skip)")
     ap.add_argument("--cpu-spp", type=int, default=128, help="spp of the bounded CPU-baseline sample (0 = skip)")
     ap.add_argument("--ref-spp", type=int, default=32, help="spp per step of --impl reference")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS["c5" if args.c5 else "c4"]
     if args.impl == "reference":
         return run_reference(args, wl)

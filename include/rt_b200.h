@@ -272,6 +272,39 @@ int rt_accum_fixed_to_float_device(const uint64_t* d_accum_fixed, float* d_accum
                                    void* stream);
 
 /*
+ * EXTENSION (no counterpart in the reference): per-pixel second moments and noise-threshold adaptive sampling.
+ *
+ * Second moments are kept beside the radiance sums as unsigned 64-bit fixed-point sums of the SQUARED samples: every
+ * sample q of the accumulation (in RT_ACCUM_FIXED_ONE units) adds (min(q, 2^44))^2 >> 40, i.e. radiance^2 in units of
+ * 1 / RT_MOMENT2_FIXED_ONE, exactly.  A sample above 4096 is capped in the square; the sum holds 2^16 such extremes.
+ * Both entry points run on the persistent pipeline only (RT_ERR_UNSUPPORTED for another pipeline).
+ *
+ * rt_render_moments_fixed_device: rt_render_accumulate_fixed_device plus d_moment2_fixed (3*W*H uint64 on the scene's
+ * device, ADDED to).  Sums of disjoint sample ranges add up exactly, so it composes with sample slices.
+ *
+ * rt_render_adaptive: samples every pixel until its noise is below a threshold, at most params->samples_per_pixel (the
+ * cap; sample_begin and sample_count must be 0).  Round 0 renders samples [0, min_samples) of every pixel (min_samples
+ * >= 2); each later round doubles the count of the pixels still active, the last capped at the maximum, so a pixel's
+ * count n is one of min_samples * 2^k or the cap, and its sums equal those of a uniform n-spp render bit for bit.  A pixel
+ * stops when n reaches the cap or when every channel, with mean mu, sample variance s^2 and standard error se =
+ * sqrt(s^2 / n), has se / (2 sqrt(max(mu, 2^-16))) <= noise_threshold (the error after the gamma-2 tonemap) or
+ * mu - 3 se >= 1 (saturated).  Host buffers, each optional: rgb (3*W*H, every pixel tonemapped with its own count; row 0
+ * at the bottom), samples (W*H counts), accum_fixed and moment2_fixed (3*W*H sums).  cb as in rt_render, paced by rounds.
+ * stats->paths is the number of paths traced (the sum of the counts).
+ */
+#define RT_MOMENT2_FIXED_ONE 16777216.0
+typedef struct RtAdaptive {
+    double noise_threshold; /* >= 0; with 0 only pixels with a zero variance estimate (or saturated) stop early */
+    int32_t min_samples;    /* >= 2 and <= samples_per_pixel */
+    int32_t reserved;
+} RtAdaptive;
+int rt_render_moments_fixed_device(const RtScene* scene, const RtCamera* cam, const RtParams* params, uint64_t* d_accum_fixed,
+                                   uint64_t* d_moment2_fixed, void* stream, RtStats* stats);
+int rt_render_adaptive(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* adaptive,
+                       int32_t* rgb, int32_t* samples, uint64_t* accum_fixed, uint64_t* moment2_fixed, RtProgressFn cb,
+                       void* user, RtStats* stats);
+
+/*
  * rt_render over several GPUs of one process (the reference's row-parallel rayon loop, raytrace.rs:176-185, becomes
  * sample slices): scenes[g] is the same description created on a distinct device; device g renders every pixel for
  * the g-th slice of the sample range (rt_sample_slice), the float accumulation buffers are summed onto scenes[0]'s

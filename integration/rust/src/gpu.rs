@@ -134,6 +134,15 @@ pub struct RtStats {
     pub bvh_layout_used: i32,
     pub reserved: i32,
 }
+/// EXTENSION: noise-threshold adaptive sampling (rt_render_adaptive)
+#[repr(C)]
+#[derive(Default)]
+pub struct RtAdaptive {
+    pub noise_threshold: f64,
+    pub min_samples: i32,
+    pub reserved: i32,
+}
+pub const RT_MOMENT2_FIXED_ONE: f64 = 16777216.0;
 pub enum RtScene {}
 /// Called once per image row j = 0 .. total-1, in increasing order, on the calling thread (include/rt_b200.h).
 pub type RtProgressFn = Option<extern "C" fn(row: c_int, total: c_int, user: *mut c_void)>;
@@ -150,6 +159,11 @@ extern "C" {
                      cb: RtProgressFn, user: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_render_multi(scenes: *const *mut RtScene, n_scenes: i32, cam: *const RtCamera, params: *const RtParams, accum_rgb: *mut f32,
                            rgb: *mut i32, cb: RtProgressFn, user: *mut c_void, stats: *mut RtStats) -> c_int;
+    pub fn rt_render_moments_fixed_device(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, d_accum_fixed: *mut u64,
+                                          d_moment2_fixed: *mut u64, stream: *mut c_void, stats: *mut RtStats) -> c_int;
+    pub fn rt_render_adaptive(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive, rgb: *mut i32,
+                              samples: *mut i32, accum_fixed: *mut u64, moment2_fixed: *mut u64, cb: RtProgressFn, user: *mut c_void,
+                              stats: *mut RtStats) -> c_int;
     pub fn rt_world_build(name: *const c_char, seed: u64, earth_rgb: *const u8, earth_w: i32, earth_h: i32, out: *mut *mut RtSceneDesc,
                           n_draws: *mut u64) -> c_int;
     pub fn rt_scene_desc_free(desc: *mut RtSceneDesc);

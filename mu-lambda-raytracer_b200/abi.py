@@ -91,6 +91,10 @@ class RtPeaks(C.Structure):
                 ("l2_read_gbs", C.c_double), ("sm_clock_mhz", C.c_double), ("sm_count", C.c_int32), ("reserved", C.c_int32)]
 
 
+class RtAdaptive(C.Structure):  # EXTENSION: noise-threshold adaptive sampling (rt_render_adaptive)
+    _fields_ = [("noise_threshold", C.c_double), ("min_samples", C.c_int32), ("reserved", C.c_int32)]
+
+
 class RtWorldInfo(C.Structure):
     _fields_ = [("lookfrom", C.c_double * 3), ("lookat", C.c_double * 3), ("vfov_deg", C.c_double),
                 ("background_kind", C.c_int32), ("needs_earthmap", C.c_int32), ("uses_rng", C.c_int32)]
@@ -119,6 +123,10 @@ PROTOTYPES = {
     "rt_tonemap_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int, C.c_void_p]),
     "rt_render_accumulate_fixed_device": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.c_void_p,
                                                     C.c_void_p, C.POINTER(RtStats)]),
+    "rt_render_moments_fixed_device": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.POINTER(RtStats)]),
+    "rt_render_adaptive": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
     "rt_tonemap_fixed_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int, C.c_void_p]),
     "rt_accum_fixed_to_float_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rt_release_cached_memory": (None, []),
@@ -138,6 +146,7 @@ PROTOTYPES = {
 }
 
 RT_ACCUM_FIXED_ONE = 4294967296.0
+RT_MOMENT2_FIXED_ONE = 16777216.0
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # RT_B200_LIB: another build of the same library (A/B measurements of compile-time choices); never a different implementation

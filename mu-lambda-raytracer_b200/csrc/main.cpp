@@ -10,7 +10,9 @@
 // reference would `unwrap()` into a panic exit with 101 (Rust's panic exit code).
 // Additions that do not exist in the reference: --gpus N (devices of this box to shard over), --pipeline NAME,
 // --earthmap FILE (decoded RGB8 as binary PPM; default $RT_EARTHMAP, ./earthmap.ppm, then the shipped asset),
-// --stats (one JSON line with paths, rays, device ms on stderr).
+// --stats (one JSON line with paths, rays, device ms on stderr), --noise_threshold T with --min_samples N (16): adaptive
+// sampling, every pixel until the standard error of its displayed value is at most T, --samples_per_pixel at most
+// (rt_render_adaptive; T = 0, the default, renders the fixed count; one GPU only).
 // There is no CPU renderer here: without a CUDA device the program fails with the library's error.
 #include <unistd.h>
 
@@ -143,9 +145,11 @@ int main(int argc, char** argv) {
     // ---- flags (main.rs:64-88)
     std::map<std::string, std::string> defaults = {{"aspect_ratio", "16:9"}, {"image_width", "400"}, {"samples_per_pixel", "200"},
                                                    {"max_depth", "50"},      {"up", "0,1.0,0"},     {"aperture", "0.0"},
-                                                   {"world", "simple"},      {"gpus", "1"},         {"pipeline", "auto"}};
+                                                   {"world", "simple"},      {"gpus", "1"},         {"pipeline", "auto"},
+                                                   {"noise_threshold", "0"}, {"min_samples", "16"}};
     const char* valued[] = {"aspect_ratio", "image_width", "samples_per_pixel", "max_depth", "lookfrom", "lookat", "up", "field_of_view",
-                            "aperture",     "focus_dist",  "world",             "seed",      "gpus",     "pipeline", "earthmap"};
+                            "aperture",     "focus_dist",  "world",             "seed",      "gpus",     "pipeline", "earthmap",
+                            "noise_threshold", "min_samples"};
     std::map<std::string, std::string> opt = defaults;
     bool randomized_rendering = false, want_stats = false;
     for (int i = 1; i < argc; ++i) {
@@ -226,6 +230,9 @@ int main(int argc, char** argv) {
     uint64_t world_seed = opt.count("seed") ? parse_u64(opt["seed"], "seed") : os_seed;
     uint64_t render_seed = (opt.count("seed") && !randomized_rendering) ? world_seed : (((uint64_t)rd() << 32) ^ (uint64_t)rd());
     long long gpus = parse_int(opt["gpus"], "gpus");
+    const double noise_threshold = parse_f64(opt["noise_threshold"], "noise_threshold");
+    const long long min_samples = parse_int(opt["min_samples"], "min_samples");
+    if (noise_threshold != 0.0 && gpus > 1) usage_error("--noise_threshold (adaptive sampling) renders on one GPU: it cannot be used with --gpus above 1");
     static const std::map<std::string, int> pipelines = {{"auto", RT_PIPELINE_AUTO}, {"megakernel", RT_PIPELINE_MEGAKERNEL},
                                                          {"wavefront", RT_PIPELINE_WAVEFRONT},
                                                          {"persistent", RT_PIPELINE_PERSISTENT}};
@@ -277,7 +284,15 @@ int main(int argc, char** argv) {
     std::vector<int32_t> rgb((size_t)3 * image_width * image_height);
     Progress prog{std::chrono::steady_clock::now(), 0};
     RtStats st;
-    int rc = rt_render_multi(scenes.data(), (int32_t)gpus, &cam, &p, nullptr, rgb.data(), progress_cb, &prog, &st);
+    int rc;
+    if (noise_threshold != 0.0) {
+        RtAdaptive ad;
+        memset(&ad, 0, sizeof ad);
+        ad.noise_threshold = noise_threshold, ad.min_samples = (int32_t)min_samples;
+        rc = rt_render_adaptive(scenes[0], &cam, &p, &ad, rgb.data(), nullptr, nullptr, nullptr, progress_cb, &prog, &st);
+    } else {
+        rc = rt_render_multi(scenes.data(), (int32_t)gpus, &cam, &p, nullptr, rgb.data(), progress_cb, &prog, &st);
+    }
     if (rc != RT_OK) {
         fprintf(stderr, "\nerror: %s\n", rt_last_error());
         return 1;
@@ -285,9 +300,9 @@ int main(int argc, char** argv) {
     double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - prog.start).count();
     fprintf(stderr, "\nRendered in %.3fs\n", secs);
     if (want_stats)
-        fprintf(stderr, "{\"paths\": %llu, \"rays\": %llu, \"device_ms\": %.3f, \"kernel_launches\": %d, \"pipeline\": %d, \"gpus\": %lld, \"mpaths_per_s\": %.1f}\n",
+        fprintf(stderr, "{\"paths\": %llu, \"rays\": %llu, \"device_ms\": %.3f, \"kernel_launches\": %d, \"pipeline\": %d, \"gpus\": %lld, \"mpaths_per_s\": %.1f, \"mean_spp\": %.3f}\n",
                 (unsigned long long)st.paths, (unsigned long long)st.rays, st.device_ms, st.kernel_launches, st.pipeline_used, gpus,
-                st.paths / (st.device_ms * 1e3));
+                st.paths / (st.device_ms * 1e3), (double)st.paths / ((double)image_width * (double)image_height));
     // ---- PPM body: rows in reverse j (top row first), one pixel per line
     std::string out;
     out.reserve((size_t)12 * image_width * image_height);

@@ -43,14 +43,6 @@ __global__ void __launch_bounds__(128) render_items_kernel(DSceneView S, DCamera
     if ((threadIdx.x & 31) == 0 && n_rays) atomicAdd(rays_out, (unsigned long long)n_rays);
 }
 
-// to_rgb (raytrace.rs:59-68): gamma 2, clamp, x255.999, truncate.  Done in f64 so that, given the same sums, the
-// bytes are the reference's.
-__device__ __forceinline__ int32_t to_rgb_f64(double mean) {
-    double x = sqrt(mean);
-    x = x < 0.0 ? 0.0 : (x > 0.99999999 ? 0.99999999 : x);  // f64::clamp keeps NaN; `as i32` maps NaN to 0
-    double y = 255.999 * x;
-    return (y != y) ? 0 : (int32_t)y;
-}
 __global__ void tonemap_kernel(const float* __restrict__ accum, int32_t* __restrict__ rgb, int n_values, double scale) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n_values) rgb[i] = to_rgb_f64((double)accum[i] * scale);
@@ -125,7 +117,7 @@ int upload(const std::vector<T>& v, T** out, std::vector<std::pair<void*, size_t
 }  // namespace
 
 
-namespace {
+namespace rtb {
 
 int have_device() {
     int n = 0;
@@ -136,6 +128,10 @@ int have_device() {
     }
     return RT_OK;
 }
+
+}  // namespace rtb
+
+namespace {
 
 int upload_scene(RtScene* s) {
     FlatScene& f = s->flat;
@@ -259,6 +255,10 @@ int create_scene(const RtSceneDesc* desc, int32_t root, bool build_bvh, int devi
     return RT_OK;
 }
 
+}  // namespace
+
+namespace rtb {
+
 int validate_render(const RtScene* scene, const RtCamera* cam, const RtParams* p) {
     if (!scene || !cam || !p) return set_error(RT_ERR_INVALID, "render: null argument");
     if (p->width < 2 || p->height < 2) return set_error(RT_ERR_INVALID, "render: image must be at least 2x2 (u = (i+U)/(W-1))");
@@ -269,9 +269,6 @@ int validate_render(const RtScene* scene, const RtCamera* cam, const RtParams* p
     return RT_OK;
 }
 
-}  // namespace
-
-namespace rtb {
 DRenderParams device_params(const RtParams* p, int first_sample, int spi, int chunks) {
     DRenderParams P{};
     P.width = p->width, P.height = p->height, P.max_depth = p->max_depth;

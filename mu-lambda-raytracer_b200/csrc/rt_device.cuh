@@ -1064,6 +1064,64 @@ RTB_DEV AccumFx radiance_fixed(float x) {
     return (AccumFx)fmaf(x, 4294967296.0f, 0.5f);
 }
 
+// EXTENSION: the square of one fixed-point sample q = radiance_fixed(x), exactly, in 2^-24 units of radiance^2
+// (RT_MOMENT2_FIXED_ONE): (min(q, 2^44))^2 >> 40.  A sample above 4096 is capped in the square, so one sample adds at
+// most 2^48 and a 64-bit sum holds 2^16 such extremes (about 2^40 ordinary ones).
+RTB_DEV AccumFx moment2_fixed(AccumFx q) {
+    q = q < (1ull << 44) ? q : (1ull << 44);
+#if defined(__CUDACC__) && !defined(RTB_HOST_EMULATION)
+    const AccumFx hi = __umul64hi(q, q);
+#else
+    const AccumFx hi = (AccumFx)(((unsigned __int128)q * q) >> 64);
+#endif
+    return (hi << 24) | ((q * q) >> 40);  // q^2 < 2^88: hi < 2^24
+}
+
+// to_rgb (raytrace.rs:59-68): gamma 2, clamp, x255.999, truncate.  Done in f64 so that, given the same sums, the
+// bytes are the reference's.
+RTB_DEV int32_t to_rgb_f64(double mean) {
+    double x = sqrt(mean);
+    x = x < 0.0 ? 0.0 : (x > 0.99999999 ? 0.99999999 : x);  // f64::clamp keeps NaN; `as i32` maps NaN to 0
+    double y = 255.999 * x;
+    return (y != y) ? 0 : (int32_t)y;
+}
+
+// EXTENSION: the stop rule of noise-threshold adaptive sampling (rt_render_adaptive) for one pixel that has received
+// samples [0, n) of at most n_max, from its fixed-point sums S1 (radiance_fixed) and S2 (moment2_fixed) per channel:
+//   mu = S1 2^-32 / n,  s^2 = max(0, (S2 2^-24 - n mu^2) / (n - 1)),  se = sqrt(s^2 / n),
+//   e = se / (2 sqrt(max(mu, 2^-16)))   (the standard error carried through the gamma-2 tonemap),
+// done when n == n_max or, for every channel, e <= threshold or mu - 3 se >= 1 (the channel saturates in to_rgb).
+// f64 with every operation rounded on its own (no contraction), so that a restatement in numpy agrees on every pixel.
+#if defined(__CUDACC__) && !defined(RTB_HOST_EMULATION)
+#define RTB_DMUL __dmul_rn
+#define RTB_DSUB __dsub_rn
+#define RTB_DDIV __ddiv_rn
+#define RTB_DSQRT __dsqrt_rn
+#else
+#define RTB_DMUL(a, b) ((double)(a) * (double)(b))
+#define RTB_DSUB(a, b) ((double)(a) - (double)(b))
+#define RTB_DDIV(a, b) ((double)(a) / (double)(b))
+#define RTB_DSQRT(a) sqrt((double)(a))
+#endif
+RTB_DEV bool adaptive_pixel_done(uint32_t n, uint32_t n_max, const AccumFx s1[3], const AccumFx s2[3], double threshold) {
+    if (n >= n_max) return true;
+    const double dn = (double)n;
+    for (int c = 0; c < 3; ++c) {
+        const double mu = RTB_DDIV(RTB_DMUL((double)s1[c], 2.3283064365386963e-10), dn);
+        const double m2 = RTB_DMUL((double)s2[c], 5.9604644775390625e-08);
+        double var = RTB_DDIV(RTB_DSUB(m2, RTB_DMUL(dn, RTB_DMUL(mu, mu))), RTB_DSUB(dn, 1.0));
+        var = var > 0.0 ? var : 0.0;
+        const double se = RTB_DSQRT(RTB_DDIV(var, dn));
+        const double e = RTB_DDIV(se, RTB_DMUL(2.0, RTB_DSQRT(mu > 1.52587890625e-05 ? mu : 1.52587890625e-05)));
+        if (!(e <= threshold || RTB_DSUB(mu, RTB_DMUL(3.0, se)) >= 1.0)) return false;
+    }
+    return true;
+}
+#undef RTB_DMUL
+#undef RTB_DSUB
+#undef RTB_DDIV
+#undef RTB_DSQRT
+
 // ------------------------------------------------------------------ one work item = one pixel x a run of samples
 // item -> (tile, lane): a warp covers an 8x4 pixel tile so that its 32 camera rays start coherent.
 RTB_DEV bool item_to_pixel(const DRenderParams& P, long long item, int& px, int& py, int& chunk) {

@@ -305,10 +305,19 @@ __device__ __forceinline__ uint2 chain_phase(float* pool, const SV& S, const DRe
 // Dynamic shared memory: [pool NS x PS_REC x NT floats][stack SD x NT keys][nodes4][prims].
 #define PS_SCENE_NODES 1
 #define PS_SCENE_PRIMS 2
-template <bool STATS, bool WIDE, int SD, int NT, int SCENE, int MEDIA, int NS, bool CHAIN, uint32_t FEAT, bool CHAINQ>
+// MOM (the moments family, persist_moments_kernel; IO = PsMomentsIO): every deposit also adds moment2_fixed of its
+// fixed-point sample to io.moment2, and path numbers run over the io.n_list pixels of io.plist (ascending pixel ids;
+// nullptr: pixel i is i).  The extra inputs ride in the type of `io` rather than in parameters of their own: one more
+// parameter, even unused, changes the instruction schedule of existing instances (DESIGN.md section 5d).
+struct PsMomentsIO : PsChainIO {
+    AccumFx* moment2;
+    const uint32_t* plist;
+    unsigned int n_list;
+};
+template <bool STATS, bool WIDE, int SD, int NT, int SCENE, int MEDIA, int NS, bool CHAIN, uint32_t FEAT, bool CHAINQ, bool MOM = false, class IO = PsChainIO>
 __device__ __forceinline__ void persist_body(const DSceneView& S_, const DCamera& cam, const DRenderParams& P, PsCounters* __restrict__ ctr,
                                              AccumFx* __restrict__ accum, unsigned long long* __restrict__ rays_out, unsigned int chunk_size,
-                                             unsigned long long* __restrict__ stats, const PsTune& tune, const PsChainIO& io) {
+                                             unsigned long long* __restrict__ stats, const PsTune& tune, const IO& io) {
     const SceneViewF<FEAT>& S = static_cast<const SceneViewF<FEAT>&>(S_);  // same record; SV::feat = what the scene can contain (rt_types.h)
     unsigned int st_[PSS_COUNT];
     if (STATS)
@@ -344,7 +353,8 @@ __device__ __forceinline__ void persist_body(const DSceneView& S_, const DCamera
     constexpr int DONE = WIDE ? (int)RTB_LINK4_DONE : PS_DONE;
     const int root_link = S.n_prims > 0 ? (WIDE ? 0 : (int)as_uint(ld4(S.nodes).w)) : DONE;
     const unsigned long long total = ctr->total_paths;
-    const unsigned int npix = (unsigned int)P.width * (unsigned int)P.height;
+    unsigned int npix = (unsigned int)P.width * (unsigned int)P.height;  // pixels the path numbers run over
+    if constexpr (MOM) npix = io.n_list;
 
     unsigned int stat = 0u;  // every slot ST_EMPTY
     // context of the traversal in flight (tslot < 0: none)
@@ -477,9 +487,17 @@ __device__ __forceinline__ void persist_body(const DSceneView& S_, const DCamera
                 if (radiance.y != 0.f) atomicAdd(reinterpret_cast<float*>(dst + 1), radiance.y);
                 if (radiance.z != 0.f) atomicAdd(reinterpret_cast<float*>(dst + 2), radiance.z);
 #else
-                if (radiance.x != 0.f) atomicAdd(dst + 0, radiance_fixed(radiance.x));
-                if (radiance.y != 0.f) atomicAdd(dst + 1, radiance_fixed(radiance.y));
-                if (radiance.z != 0.f) atomicAdd(dst + 2, radiance_fixed(radiance.z));
+                if constexpr (MOM) {  // the same sums (a zero sample adds nothing to either) and the squares of the samples
+                    AccumFx* dst2 = io.moment2 + 3 * (size_t)pixel_out;
+                    const AccumFx q0 = radiance_fixed(radiance.x), q1 = radiance_fixed(radiance.y), q2 = radiance_fixed(radiance.z);
+                    if (q0) atomicAdd(dst + 0, q0), atomicAdd(dst2 + 0, moment2_fixed(q0));
+                    if (q1) atomicAdd(dst + 1, q1), atomicAdd(dst2 + 1, moment2_fixed(q1));
+                    if (q2) atomicAdd(dst + 2, q2), atomicAdd(dst2 + 2, moment2_fixed(q2));
+                } else {
+                    if (radiance.x != 0.f) atomicAdd(dst + 0, radiance_fixed(radiance.x));
+                    if (radiance.y != 0.f) atomicAdd(dst + 1, radiance_fixed(radiance.y));
+                    if (radiance.z != 0.f) atomicAdd(dst + 2, radiance_fixed(radiance.z));
+                }
 #endif
             }
             // regenerate: the next camera paths of the job, handed out in reservation order
@@ -532,6 +550,9 @@ __device__ __forceinline__ void persist_body(const DSceneView& S_, const DCamera
                 if (need && rank < take) {
                     uint32_t pixel = chunk_pixel + rank, sample = chunk_sample;
                     while (pixel >= npix) pixel -= npix, sample += 1u;
+                    if constexpr (MOM) {
+                        if (io.plist) pixel = __ldg(io.plist + pixel);
+                    }
                     wf_init_camera<FEAT>(cam, P, pixel, sample, s);
                     segment_next = 0;
                     alive = true, need = false;
@@ -709,6 +730,20 @@ __global__ void __launch_bounds__(NT, (STATS || NT > 128) ? 1 : PS_MIN_BLOCKS) p
     persist_body<STATS, WIDE, SD, NT, SCENE, MEDIA, NS, CHAIN, FEAT, CHAINQ>(S, cam, P, ctr, accum, rays_out, chunk_size, stats, tune, io);
 }
 
+// EXTENSION: the moments family (rt_render_moments_fixed_device, rt_render_adaptive) — the product placement (two slots per
+// lane, no scene copy, no chain phase / queues / statistics) with second moments and a pixel list.  A kernel of its own, so
+// that the instances above stay as they were, instruction for instruction (DESIGN.md section 5b).
+template <bool WIDE, int NT, int MEDIA, uint32_t FEAT>
+__global__ void __launch_bounds__(NT, NT > 128 ? 1 : PS_MIN_BLOCKS) persist_moments_kernel(DSceneView S, DCamera cam, DRenderParams P, PsCounters* __restrict__ ctr,
+                                                                      AccumFx* __restrict__ accum, AccumFx* __restrict__ moment2,
+                                                                      const uint32_t* __restrict__ plist, unsigned int n_list,
+                                                                      unsigned long long* __restrict__ rays_out, unsigned int chunk_size, PsTune tune) {
+    PsMomentsIO io;
+    io.chain = io.exitq = nullptr, io.cc = nullptr, io.cap = 0u;
+    io.moment2 = moment2, io.plist = plist, io.n_list = n_list;
+    persist_body<false, WIDE, 0, NT, 0, MEDIA, 2, false, FEAT, false, true>(S, cam, P, ctr, accum, rays_out, chunk_size, nullptr, tune, io);
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 void free_persist(RtScene* s) {
     if (!s->ps) return;
@@ -831,6 +866,76 @@ int pick_variant(const RtScene* s, const RtParams* p) {
     return vi;
 }
 
+// the resident grid of a kernel instance (cached per instance in w->blocks under `key`), and the shared-memory carve-out
+int size_grid(RtScene* s, PersistState* w, const void* key, const void* kernel, int NT, size_t smem, const char* name) {
+    if (w->blocks.find(key) != w->blocks.end()) return RT_OK;
+    int per_sm = 0, sms = 0;
+    CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT, smem));
+    if (per_sm < 1) return set_error(RT_ERR_CUDA, "persistent pipeline: kernel instance '%s' does not fit an SM", name);
+    if (const char* e = getenv("RT_PS_BLOCKS_PER_SM")) per_sm = std::min(per_sm, std::max(1, atoi(e)));
+    // Ask for exactly the shared memory the resident blocks need (+1 KB per block the runtime reserves); whatever is left
+    // of the SM's 228 KB is L1, which holds the BVH, the primitives and the traversal stacks.  The driver's
+    // default carve-out was larger than needed and cost 5 % (L1 hit rate 92 %).
+    int need_kb = (int)((per_sm * (smem + 1024) + 1023) / 1024);
+    int percent = std::min(100, (need_kb * 100 + 227) / 228);
+    if (const char* e = getenv("RT_PS_CARVEOUT")) percent = atoi(e);
+    CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, percent));
+    CU_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
+    w->blocks[key] = per_sm * std::max(1, sms);  // persistent: exactly what is co-resident
+    return RT_OK;
+}
+
+// one launch of `total` camera paths over `npix` pixels: the grid (at most the resident one) and the reservation size
+void launch_shape(int resident, unsigned long long total, int NT, unsigned long long npix, int* blocks, unsigned int* chunk) {
+    *blocks = (int)std::min<unsigned long long>((unsigned long long)resident, (total + 2 * NT - 1) / (2 * NT));
+    // small jobs: smaller reservations so that every warp gets work
+    unsigned long long per_warp = total / ((unsigned long long)*blocks * (NT / 32) * 4ull);
+    *chunk = (unsigned int)std::min<unsigned long long>(PS_CHUNK, std::max<unsigned long long>(32ull, per_warp));
+    *chunk = (unsigned int)std::min<unsigned long long>(*chunk, std::max<unsigned long long>(1ull, npix));
+}
+
+PsTune read_tune() {
+    PsTune tune = {PS_WORK, PS_STALL, PS_LEAVE, PS_MIN_DESCEND, PS_CHAIN_TRIG, PS_CHAIN_MIN};
+    if (const char* e = getenv("RT_PS_CHAIN_TRIG")) tune.chain_trig = atoi(e);
+    if (const char* e = getenv("RT_PS_CHAIN_MIN")) tune.chain_min = std::max(1, atoi(e));
+    if (const char* e = getenv("RT_PS_WORK")) tune.work = atoi(e);
+    if (const char* e = getenv("RT_PS_STALL")) tune.stall = atoi(e);
+    if (const char* e = getenv("RT_PS_LEAVE")) tune.leave = atoi(e);
+    if (const char* e = getenv("RT_PS_DESCEND")) tune.descend = atoi(e);
+    return tune;
+}
+
+// ---- the moments family: the feature masks and media forms the default path picks (pick_feature_instance, the general
+// media sampler) on the 4-wide product placement, and the binary tree's variant for scenes beyond the 16-bit links of the
+// 4-wide tree.  RT_PS_VARIANT, RT_PS_CHAIN, RT_PS_CHAINQ and RT_PS_STATS do not apply to it.
+typedef void (*MomentsFn)(DSceneView, DCamera, DRenderParams, PsCounters*, AccumFx*, AccumFx*, const uint32_t*, unsigned int, unsigned long long*,
+                          unsigned int, PsTune);
+struct MomentsInstance {
+    uint32_t mask;
+    MomentsFn fn;
+};
+const MomentsInstance kMomentsFeat[] = {
+    {kFeatSpheres, persist_moments_kernel<true, 768, MEDIA_FAST, kFeatSpheres>},
+    {kFeatBoxes, persist_moments_kernel<true, 768, MEDIA_FAST, kFeatBoxes>},
+    {kFeatFinal, persist_moments_kernel<true, 768, MEDIA_FAST, kFeatFinal>},
+    {F_ALL, persist_moments_kernel<true, 768, MEDIA_FAST, F_ALL>},
+};
+const MomentsFn kMomentsWideGeneral = persist_moments_kernel<true, 768, MEDIA_GENERAL, F_ALL>;
+const MomentsFn kMomentsBinary = persist_moments_kernel<false, 128, MEDIA_FAST, F_ALL>;
+const MomentsFn kMomentsBinaryGeneral = persist_moments_kernel<false, 128, MEDIA_GENERAL, F_ALL>;
+
+MomentsFn pick_moments_instance(const RtScene* s, const RtParams* p, int* vi) {
+    *vi = pick_variant(s, p) == 0 ? 0 : PS_DEFAULT_VARIANT;
+    if (*vi == 0) return s->view.media_general ? kMomentsBinaryGeneral : kMomentsBinary;
+    if (s->view.media_general) return kMomentsWideGeneral;
+    bool specialise = true;
+    if (const char* e = getenv("RT_PS_FEAT")) specialise = atoi(e) != 0;
+    for (const MomentsInstance& f : kMomentsFeat)
+        if ((s->flat.features & ~f.mask) == 0u && (specialise || f.mask == F_ALL)) return f.fn;
+    return kMomentsFeat[3].fn;
+}
+
 }  // namespace
 
 int persist_layout_used(const RtScene* s, const RtParams* p) { return kVariants[pick_variant(s, p)].layout; }
@@ -868,22 +973,10 @@ int launch_persist(RtScene* s, const DCamera& cam, const RtParams* p, int begin,
     const size_t smem = variant_smem(V, s) / V.threads * NT;  // (every term of it is per thread for the variant feature instances exist for)
     const void* const key = getenv("RT_PS_STATS") ? (const void*)V.fn_stats : (const void*)kernel;
     if (w->blocks.find(key) == w->blocks.end()) {
-        int per_sm = 0, sms = 0;
         // (the statistics instance only when it will be launched: touching a kernel makes the driver load it, which a 3 ms job notices)
-        CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         if (getenv("RT_PS_STATS")) CU_TRY(cudaFuncSetAttribute(V.fn_stats, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT, smem));
-        if (per_sm < 1) return set_error(RT_ERR_CUDA, "persistent pipeline: kernel instance '%s' does not fit an SM", V.name);
-        if (const char* e = getenv("RT_PS_BLOCKS_PER_SM")) per_sm = std::min(per_sm, std::max(1, atoi(e)));
-        // Ask for exactly the shared memory the resident blocks need (+1 KB per block the runtime reserves); whatever is left
-        // of the SM's 228 KB is L1, which holds the BVH, the primitives and the traversal stacks.  The driver's
-        // default carve-out was larger than needed and cost 5 % (L1 hit rate 92 %).
-        int need_kb = (int)((per_sm * (smem + 1024) + 1023) / 1024);
-        int percent = std::min(100, (need_kb * 100 + 227) / 228);
-        if (const char* e = getenv("RT_PS_CARVEOUT")) percent = atoi(e);
-        CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, percent));
-        CU_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
-        w->blocks[key] = per_sm * std::max(1, sms);  // persistent: exactly what is co-resident
+        const int rc = size_grid(s, w, key, (const void*)kernel, NT, smem, V.name);
+        if (rc != RT_OK) return rc;
     }
     const unsigned long long npix = (unsigned long long)p->width * p->height;
     // one launch = up to 2^29 camera paths when progress is reported (a quarter of a second on C4), 2^33 otherwise: every
@@ -917,23 +1010,15 @@ int launch_persist(RtScene* s, const DCamera& cam, const RtParams* p, int begin,
         CU_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
         chain_blocks = std::max(1, per_sm) * std::max(1, sms);
     }
-    PsTune tune = {PS_WORK, PS_STALL, PS_LEAVE, PS_MIN_DESCEND, PS_CHAIN_TRIG, PS_CHAIN_MIN};
-    if (const char* e = getenv("RT_PS_CHAIN_TRIG")) tune.chain_trig = atoi(e);
-    if (const char* e = getenv("RT_PS_CHAIN_MIN")) tune.chain_min = std::max(1, atoi(e));
-    if (const char* e = getenv("RT_PS_WORK")) tune.work = atoi(e);
-    if (const char* e = getenv("RT_PS_STALL")) tune.stall = atoi(e);
-    if (const char* e = getenv("RT_PS_LEAVE")) tune.leave = atoi(e);
-    if (const char* e = getenv("RT_PS_DESCEND")) tune.descend = atoi(e);
+    const PsTune tune = read_tune();
     int done = 0;
     while (done < count) {
         int samples = std::min(count - done, samples_per_launch);
         unsigned long long total = npix * (unsigned long long)samples;
         DRenderParams P = device_params(p, begin + done, 1, 1);
-        int blocks = (int)std::min<unsigned long long>((unsigned long long)w->blocks[key], (total + 2 * NT - 1) / (2 * NT));
-        // small jobs: smaller reservations so that every warp gets work
-        unsigned long long per_warp = total / ((unsigned long long)blocks * (NT / 32) * 4ull);
-        unsigned int chunk = (unsigned int)std::min<unsigned long long>(PS_CHUNK, std::max<unsigned long long>(32ull, per_warp));
-        chunk = (unsigned int)std::min<unsigned long long>(chunk, std::max<unsigned long long>(1ull, npix));
+        int blocks = 0;
+        unsigned int chunk = 0u;
+        launch_shape(w->blocks[key], total, NT, npix, &blocks, &chunk);
         ps_reset_kernel<<<1, 1, 0, stream>>>(w->ctr, total, io.cc);
         if (getenv("RT_PS_STATS")) {  // debug: phase statistics on stderr (slower kernel; never used by the bench)
             unsigned long long* d_stats = nullptr;
@@ -983,6 +1068,42 @@ int launch_persist(RtScene* s, const DCamera& cam, const RtParams* p, int begin,
         chain_kernel<<<chain_blocks, CHAIN_THREADS, 0, stream>>>(s->view, P, io, s->d_rays);
         CU_TRY(cudaGetLastError());
         *launches += 4;
+    }
+    return RT_OK;
+}
+
+int launch_persist_moments(RtScene* s, const DCamera& cam, const RtParams* p, int begin, int count, AccumFx* d_accum, AccumFx* d_moment2,
+                           const uint32_t* d_list, unsigned int n_list, cudaStream_t stream, int* launches) {
+    if (!persist_supports(s, p)) return set_error(RT_ERR_UNSUPPORTED, "persistent pipeline: max_depth above %d or more than 2^24 primitives", WF_DEPTH_MASK);
+    if (p->bvh_layout != 0 && p->bvh_layout != 2 && p->bvh_layout != 4) return set_error(RT_ERR_INVALID, "render: bvh_layout must be 0 (auto), 2 or 4");
+    if (p->max_depth <= 0 || n_list == 0u) return RT_OK;
+    if (!s->ps) {
+        s->ps = new PersistState();
+        CU_TRY(rtb::cache_malloc((void**)&s->ps->ctr, sizeof(PsCounters)));
+    }
+    PersistState* w = s->ps;
+    int vi = 0;
+    const MomentsFn kernel = pick_moments_instance(s, p, &vi);
+    const Variant& V = kVariants[vi];
+    const int NT = V.threads;
+    const size_t smem = variant_smem(V, s);
+    int rc = size_grid(s, w, (const void*)kernel, (const void*)kernel, NT, smem, "moments");
+    if (rc != RT_OK) return rc;
+    const PsTune tune = read_tune();
+    const int samples_per_launch = (int)std::min<unsigned long long>(1u << 30, std::max<unsigned long long>(1, (1ull << 33) / n_list));
+    for (int done = 0; done < count;) {
+        const int samples = std::min(count - done, samples_per_launch);
+        const unsigned long long total = (unsigned long long)n_list * (unsigned long long)samples;
+        DRenderParams P = device_params(p, begin + done, 1, 1);
+        P.inv_npix = 1.0 / (double)n_list;
+        int blocks = 0;
+        unsigned int chunk = 0u;
+        launch_shape(w->blocks[(const void*)kernel], total, NT, n_list, &blocks, &chunk);
+        ps_reset_kernel<<<1, 1, 0, stream>>>(w->ctr, total, nullptr);
+        kernel<<<blocks, NT, smem, stream>>>(s->view, cam, P, w->ctr, d_accum, d_moment2, d_list, n_list, s->d_rays, chunk, tune);
+        CU_TRY(cudaGetLastError());
+        *launches += 2;
+        done += samples;
     }
     return RT_OK;
 }

@@ -84,4 +84,10 @@ int launch_persist(RtScene* s, const DCamera& cam, const RtParams* p, int begin,
                    RtProgressFn cb, void* user, int* launches);
 bool persist_supports(const RtScene* s, const RtParams* p);
 void free_persist(RtScene* s);
+// the moments family of the persistent kernel (EXTENSION): samples [begin, begin + count) of the n_list pixels of d_list
+// (ascending pixel ids; nullptr with n_list = W*H: every pixel), radiance_fixed ADDED into d_accum and moment2_fixed into d_moment2
+int launch_persist_moments(RtScene* s, const DCamera& cam, const RtParams* p, int begin, int count, AccumFx* d_accum, AccumFx* d_moment2,
+                           const uint32_t* d_list, unsigned int n_list, cudaStream_t stream, int* launches);
+int have_device();  // RT_OK, or RT_ERR_NO_DEVICE with the message set
+int validate_render(const RtScene* scene, const RtCamera* cam, const RtParams* p);
 }  // namespace rtb

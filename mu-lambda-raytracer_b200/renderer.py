@@ -212,6 +212,30 @@ class Renderer:  # raytrace.rs:137-198
                       "bvh_layout": stats.bvh_layout_used}
         return rgb, accum
 
+    def render_adaptive(self, noise_threshold, min_samples=16, logger=None):
+        """EXTENSION: noise-threshold adaptive sampling (rt_render_adaptive).  Every pixel gets samples until the standard
+        error of its tonemapped value is at most `noise_threshold` in every channel (or the channel saturates), at least
+        `min_samples` and at most parameters.samples_per_pixel.  Returns (rgb int32 [H,W,3], samples int32 [H,W],
+        accum_fixed uint64 [H,W,3], moment2_fixed uint64 [H,W,3]) with row 0 at the bottom; the sums are in
+        1 / RT_ACCUM_FIXED_ONE and 1 / RT_MOMENT2_FIXED_ONE units.  logger(j, H) as in render_arrays, paced by rounds."""
+        p = self._params()
+        h, w = p.height, p.width
+        rgb = np.empty((h, w, 3), dtype=np.int32)
+        samples = np.empty((h, w), dtype=np.int32)
+        accum = np.empty((h, w, 3), dtype=np.uint64)
+        moment2 = np.empty((h, w, 3), dtype=np.uint64)
+        ad = abi.RtAdaptive()
+        ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
+        cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
+        stats = abi.RtStats()
+        abi.check(abi.load().rt_render_adaptive(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad),
+                                                rgb.ctypes.data, samples.ctypes.data, accum.ctypes.data, moment2.ctypes.data,
+                                                cb, None, C.byref(stats)))
+        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
+                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
+                      "bvh_layout": stats.bvh_layout_used}
+        return rgb, samples, accum, moment2
+
     def render(self, logger=None):
         """Renderer::render: H rows of W (r, g, b) tuples, row j = 0 at the BOTTOM; logger(j, H) called H times."""
         rgb, _ = self.render_arrays(logger, want_accum=False)

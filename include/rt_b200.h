@@ -305,6 +305,48 @@ int rt_render_adaptive(const RtScene* scene, const RtCamera* cam, const RtParams
                        void* user, RtStats* stats);
 
 /*
+ * EXTENSION (no counterpart in the reference): a non-local-means denoiser guided by the per-pixel variance of the mean
+ * (Rousselle, Knaus & Zwicker, "Adaptive Rendering with Non-Local Means Filtering", SIGGRAPH Asia 2012).
+ *
+ * Per pixel p and channel c, with mean mu and variance of the mean v (f32, [H][W][3]), for every offset d of the search
+ * window [-r, r]^2 whose candidate q = p + d lies in the image, and y = clamp(x + d) (clamp = to the image):
+ *   e_d(x) = sum_c [(mu_c(x) - mu_c(y))^2 - alpha (v_c(x) + min(v_c(x), v_c(y)))] / (1e-10 + k^2 (v_c(x) + v_c(y)))
+ *   D(p, d) = mean of e_d(clamp(p + o)) over o in [-f, f]^2, / 3;   w = exp(-max(0, D)), and w = 1 for d = 0
+ *   out_c(p) = sum_d w mu_c(q) / sum_d w   (one weight for the three channels)
+ * The filter is biased: it trades noise for blur where patches look alike within their noise.
+ *
+ * rt_denoise_device: the filter on device buffers of `device` (3*W*H floats each; d_out_rgb must not overlap an input;
+ * height at most RT_DENOISE_MAX_HEIGHT, the rows of 65 535 tiles of 16).
+ * Deterministic: the same inputs give the same bits.  Asynchronous on `stream` (a cudaStream_t, NULL = default stream).
+ *
+ * rt_render_denoised: renders through the moments family of rt_render_moments_fixed_device — a uniform render of
+ * samples_per_pixel (>= 2) when `adaptive` is NULL, else the rounds of rt_render_adaptive — then, per pixel with its own
+ * count n, mu = S1 2^-32 / n and v = max(0, (S2 2^-24 - n mu^2) / (n - 1)) / n (f64, each rounded once to f32), denoises
+ * and tonemaps the result with to_rgb.  Host buffers, each optional, row 0 at the bottom: rgb (3*W*H int32) and
+ * denoised_rgb (3*W*H floats, the filtered means).  Persistent pipeline only; sample_begin and sample_count must be 0.
+ * cb: called once per row index as in rt_render; an adaptive render paces it by rounds, a uniform one reports every row
+ * when the render has finished (the moments family runs as one launch).  stats: paths traced, device_ms from the first render launch to the
+ * end of the tonemap.
+ */
+#define RT_DENOISE_DEFAULT_SEARCH_RADIUS 10
+#define RT_DENOISE_DEFAULT_PATCH_RADIUS 3
+#define RT_DENOISE_DEFAULT_K 0.45
+#define RT_DENOISE_DEFAULT_ALPHA 1.0
+#define RT_DENOISE_MAX_SEARCH_RADIUS 15
+#define RT_DENOISE_MAX_PATCH_RADIUS 7
+#define RT_DENOISE_MAX_HEIGHT 1048560
+typedef struct RtDenoise {
+    double k;              /* strength, > 0: larger blurs more */
+    double alpha;          /* variance cancellation, >= 0 */
+    int32_t search_radius; /* r in [0, RT_DENOISE_MAX_SEARCH_RADIUS]; 0 returns the input */
+    int32_t patch_radius;  /* f in [0, RT_DENOISE_MAX_PATCH_RADIUS] */
+} RtDenoise;
+int rt_denoise_device(const float* d_mean_rgb, const float* d_var_rgb, int32_t width, int32_t height, const RtDenoise* opt,
+                      float* d_out_rgb, int device, void* stream);
+int rt_render_denoised(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* adaptive,
+                       const RtDenoise* opt, int32_t* rgb, float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats);
+
+/*
  * rt_render over several GPUs of one process (the reference's row-parallel rayon loop, raytrace.rs:176-185, becomes
  * sample slices): scenes[g] is the same description created on a distinct device; device g renders every pixel for
  * the g-th slice of the sample range (rt_sample_slice), the float accumulation buffers are summed onto scenes[0]'s

@@ -143,6 +143,31 @@ pub struct RtAdaptive {
     pub reserved: i32,
 }
 pub const RT_MOMENT2_FIXED_ONE: f64 = 16777216.0;
+/// EXTENSION: variance-guided non-local-means denoiser (rt_denoise_device, rt_render_denoised)
+#[repr(C)]
+pub struct RtDenoise {
+    pub k: f64,
+    pub alpha: f64,
+    pub search_radius: i32,
+    pub patch_radius: i32,
+}
+pub const RT_DENOISE_DEFAULT_SEARCH_RADIUS: i32 = 10;
+pub const RT_DENOISE_DEFAULT_PATCH_RADIUS: i32 = 3;
+pub const RT_DENOISE_DEFAULT_K: f64 = 0.45;
+pub const RT_DENOISE_DEFAULT_ALPHA: f64 = 1.0;
+pub const RT_DENOISE_MAX_SEARCH_RADIUS: i32 = 15;
+pub const RT_DENOISE_MAX_PATCH_RADIUS: i32 = 7;
+pub const RT_DENOISE_MAX_HEIGHT: i32 = 1048560;
+impl Default for RtDenoise {
+    fn default() -> RtDenoise {
+        RtDenoise {
+            k: RT_DENOISE_DEFAULT_K,
+            alpha: RT_DENOISE_DEFAULT_ALPHA,
+            search_radius: RT_DENOISE_DEFAULT_SEARCH_RADIUS,
+            patch_radius: RT_DENOISE_DEFAULT_PATCH_RADIUS,
+        }
+    }
+}
 pub enum RtScene {}
 /// Called once per image row j = 0 .. total-1, in increasing order, on the calling thread (include/rt_b200.h).
 pub type RtProgressFn = Option<extern "C" fn(row: c_int, total: c_int, user: *mut c_void)>;
@@ -164,6 +189,10 @@ extern "C" {
     pub fn rt_render_adaptive(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive, rgb: *mut i32,
                               samples: *mut i32, accum_fixed: *mut u64, moment2_fixed: *mut u64, cb: RtProgressFn, user: *mut c_void,
                               stats: *mut RtStats) -> c_int;
+    pub fn rt_denoise_device(d_mean_rgb: *const f32, d_var_rgb: *const f32, width: i32, height: i32, opt: *const RtDenoise, d_out_rgb: *mut f32,
+                             device: c_int, stream: *mut c_void) -> c_int;
+    pub fn rt_render_denoised(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive, opt: *const RtDenoise,
+                              rgb: *mut i32, denoised_rgb: *mut f32, cb: RtProgressFn, user: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_world_build(name: *const c_char, seed: u64, earth_rgb: *const u8, earth_w: i32, earth_h: i32, out: *mut *mut RtSceneDesc,
                           n_draws: *mut u64) -> c_int;
     pub fn rt_scene_desc_free(desc: *mut RtSceneDesc);

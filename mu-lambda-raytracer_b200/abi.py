@@ -95,6 +95,14 @@ class RtAdaptive(C.Structure):  # EXTENSION: noise-threshold adaptive sampling (
     _fields_ = [("noise_threshold", C.c_double), ("min_samples", C.c_int32), ("reserved", C.c_int32)]
 
 
+class RtDenoise(C.Structure):  # EXTENSION: variance-guided non-local-means denoiser (rt_denoise_device, rt_render_denoised)
+    _fields_ = [("k", C.c_double), ("alpha", C.c_double), ("search_radius", C.c_int32), ("patch_radius", C.c_int32)]
+
+
+RT_DENOISE_DEFAULT_SEARCH_RADIUS, RT_DENOISE_DEFAULT_PATCH_RADIUS, RT_DENOISE_DEFAULT_K, RT_DENOISE_DEFAULT_ALPHA = 10, 3, 0.45, 1.0
+RT_DENOISE_MAX_SEARCH_RADIUS, RT_DENOISE_MAX_PATCH_RADIUS, RT_DENOISE_MAX_HEIGHT = 15, 7, 1048560
+
+
 class RtWorldInfo(C.Structure):
     _fields_ = [("lookfrom", C.c_double * 3), ("lookat", C.c_double * 3), ("vfov_deg", C.c_double),
                 ("background_kind", C.c_int32), ("needs_earthmap", C.c_int32), ("uses_rng", C.c_int32)]
@@ -127,6 +135,9 @@ PROTOTYPES = {
                                                  C.c_void_p, C.POINTER(RtStats)]),
     "rt_render_adaptive": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
+    "rt_denoise_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(RtDenoise), C.c_void_p, C.c_int, C.c_void_p]),
+    "rt_render_denoised": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtDenoise),
+                                     C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
     "rt_tonemap_fixed_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int, C.c_void_p]),
     "rt_accum_fixed_to_float_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rt_release_cached_memory": (None, []),

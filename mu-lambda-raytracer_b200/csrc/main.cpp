@@ -12,7 +12,9 @@
 // --earthmap FILE (decoded RGB8 as binary PPM; default $RT_EARTHMAP, ./earthmap.ppm, then the shipped asset),
 // --stats (one JSON line with paths, rays, device ms on stderr), --noise_threshold T with --min_samples N (16): adaptive
 // sampling, every pixel until the standard error of its displayed value is at most T, --samples_per_pixel at most
-// (rt_render_adaptive; T = 0, the default, renders the fixed count; one GPU only).
+// (rt_render_adaptive; T = 0, the default, renders the fixed count; one GPU only), --denoise: the variance-guided
+// non-local-means filter with the library's default parameters after the render, uniform or adaptive (rt_render_denoised;
+// one GPU only; --stats then covers the render and the filter).
 // There is no CPU renderer here: without a CUDA device the program fails with the library's error.
 #include <unistd.h>
 
@@ -151,7 +153,7 @@ int main(int argc, char** argv) {
                             "aperture",     "focus_dist",  "world",             "seed",      "gpus",     "pipeline", "earthmap",
                             "noise_threshold", "min_samples"};
     std::map<std::string, std::string> opt = defaults;
-    bool randomized_rendering = false, want_stats = false;
+    bool randomized_rendering = false, want_stats = false, want_denoise = false;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "--randomized_rendering" || a == "-r") {
@@ -162,8 +164,12 @@ int main(int argc, char** argv) {
             want_stats = true;
             continue;
         }
+        if (a == "--denoise") {
+            want_denoise = true;
+            continue;
+        }
         if (a == "--help" || a == "-h") {
-            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n\nOPTIONS:\n");
+            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n        --denoise\n\nOPTIONS:\n");
             for (const char* v : valued) {
                 auto d = defaults.find(v);
                 printf("        --%s <%s>%s%s%s\n", v, v, d != defaults.end() ? " [default: " : "", d != defaults.end() ? d->second.c_str() : "",
@@ -233,6 +239,7 @@ int main(int argc, char** argv) {
     const double noise_threshold = parse_f64(opt["noise_threshold"], "noise_threshold");
     const long long min_samples = parse_int(opt["min_samples"], "min_samples");
     if (noise_threshold != 0.0 && gpus > 1) usage_error("--noise_threshold (adaptive sampling) renders on one GPU: it cannot be used with --gpus above 1");
+    if (want_denoise && gpus > 1) usage_error("--denoise renders and filters on one GPU: it cannot be used with --gpus above 1");
     static const std::map<std::string, int> pipelines = {{"auto", RT_PIPELINE_AUTO}, {"megakernel", RT_PIPELINE_MEGAKERNEL},
                                                          {"wavefront", RT_PIPELINE_WAVEFRONT},
                                                          {"persistent", RT_PIPELINE_PERSISTENT}};
@@ -285,10 +292,16 @@ int main(int argc, char** argv) {
     Progress prog{std::chrono::steady_clock::now(), 0};
     RtStats st;
     int rc;
-    if (noise_threshold != 0.0) {
-        RtAdaptive ad;
-        memset(&ad, 0, sizeof ad);
-        ad.noise_threshold = noise_threshold, ad.min_samples = (int32_t)min_samples;
+    RtAdaptive ad;
+    memset(&ad, 0, sizeof ad);
+    ad.noise_threshold = noise_threshold, ad.min_samples = (int32_t)min_samples;
+    if (want_denoise) {
+        RtDenoise dn;
+        memset(&dn, 0, sizeof dn);
+        dn.k = RT_DENOISE_DEFAULT_K, dn.alpha = RT_DENOISE_DEFAULT_ALPHA;
+        dn.search_radius = RT_DENOISE_DEFAULT_SEARCH_RADIUS, dn.patch_radius = RT_DENOISE_DEFAULT_PATCH_RADIUS;
+        rc = rt_render_denoised(scenes[0], &cam, &p, noise_threshold != 0.0 ? &ad : nullptr, &dn, rgb.data(), nullptr, progress_cb, &prog, &st);
+    } else if (noise_threshold != 0.0) {
         rc = rt_render_adaptive(scenes[0], &cam, &p, &ad, rgb.data(), nullptr, nullptr, nullptr, progress_cb, &prog, &st);
     } else {
         rc = rt_render_multi(scenes.data(), (int32_t)gpus, &cam, &p, nullptr, rgb.data(), progress_cb, &prog, &st);

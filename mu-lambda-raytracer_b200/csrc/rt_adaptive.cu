@@ -23,6 +23,26 @@
 
 using namespace rtb;
 
+namespace rtb {
+
+int check_pipeline(const RtParams* p) {
+    if (p->pipeline != RT_PIPELINE_AUTO && p->pipeline != RT_PIPELINE_PERSISTENT)
+        return set_error(RT_ERR_UNSUPPORTED, "moments and adaptive sampling run on the persistent pipeline only (pipeline AUTO or PERSISTENT)");
+    return RT_OK;
+}
+
+int check_adaptive(const RtParams* params, const RtAdaptive* ad, const char* who) {
+    if (!ad) return set_error(RT_ERR_INVALID, "%s: null RtAdaptive", who);
+    if (params->sample_begin != 0 || params->sample_count != 0)
+        return set_error(RT_ERR_INVALID, "%s: sample_begin and sample_count must be 0 (the render owns the sample range)", who);
+    if (ad->min_samples < 2 || ad->min_samples > params->samples_per_pixel)
+        return set_error(RT_ERR_INVALID, "%s: min_samples must lie in [2, samples_per_pixel]", who);
+    if (!(ad->noise_threshold >= 0.0)) return set_error(RT_ERR_INVALID, "%s: noise_threshold must be >= 0", who);
+    return RT_OK;
+}
+
+}  // namespace rtb
+
 namespace {
 
 __global__ void iota_kernel(uint32_t* __restrict__ list, unsigned int n) {
@@ -47,32 +67,96 @@ __global__ void tonemap_counts_kernel(const AccumFx* __restrict__ accum, const i
     if (i < n_values) rgb[i] = to_rgb_f64((double)accum[i] * (1.0 / (RT_ACCUM_FIXED_ONE * (double)samples[i / 3])));
 }
 
-int check_pipeline(const RtParams* p) {
-    if (p->pipeline != RT_PIPELINE_AUTO && p->pipeline != RT_PIPELINE_PERSISTENT)
-        return set_error(RT_ERR_UNSUPPORTED, "moments and adaptive sampling run on the persistent pipeline only (pipeline AUTO or PERSISTENT)");
-    return RT_OK;
-}
-
-// device blocks of one adaptive render, returned to the device cache on every exit
-struct AdaptiveBuffers {
-    AccumFx *accum = nullptr, *moment2 = nullptr;
-    int32_t *samples = nullptr, *rgb = nullptr;
+// device blocks of the rounds (lists, flags, selection scratch), returned to the device cache on every exit
+struct RoundBuffers {
     uint32_t *list_a = nullptr, *list_b = nullptr;
     unsigned char* keep = nullptr;
     int* n_sel = nullptr;
     void* temp = nullptr;
     size_t n_pixels = 0, temp_bytes = 0;
-    ~AdaptiveBuffers() {
+    ~RoundBuffers() {
         cudaStreamSynchronize(0);  // (an error return may leave work in flight; the cache hands blocks on without a free)
         const size_t n = n_pixels;
-        rtb::cache_free(accum, 3 * n * sizeof(AccumFx)), rtb::cache_free(moment2, 3 * n * sizeof(AccumFx));
-        rtb::cache_free(samples, n * sizeof(int32_t)), rtb::cache_free(rgb, 3 * n * sizeof(int32_t));
         rtb::cache_free(list_a, n * sizeof(uint32_t)), rtb::cache_free(list_b, n * sizeof(uint32_t));
         rtb::cache_free(keep, n), rtb::cache_free(n_sel, sizeof(int)), rtb::cache_free(temp, temp_bytes);
     }
 };
 
+// the outputs of one adaptive render on the device
+struct AdaptiveBuffers {
+    AccumFx *accum = nullptr, *moment2 = nullptr;
+    int32_t *samples = nullptr, *rgb = nullptr;
+    size_t n_pixels = 0;
+    ~AdaptiveBuffers() {
+        cudaStreamSynchronize(0);
+        const size_t n = n_pixels;
+        rtb::cache_free(accum, 3 * n * sizeof(AccumFx)), rtb::cache_free(moment2, 3 * n * sizeof(AccumFx));
+        rtb::cache_free(samples, n * sizeof(int32_t)), rtb::cache_free(rgb, 3 * n * sizeof(int32_t));
+    }
+};
+
 }  // namespace
+
+namespace rtb {
+
+int adaptive_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, AccumFx* d_accum, AccumFx* d_moment2,
+                    int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches_out, uint64_t* paths_out) {
+    const unsigned int npix = (unsigned int)params->width * (unsigned int)params->height;
+    const size_t n_values = 3 * (size_t)npix;
+    const uint32_t n_max = (uint32_t)params->samples_per_pixel, m = (uint32_t)ad->min_samples;
+
+    RoundBuffers b;
+    b.n_pixels = npix;
+    CU_TRY(rtb::cache_malloc((void**)&b.list_a, npix * sizeof(uint32_t)));
+    CU_TRY(rtb::cache_malloc((void**)&b.list_b, npix * sizeof(uint32_t)));
+    CU_TRY(rtb::cache_malloc((void**)&b.keep, npix));
+    CU_TRY(rtb::cache_malloc((void**)&b.n_sel, sizeof(int)));
+    CU_TRY(cub::DeviceSelect::Flagged(nullptr, b.temp_bytes, b.list_a, b.keep, b.list_b, b.n_sel, (int)npix, stream));
+    CU_TRY(rtb::cache_malloc(&b.temp, b.temp_bytes));
+
+    DCamera dc;
+    make_camera(*cam, dc);
+    int n_rounds = 1;  // the schedule depends on (m, max) alone: the logger is paced by rounds
+    for (uint32_t n = m; n < n_max; n += std::min(n, n_max - n)) n_rounds += 1;
+
+    CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
+    CU_TRY(cudaEventRecord(scene->ev0, stream));
+    CU_TRY(cudaMemsetAsync(d_accum, 0, n_values * sizeof(AccumFx), stream));
+    CU_TRY(cudaMemsetAsync(d_moment2, 0, n_values * sizeof(AccumFx), stream));
+    iota_kernel<<<(npix + 255) / 256, 256, 0, stream>>>(b.list_a, npix);
+    CU_TRY(cudaGetLastError());
+    int launches = 1;
+    uint64_t paths = 0;
+    unsigned int n_list = npix;
+    uint32_t n_done = 0;  // samples every active pixel holds
+    for (int round = 0; n_list > 0u; ++round) {
+        const uint32_t count = round == 0 ? m : std::min(n_done, n_max - n_done);
+        // round 0 covers every pixel: the list is the identity, which the kernel takes as a null list
+        int rc = launch_persist_moments(scene, dc, params, (int)n_done, (int)count, d_accum, d_moment2, round == 0 ? nullptr : b.list_a, n_list, stream,
+                                        &launches);
+        if (rc != RT_OK) return rc;
+        paths += (uint64_t)n_list * count;
+        n_done += count;
+        adaptive_eval_kernel<<<(n_list + 255) / 256, 256, 0, stream>>>(b.list_a, n_list, n_done, n_max, ad->noise_threshold, d_accum, d_moment2, d_samples,
+                                                                       b.keep);
+        CU_TRY(cudaGetLastError());
+        launches += 1;
+        int n_next = 0;
+        if (n_done < n_max) {
+            CU_TRY(cub::DeviceSelect::Flagged(b.temp, b.temp_bytes, b.list_a, b.keep, b.list_b, b.n_sel, (int)n_list, stream));
+            CU_TRY(cudaMemcpyAsync(&n_next, b.n_sel, sizeof(int), cudaMemcpyDeviceToHost, stream));
+            launches += 1;
+        }
+        CU_TRY(cudaStreamSynchronize(stream));
+        std::swap(b.list_a, b.list_b);
+        n_list = (unsigned int)n_next;
+        rtb::row_progress(round + 1, n_rounds, rows);
+    }
+    *launches_out += launches, *paths_out += paths;
+    return RT_OK;
+}
+
+}  // namespace rtb
 
 extern "C" {
 
@@ -121,19 +205,13 @@ int rt_render_adaptive(const RtScene* scene_, const RtCamera* cam, const RtParam
     int rc = have_device();
     if (rc != RT_OK) return rc;
     if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
-    if (!ad) return set_error(RT_ERR_INVALID, "rt_render_adaptive: null RtAdaptive");
-    if (params->sample_begin != 0 || params->sample_count != 0)
-        return set_error(RT_ERR_INVALID, "rt_render_adaptive: sample_begin and sample_count must be 0 (the render owns the sample range)");
-    if (ad->min_samples < 2 || ad->min_samples > params->samples_per_pixel)
-        return set_error(RT_ERR_INVALID, "rt_render_adaptive: min_samples must lie in [2, samples_per_pixel]");
-    if (!(ad->noise_threshold >= 0.0)) return set_error(RT_ERR_INVALID, "rt_render_adaptive: noise_threshold must be >= 0");
+    if ((rc = check_adaptive(params, ad, "rt_render_adaptive")) != RT_OK) return rc;
     if ((rc = check_pipeline(params)) != RT_OK) return rc;
     RtScene* scene = const_cast<RtScene*>(scene_);
     DeviceGuard g(scene->device);
     cudaStream_t stream = 0;
     const unsigned int npix = (unsigned int)params->width * (unsigned int)params->height;
     const size_t n_values = 3 * (size_t)npix;
-    const uint32_t n_max = (uint32_t)params->samples_per_pixel, m = (uint32_t)ad->min_samples;
 
     AdaptiveBuffers b;
     b.n_pixels = npix;
@@ -141,51 +219,12 @@ int rt_render_adaptive(const RtScene* scene_, const RtCamera* cam, const RtParam
     CU_TRY(rtb::cache_malloc((void**)&b.moment2, n_values * sizeof(AccumFx)));
     CU_TRY(rtb::cache_malloc((void**)&b.samples, npix * sizeof(int32_t)));
     CU_TRY(rtb::cache_malloc((void**)&b.rgb, n_values * sizeof(int32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.list_a, npix * sizeof(uint32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.list_b, npix * sizeof(uint32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.keep, npix));
-    CU_TRY(rtb::cache_malloc((void**)&b.n_sel, sizeof(int)));
-    CU_TRY(cub::DeviceSelect::Flagged(nullptr, b.temp_bytes, b.list_a, b.keep, b.list_b, b.n_sel, (int)npix, stream));
-    CU_TRY(rtb::cache_malloc(&b.temp, b.temp_bytes));
 
-    DCamera dc;
-    make_camera(*cam, dc);
     rtb::RowProgress rows{cb, user, params->height, 0};
-    int n_rounds = 1;  // the schedule depends on (m, max) alone: the logger is paced by rounds
-    for (uint32_t n = m; n < n_max; n += std::min(n, n_max - n)) n_rounds += 1;
-
-    CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
-    CU_TRY(cudaEventRecord(scene->ev0, stream));
-    CU_TRY(cudaMemsetAsync(b.accum, 0, n_values * sizeof(AccumFx), stream));
-    CU_TRY(cudaMemsetAsync(b.moment2, 0, n_values * sizeof(AccumFx), stream));
-    iota_kernel<<<(npix + 255) / 256, 256, 0, stream>>>(b.list_a, npix);
-    CU_TRY(cudaGetLastError());
-    int launches = 1;
+    int launches = 0;
     uint64_t paths = 0;
-    unsigned int n_list = npix;
-    uint32_t n_done = 0;  // samples every active pixel holds
-    for (int round = 0; n_list > 0u; ++round) {
-        const uint32_t count = round == 0 ? m : std::min(n_done, n_max - n_done);
-        // round 0 covers every pixel: the list is the identity, which the kernel takes as a null list
-        rc = launch_persist_moments(scene, dc, params, (int)n_done, (int)count, b.accum, b.moment2, round == 0 ? nullptr : b.list_a, n_list, stream, &launches);
-        if (rc != RT_OK) return rc;
-        paths += (uint64_t)n_list * count;
-        n_done += count;
-        adaptive_eval_kernel<<<(n_list + 255) / 256, 256, 0, stream>>>(b.list_a, n_list, n_done, n_max, ad->noise_threshold, b.accum, b.moment2, b.samples,
-                                                                       b.keep);
-        CU_TRY(cudaGetLastError());
-        launches += 1;
-        int n_next = 0;
-        if (n_done < n_max) {
-            CU_TRY(cub::DeviceSelect::Flagged(b.temp, b.temp_bytes, b.list_a, b.keep, b.list_b, b.n_sel, (int)n_list, stream));
-            CU_TRY(cudaMemcpyAsync(&n_next, b.n_sel, sizeof(int), cudaMemcpyDeviceToHost, stream));
-            launches += 1;
-        }
-        CU_TRY(cudaStreamSynchronize(stream));
-        std::swap(b.list_a, b.list_b);
-        n_list = (unsigned int)n_next;
-        rtb::row_progress(round + 1, n_rounds, &rows);
-    }
+    rc = adaptive_rounds(scene, cam, params, ad, b.accum, b.moment2, b.samples, stream, &rows, &launches, &paths);
+    if (rc != RT_OK) return rc;
     tonemap_counts_kernel<<<(unsigned)((n_values + 255) / 256), 256, 0, stream>>>(b.accum, b.samples, b.rgb, (int)n_values);
     CU_TRY(cudaGetLastError());
     launches += 1;

@@ -1,0 +1,314 @@
+// EXTENSION (no counterpart in the reference): a non-local-means denoiser guided by the exact per-pixel variance of the
+// moments family (Rousselle, Knaus & Zwicker 2012; the definition is in include/rt_b200.h, the per-pixel functions in
+// rt_denoise.cuh).
+//
+// denoise_nlm_kernel: one block of 32 x 8 threads filters a tile of 32 x 16 pixels.  It loads mu and v of the tile plus a halo of
+// r + f pixels (clamped to the image) into shared memory as six planes, then loops over the offsets d of the search window:
+//   1. e_d on the tile plus a halo of f (each thread keeps the terms of its own locations x in registers), into E;
+//   2. the horizontal box sums of E over 2f + 1 columns, into H;
+//   3. per output pixel, the vertical box sum of H over 2f + 1 rows gives D; w = exp(-max(0, D)) and w mu(q) are
+//      accumulated in registers.
+// Two barriers per offset; no atomics, and every sum runs in a fixed order, so the output is reproducible bit for bit.
+// d = 0 has weight 1 and is not evaluated; an offset that puts every candidate of the tile outside the image is skipped.
+//
+// rt_render_denoised renders through the moments family (rt_adaptive.cu), converts the sums (denoise_mean_var), filters and
+// tonemaps.
+#include <cuda_runtime.h>
+
+#include <algorithm>
+#include <cmath>
+#include <cstring>
+
+#include "rt_denoise.cuh"
+#include "rt_device.cuh"
+#include "scene_internal.h"
+
+using namespace rtb;
+
+namespace {
+
+constexpr int kTileX = 32, kTileY = 16, kThreadsY = 8, kThreads = kTileX * kThreadsY;
+static_assert(RT_DENOISE_MAX_HEIGHT == 65535 * kTileY, "the grid's y dimension holds at most 65 535 tiles");
+
+// shared-memory locations of e per thread: ceil((32 + 2f)(16 + 2f) / 256)
+constexpr int locations_per_thread(int f) { return ((kTileX + 2 * f) * (kTileY + 2 * f) + kThreads - 1) / kThreads; }
+
+size_t smem_bytes(int r, int f) {
+    const size_t R = (size_t)r + f;
+    return sizeof(float) * (6 * (kTileX + 2 * R) * (kTileY + 2 * R) + (size_t)(kTileX + 2 * f) * (kTileY + 2 * f) + (size_t)kTileX * (kTileY + 2 * f));
+}
+
+__device__ __forceinline__ int clampi(int x, int hi) { return x < 0 ? 0 : (x > hi ? hi : x); }
+
+}  // namespace
+
+namespace rtb {  // kernels with stable names (profiles)
+
+template <int NE>
+__global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const float* __restrict__ mean, const float* __restrict__ var, int W, int H, int r, int f,
+                                                               float k2, float alpha, float inv_norm, float* __restrict__ out) {
+    extern __shared__ float smem[];
+    const int R = r + f;
+    const int SW = kTileX + 2 * R, SH = kTileY + 2 * R, plane = SW * SH;
+    const int EW = kTileX + 2 * f, EH = kTileY + 2 * f, n_e = EW * EH;
+    float* E = smem + 6 * plane;
+    float* Hs = E + n_e;
+    const int tid = threadIdx.y * kTileX + threadIdx.x;
+    const int x0 = blockIdx.x * kTileX, y0 = blockIdx.y * kTileY;
+    const int sx0 = x0 - R, sy0 = y0 - R;
+
+    // mu and v of the tile plus its halo, clamped to the image, as planes mu_r mu_g mu_b v_r v_g v_b
+    for (int i = tid; i < plane; i += kThreads) {
+        const int gx = clampi(sx0 + i % SW, W - 1), gy = clampi(sy0 + i / SW, H - 1);
+        const size_t g = 3 * ((size_t)gy * W + gx);
+        for (int c = 0; c < 3; ++c) smem[c * plane + i] = mean[g + c], smem[(3 + c) * plane + i] = var[g + c];
+    }
+    __syncthreads();
+
+    // this thread's locations x of e (clamped image coordinates) and their terms that do not depend on the offset
+    int xs[NE], ys[NE];
+    float mx[NE][3], vx[NE][3], ax[NE][3], cx[NE][3];
+#pragma unroll
+    for (int k = 0; k < NE; ++k) {
+        const int l = tid + k * kThreads;
+        xs[k] = clampi(x0 - f + l % EW, W - 1), ys[k] = clampi(y0 - f + l / EW, H - 1);
+        const int s = l < n_e ? (ys[k] - sy0) * SW + (xs[k] - sx0) : 0;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            mx[k][c] = smem[c * plane + s], vx[k][c] = smem[(3 + c) * plane + s];
+            denoise_x_terms(vx[k][c], alpha, k2, &ax[k][c], &cx[k][c]);
+        }
+    }
+
+    // output pixels (x0 + tx, y0 + ty + 8m), m = 0, 1; d = 0 has weight 1
+    const int px = x0 + threadIdx.x;
+    float wsum[2], acc[2][3];
+#pragma unroll
+    for (int m = 0; m < 2; ++m) {
+        const int s = (y0 + threadIdx.y + kThreadsY * m - sy0) * SW + (px - sx0);
+        wsum[m] = 1.0f;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) acc[m][c] = smem[c * plane + s];
+    }
+
+    const int taps = 2 * f + 1;
+    for (int dy = -r; dy <= r; ++dy) {
+        if (y0 + dy > H - 1 || y0 + kTileY - 1 + dy < 0) continue;  // every candidate of the tile is outside the image
+        for (int dx = -r; dx <= r; ++dx) {
+            if ((dx | dy) == 0 || x0 + dx > W - 1 || x0 + kTileX - 1 + dx < 0) continue;
+            // 1. e_d at this thread's locations
+#pragma unroll
+            for (int k = 0; k < NE; ++k) {
+                const int l = tid + k * kThreads;
+                if (NE * kThreads <= n_e || l < n_e) {
+                    const int s = (clampi(ys[k] + dy, H - 1) - sy0) * SW + (clampi(xs[k] + dx, W - 1) - sx0);
+                    float e = 0.0f;
+#pragma unroll
+                    for (int c = 0; c < 3; ++c)
+                        e += denoise_term(mx[k][c], vx[k][c], ax[k][c], cx[k][c], smem[c * plane + s], smem[(3 + c) * plane + s], alpha, k2);
+                    E[l] = e;
+                }
+            }
+            __syncthreads();
+            // 2. horizontal box sums
+            for (int l = tid; l < kTileX * EH; l += kThreads) {
+                const float* row = E + (l / kTileX) * EW + l % kTileX;
+                float h = 0.0f;
+                for (int a = 0; a < taps; ++a) h += row[a];
+                Hs[l] = h;
+            }
+            __syncthreads();
+            // 3. vertical box sums, weights, weighted means
+#pragma unroll
+            for (int m = 0; m < 2; ++m) {
+                const int j = threadIdx.y + kThreadsY * m;
+                const int qx = px + dx, qy = y0 + j + dy;
+                if (qx < 0 || qx >= W || qy < 0 || qy >= H) continue;
+                const float* col = Hs + j * kTileX + threadIdx.x;
+                float D = 0.0f;
+                for (int b = 0; b < taps; ++b) D += col[b * kTileX];
+                const float w = __expf(-fmaxf(D * inv_norm, 0.0f));
+                const int s = (qy - sy0) * SW + (qx - sx0);
+                wsum[m] += w;
+#pragma unroll
+                for (int c = 0; c < 3; ++c) acc[m][c] = fmaf(w, smem[c * plane + s], acc[m][c]);
+            }
+        }
+    }
+#pragma unroll
+    for (int m = 0; m < 2; ++m) {
+        const int py = y0 + threadIdx.y + kThreadsY * m;
+        if (px >= W || py >= H) continue;
+        const size_t g = 3 * ((size_t)py * W + px);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) out[g + c] = __fdiv_rn(acc[m][c], wsum[m]);
+    }
+}
+
+// the sums of 3*W*H values over `counts` (per pixel) or `n` samples each -> mu, v (denoise_mean_var)
+__global__ void denoise_convert_kernel(const AccumFx* __restrict__ s1, const AccumFx* __restrict__ s2, const int32_t* __restrict__ counts, uint32_t n,
+                                       long long n_values, float* __restrict__ mean, float* __restrict__ var) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_values) return;
+    denoise_mean_var(s1[i], s2[i], counts ? (uint32_t)counts[i / 3] : n, mean + i, var + i);
+}
+
+__global__ void denoise_tonemap_kernel(const float* __restrict__ x, int32_t* __restrict__ rgb, long long n_values) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_values) rgb[i] = to_rgb_f64((double)x[i]);
+}
+
+}  // namespace rtb
+
+namespace {
+
+template <int NE>
+cudaError_t launch_nlm(const float* mean, const float* var, int W, int H, int r, int f, float k2, float alpha, float inv_norm, float* out,
+                       cudaStream_t stream) {
+    const size_t smem = smem_bytes(r, f);  // at most 116 KB (r = 15, f = 7)
+    cudaError_t e = cudaFuncSetAttribute(denoise_nlm_kernel<NE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    const dim3 grid((unsigned)((W + kTileX - 1) / kTileX), (unsigned)((H + kTileY - 1) / kTileY)), block(kTileX, kThreadsY);
+    denoise_nlm_kernel<NE><<<grid, block, smem, stream>>>(mean, var, W, H, r, f, k2, alpha, inv_norm, out);
+    return cudaGetLastError();
+}
+
+int check_denoise(const RtDenoise* opt, const char* who) {
+    if (!opt) return set_error(RT_ERR_INVALID, "%s: null RtDenoise", who);
+    if (opt->search_radius < 0 || opt->search_radius > RT_DENOISE_MAX_SEARCH_RADIUS || opt->patch_radius < 0 || opt->patch_radius > RT_DENOISE_MAX_PATCH_RADIUS)
+        return set_error(RT_ERR_INVALID, "%s: search_radius must lie in [0, %d] and patch_radius in [0, %d]", who, RT_DENOISE_MAX_SEARCH_RADIUS,
+                         RT_DENOISE_MAX_PATCH_RADIUS);
+    if (!(opt->k > 0.0) || !(opt->alpha >= 0.0)) return set_error(RT_ERR_INVALID, "%s: k must be > 0 and alpha >= 0", who);
+    return RT_OK;
+}
+
+// the filter on device buffers of the current device (arguments checked)
+int denoise(const float* mean, const float* var, int W, int H, const RtDenoise* opt, float* out, cudaStream_t stream) {
+    const int r = opt->search_radius, f = opt->patch_radius;
+    const float k2 = (float)(opt->k * opt->k), alpha = (float)opt->alpha, inv_norm = (float)(1.0 / (3.0 * (2 * f + 1) * (2 * f + 1)));
+    cudaError_t e;
+    switch (locations_per_thread(f)) {
+        case 2: e = launch_nlm<2>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
+        case 3: e = launch_nlm<3>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
+        case 4: e = launch_nlm<4>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
+        case 5: e = launch_nlm<5>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
+        default: e = launch_nlm<6>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
+    }
+    static_assert(locations_per_thread(0) == 2 && locations_per_thread(RT_DENOISE_MAX_PATCH_RADIUS) == 6, "denoise_nlm_kernel instances");
+    if (e != cudaSuccess) return set_error(RT_ERR_CUDA, "denoise: %s", cudaGetErrorString(e));
+    return RT_OK;
+}
+
+bool overlaps(const float* a, const float* b, size_t n) { return a < b + n && b < a + n; }
+
+// device blocks of one denoised render, returned to the device cache on every exit
+struct DenoiseBuffers {
+    AccumFx *accum = nullptr, *moment2 = nullptr;
+    int32_t *samples = nullptr, *rgb = nullptr;
+    float *mean = nullptr, *var = nullptr, *out = nullptr;
+    size_t n_pixels = 0;
+    ~DenoiseBuffers() {
+        cudaStreamSynchronize(0);
+        const size_t n = n_pixels;
+        rtb::cache_free(accum, 3 * n * sizeof(AccumFx)), rtb::cache_free(moment2, 3 * n * sizeof(AccumFx));
+        rtb::cache_free(samples, n * sizeof(int32_t)), rtb::cache_free(rgb, 3 * n * sizeof(int32_t));
+        rtb::cache_free(mean, 3 * n * sizeof(float)), rtb::cache_free(var, 3 * n * sizeof(float)), rtb::cache_free(out, 3 * n * sizeof(float));
+    }
+};
+
+}  // namespace
+
+extern "C" {
+
+int rt_denoise_device(const float* d_mean_rgb, const float* d_var_rgb, int32_t width, int32_t height, const RtDenoise* opt, float* d_out_rgb, int device,
+                      void* stream) {
+    int rc = have_device();
+    if (rc != RT_OK) return rc;
+    if (!d_mean_rgb || !d_var_rgb || !d_out_rgb) return set_error(RT_ERR_INVALID, "rt_denoise_device: null buffer");
+    if (width <= 0 || height <= 0 || height > RT_DENOISE_MAX_HEIGHT)
+        return set_error(RT_ERR_INVALID, "rt_denoise_device: width must be > 0 and height in [1, %d]", RT_DENOISE_MAX_HEIGHT);
+    if ((rc = check_denoise(opt, "rt_denoise_device")) != RT_OK) return rc;
+    const size_t n_values = 3 * (size_t)width * (size_t)height;
+    if (overlaps(d_out_rgb, d_mean_rgb, n_values) || overlaps(d_out_rgb, d_var_rgb, n_values))
+        return set_error(RT_ERR_INVALID, "rt_denoise_device: d_out_rgb overlaps an input");
+    if (device < 0) cudaGetDevice(&device);
+    DeviceGuard g(device);
+    return denoise(d_mean_rgb, d_var_rgb, width, height, opt, d_out_rgb, (cudaStream_t)stream);
+}
+
+int rt_render_denoised(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt, int32_t* rgb,
+                       float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats) {
+    int rc = have_device();
+    if (rc != RT_OK) return rc;
+    if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
+    if ((rc = check_denoise(opt, "rt_render_denoised")) != RT_OK) return rc;
+    if (ad) {
+        if ((rc = check_adaptive(params, ad, "rt_render_denoised")) != RT_OK) return rc;
+    } else {
+        if (params->sample_begin != 0 || params->sample_count != 0)
+            return set_error(RT_ERR_INVALID, "rt_render_denoised: sample_begin and sample_count must be 0 (the render owns the sample range)");
+        if (params->samples_per_pixel < 2) return set_error(RT_ERR_INVALID, "rt_render_denoised: a uniform render needs samples_per_pixel >= 2 (a variance)");
+    }
+    if ((rc = check_pipeline(params)) != RT_OK) return rc;
+    RtScene* scene = const_cast<RtScene*>(scene_);
+    DeviceGuard g(scene->device);
+    cudaStream_t stream = 0;
+    const int W = params->width, H = params->height;
+    const unsigned int npix = (unsigned int)W * (unsigned int)H;
+    const size_t n_values = 3 * (size_t)npix;
+
+    DenoiseBuffers b;
+    b.n_pixels = npix;
+    CU_TRY(rtb::cache_malloc((void**)&b.accum, n_values * sizeof(AccumFx)));
+    CU_TRY(rtb::cache_malloc((void**)&b.moment2, n_values * sizeof(AccumFx)));
+    if (ad) CU_TRY(rtb::cache_malloc((void**)&b.samples, npix * sizeof(int32_t)));
+    CU_TRY(rtb::cache_malloc((void**)&b.rgb, n_values * sizeof(int32_t)));
+    CU_TRY(rtb::cache_malloc((void**)&b.mean, n_values * sizeof(float)));
+    CU_TRY(rtb::cache_malloc((void**)&b.var, n_values * sizeof(float)));
+    CU_TRY(rtb::cache_malloc((void**)&b.out, n_values * sizeof(float)));
+
+    rtb::RowProgress rows{cb, user, H, 0};
+    int launches = 0;
+    uint64_t paths = 0;
+    if (ad) {
+        rc = adaptive_rounds(scene, cam, params, ad, b.accum, b.moment2, b.samples, stream, &rows, &launches, &paths);
+        if (rc != RT_OK) return rc;
+    } else {
+        DCamera dc;
+        make_camera(*cam, dc);
+        CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
+        CU_TRY(cudaEventRecord(scene->ev0, stream));
+        CU_TRY(cudaMemsetAsync(b.accum, 0, n_values * sizeof(AccumFx), stream));
+        CU_TRY(cudaMemsetAsync(b.moment2, 0, n_values * sizeof(AccumFx), stream));
+        rc = launch_persist_moments(scene, dc, params, 0, params->samples_per_pixel, b.accum, b.moment2, nullptr, npix, stream, &launches);
+        if (rc != RT_OK) return rc;
+        paths = (uint64_t)npix * (uint64_t)params->samples_per_pixel;
+    }
+    const unsigned blocks = (unsigned)((n_values + 255) / 256);
+    denoise_convert_kernel<<<blocks, 256, 0, stream>>>(b.accum, b.moment2, b.samples, (uint32_t)params->samples_per_pixel, (long long)n_values, b.mean,
+                                                       b.var);
+    CU_TRY(cudaGetLastError());
+    if ((rc = denoise(b.mean, b.var, W, H, opt, b.out, stream)) != RT_OK) return rc;
+    denoise_tonemap_kernel<<<blocks, 256, 0, stream>>>(b.out, b.rgb, (long long)n_values);
+    CU_TRY(cudaGetLastError());
+    launches += 3;
+    CU_TRY(cudaEventRecord(scene->ev1, stream));
+    if (rgb) CU_TRY(cudaMemcpyAsync(rgb, b.rgb, n_values * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    if (denoised_rgb) CU_TRY(cudaMemcpyAsync(denoised_rgb, b.out, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
+    CU_TRY(cudaStreamSynchronize(stream));
+    rtb::row_progress(1, 1, &rows);  // every row of a uniform render; whatever rows the rounds did not cover
+    if (stats) {
+        std::memset(stats, 0, sizeof *stats);
+        float ms = 0;
+        CU_TRY(cudaEventElapsedTime(&ms, scene->ev0, scene->ev1));
+        unsigned long long rays = 0;
+        CU_TRY(cudaMemcpy(&rays, scene->d_rays, sizeof rays, cudaMemcpyDeviceToHost));
+        stats->paths = paths, stats->rays = rays, stats->device_ms = ms;
+        stats->kernel_launches = launches;
+        stats->pipeline_used = RT_PIPELINE_PERSISTENT;
+        stats->bvh_layout_used = persist_layout_used(scene, params);
+    }
+    return RT_OK;
+}
+
+}  // extern "C"

@@ -90,4 +90,12 @@ int launch_persist_moments(RtScene* s, const DCamera& cam, const RtParams* p, in
                            const uint32_t* d_list, unsigned int n_list, cudaStream_t stream, int* launches);
 int have_device();  // RT_OK, or RT_ERR_NO_DEVICE with the message set
 int validate_render(const RtScene* scene, const RtCamera* cam, const RtParams* p);
+// rt_adaptive.cu: RT_ERR_UNSUPPORTED unless the persistent pipeline; the checks of an RtAdaptive and the sample range
+int check_pipeline(const RtParams* p);
+int check_adaptive(const RtParams* params, const RtAdaptive* ad, const char* who);
+// the rounds of rt_render_adaptive on a validated job: zeroes d_accum / d_moment2 (3*W*H) and leaves each pixel's sums and its
+// count (d_samples, W*H) on the device; records scene->ev0 before the first launch, reports rows through `rows`, synchronises
+// `stream` after every round.  Adds to *launches and *paths.
+int adaptive_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, AccumFx* d_accum, AccumFx* d_moment2,
+                    int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths);
 }  // namespace rtb

@@ -236,10 +236,63 @@ class Renderer:  # raytrace.rs:137-198
                       "bvh_layout": stats.bvh_layout_used}
         return rgb, samples, accum, moment2
 
+    def render_denoised(self, noise_threshold=None, min_samples=16, logger=None, **denoise_options):
+        """EXTENSION: a render through the moments family, then the variance-guided non-local-means filter (rt_render_denoised).
+        noise_threshold None: a uniform render of parameters.samples_per_pixel (>= 2); else adaptive sampling as in
+        render_adaptive.  denoise_options: search_radius, patch_radius, k, alpha (see `denoise`).  Returns (rgb int32
+        [H,W,3], to_rgb of the filtered means; denoised float32 [H,W,3], the filtered means), row 0 at the bottom."""
+        p = self._params()
+        h, w = p.height, p.width
+        rgb = np.empty((h, w, 3), dtype=np.int32)
+        out = np.empty((h, w, 3), dtype=np.float32)
+        ad = None
+        if noise_threshold is not None:
+            ad = abi.RtAdaptive()
+            ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
+        cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
+        stats = abi.RtStats()
+        abi.check(abi.load().rt_render_denoised(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None,
+                                                C.byref(denoise_options_struct(**denoise_options)), rgb.ctypes.data, out.ctypes.data,
+                                                cb, None, C.byref(stats)))
+        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
+                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
+                      "bvh_layout": stats.bvh_layout_used}
+        return rgb, out
+
     def render(self, logger=None):
         """Renderer::render: H rows of W (r, g, b) tuples, row j = 0 at the BOTTOM; logger(j, H) called H times."""
         rgb, _ = self.render_arrays(logger, want_accum=False)
         return [[tuple(int(c) for c in px) for px in row] for row in rgb]
+
+
+def denoise_options_struct(search_radius=abi.RT_DENOISE_DEFAULT_SEARCH_RADIUS, patch_radius=abi.RT_DENOISE_DEFAULT_PATCH_RADIUS,
+                           k=abi.RT_DENOISE_DEFAULT_K, alpha=abi.RT_DENOISE_DEFAULT_ALPHA):
+    """the RtDenoise of the keyword arguments (defaults: the header's RT_DENOISE_DEFAULT_*)"""
+    opt = abi.RtDenoise()
+    opt.search_radius, opt.patch_radius, opt.k, opt.alpha = int(search_radius), int(patch_radius), float(k), float(alpha)
+    return opt
+
+
+def denoise(mean, var, search_radius=abi.RT_DENOISE_DEFAULT_SEARCH_RADIUS, patch_radius=abi.RT_DENOISE_DEFAULT_PATCH_RADIUS,
+            k=abi.RT_DENOISE_DEFAULT_K, alpha=abi.RT_DENOISE_DEFAULT_ALPHA):
+    """EXTENSION: the variance-guided non-local-means filter (rt_denoise_device) of a mean image and the variance of each mean,
+    both contiguous CUDA float32 tensors [H, W, 3] on one device.  search_radius r: the window of candidates [-r, r]^2;
+    patch_radius f: patches of (2f + 1)^2 pixels; k > 0: strength; alpha >= 0: how much of the variance the patch distance
+    cancels.  Returns a new tensor [H, W, 3], computed on the tensors' device and ordered on its current stream."""
+    import torch
+    if not (isinstance(mean, torch.Tensor) and isinstance(var, torch.Tensor)):
+        raise TypeError("denoise: mean and var must be torch tensors")
+    if mean.dtype != torch.float32 or var.dtype != torch.float32 or not mean.is_cuda or var.device != mean.device:
+        raise ValueError("denoise: mean and var must be float32 CUDA tensors on one device")
+    if mean.dim() != 3 or mean.shape[2] != 3 or var.shape != mean.shape:
+        raise ValueError("denoise: mean and var must have the shape [H, W, 3]")
+    mean, var = mean.contiguous(), var.contiguous()
+    out = torch.empty_like(mean)
+    stream = torch.cuda.current_stream(mean.device).cuda_stream
+    abi.check(abi.load().rt_denoise_device(mean.data_ptr(), var.data_ptr(), mean.shape[1], mean.shape[0],
+                                           C.byref(denoise_options_struct(search_radius, patch_radius, k, alpha)), out.data_ptr(),
+                                           mean.device.index, stream))
+    return out
 
 
 def to_ppm(rgb):

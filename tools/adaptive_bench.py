@@ -52,6 +52,49 @@ def gpu_info():
     return name, power
 
 
+def setup(world_name):
+    """(world, scene, camera) of a square job of the world at its own camera"""
+    import support as S
+    world = rt.World(world_name)
+    scene = rt.Scene(world.build(42))
+    info = world.camera()
+    return world, scene, S.make_camera(info["lookfrom"], info["lookat"], info["field_of_view"], 1.0)
+
+
+def params(W, H, spp, seed=42, begin=0, count=0):
+    p = abi.RtParams()
+    p.width, p.height, p.samples_per_pixel, p.max_depth, p.seed = W, H, spp, 50, seed
+    p.sample_begin, p.sample_count, p.pipeline, p.device = begin, count, abi.RT_PIPELINE_AUTO, -1
+    return p
+
+
+def render_uniform(scene, cam, s1, s2, spp, seed=42, moments=True):
+    """a uniform render of spp samples into the zeroed device sums s1, s2 (int64 tensors [H, W, 3]); returns RtStats"""
+    import torch
+    H, W = s1.shape[:2]
+    lib = abi.load()
+    s1.zero_(), s2.zero_()
+    st = abi.RtStats()
+    if moments:
+        abi.check(lib.rt_render_moments_fixed_device(scene.handle, C.byref(cam.c), C.byref(params(W, H, spp, seed)), s1.data_ptr(), s2.data_ptr(), None,
+                                                     C.byref(st)))
+    else:
+        abi.check(lib.rt_render_accumulate_fixed_device(scene.handle, C.byref(cam.c), C.byref(params(W, H, spp, seed)), s1.data_ptr(), None, C.byref(st)))
+    torch.cuda.synchronize()
+    return st
+
+
+def display(mean):
+    """the displayed value of a radiance: gamma 2 of the clamped mean"""
+    return np.sqrt(np.clip(np.asarray(mean, np.float64), 0.0, 1.0))
+
+
+def display_errors(mean, gt):
+    """50th / 95th / 99th percentile over the pixels of the largest channel's display error against gt = display(truth)"""
+    e = np.abs(display(mean) - gt).max(axis=2)
+    return [float(np.percentile(e, q)) for q in (50, 95, 99)]
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out")
@@ -59,7 +102,6 @@ def main():
     ap.add_argument("--quick", action="store_true", help="small sizes (a rehearsal, not a measurement)")
     args = ap.parse_args()
     import torch
-    import support as S
     lib = abi.load()
     if lib.rt_device_count() < 1:
         raise SystemExit("adaptive_bench needs a CUDA device")
@@ -68,31 +110,13 @@ def main():
     for key, world_name, size, cap, job_spp, gt_spp, thresholds in CONFIGS:
         if args.quick:
             size, cap, job_spp, gt_spp = 96, 64, 32, 256
-        world = rt.World(world_name)
-        scene = rt.Scene(world.build(42))
-        info = world.camera()
-        cam = S.make_camera(info["lookfrom"], info["lookat"], info["field_of_view"], 1.0)
+        world, scene, cam = setup(world_name)
         W = H = size
-
-        def params(spp, seed=42, begin=0, count=0):
-            p = abi.RtParams()
-            p.width, p.height, p.samples_per_pixel, p.max_depth, p.seed = W, H, spp, 50, seed
-            p.sample_begin, p.sample_count, p.pipeline, p.device = begin, count, abi.RT_PIPELINE_AUTO, -1
-            return p
-
         s1 = torch.zeros(H, W, 3, dtype=torch.int64, device="cuda")
         s2 = torch.zeros_like(s1)
 
         def uniform(spp, seed=42, moments=True):
-            s1.zero_(), s2.zero_()
-            st = abi.RtStats()
-            if moments:
-                abi.check(lib.rt_render_moments_fixed_device(scene.handle, C.byref(cam.c), C.byref(params(spp, seed)), s1.data_ptr(), s2.data_ptr(), None,
-                                                             C.byref(st)))
-            else:
-                abi.check(lib.rt_render_accumulate_fixed_device(scene.handle, C.byref(cam.c), C.byref(params(spp, seed)), s1.data_ptr(), None, C.byref(st)))
-            torch.cuda.synchronize()
-            return st
+            return render_uniform(scene, cam, s1, s2, spp, seed, moments)
 
         # (a) cost of the family on a uniform job
         uniform(min(job_spp, 16)), uniform(min(job_spp, 16), moments=False)  # warm-up: module load, grid sizing
@@ -107,12 +131,10 @@ def main():
                 "ptxas_product": ptxas_usage(prod_inst), "ptxas_moments": ptxas_usage(mom_inst)}
         # (b) what adaptivity buys
         uniform(gt_spp, seed=7)
-        gt = np.sqrt(np.clip(s1.cpu().numpy().view(np.uint64).astype(np.float64) * 2.0 ** -32 / gt_spp, 0.0, 1.0))
+        gt = display(s1.cpu().numpy().view(np.uint64).astype(np.float64) * 2.0 ** -32 / gt_spp)
 
         def errors(acc, n):
-            disp = np.sqrt(np.clip(acc.astype(np.float64) * 2.0 ** -32 / n, 0.0, 1.0))
-            e = np.abs(disp - gt).max(axis=2)
-            return [float(np.percentile(e, q)) for q in (50, 95, 99)]
+            return display_errors(acc.astype(np.float64) * 2.0 ** -32 / n, gt)
 
         runs = []
         for t in thresholds:

@@ -347,6 +347,56 @@ int rt_render_denoised(const RtScene* scene, const RtCamera* cam, const RtParams
                        const RtDenoise* opt, int32_t* rgb, float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats);
 
 /*
+ * EXTENSION: a feature-guided mode of the denoiser above.  The form follows Rousselle, Knaus & Zwicker, "Robust Denoising
+ * using Feature and Color Information" (Pacific Graphics 2013); it was not checked against the paper's text.
+ *
+ * Features: the albedo and the normal at the FIRST EVENT of each path, which the render computes with the same Philox
+ * draws (camera ray, then the medium event, then the closest surface below it through the render's tree layout):
+ *   surface, Lambertian / metal / diffuse light: albedo = the material's colour (texture value or albedo), each channel
+ *     clamped to [0, 1]; normal = the face-forwarded world normal (RtHit.normal)
+ *   surface, dielectric: albedo (1, 1, 1); normal as above.  (Glass is a first event: what lies behind it is not guided.)
+ *   medium event: albedo = the isotropic material's colour at the event; normal (0, 0, 0).  Media are not transparent.
+ *   miss: albedo = the background colour of the ray; normal (0, 0, 0)
+ * Per pixel and channel over n samples: the mean m and the variance of the mean s = max(0, (sum f^2 - n m^2) / (n - 1)) / n,
+ * s = 0 for n = 1 (f64, each rounded once to f32).
+ *
+ * Guided filter: the weight of candidate q for pixel p becomes
+ *   w(p, q) = min(w_colour(p, q), exp(-max(0, d_albedo(p, q))), exp(-max(0, d_normal(p, q))))
+ * with w_colour the weight of rt_denoise_device, and per feature, with g_c(p)^2 the squared central-difference gradient of the
+ * channel's mean at p (neighbours clamped to the image):
+ *   g_c(p)^2 = ((m_c(x+1,y) - m_c(x-1,y)) / 2)^2 + ((m_c(x,y+1) - m_c(x,y-1)) / 2)^2
+ *   d(p, q)  = (1/3) sum_c [(m_c(p) - m_c(q))^2 - (s_c(p) + min(s_c(p), s_c(q)))] / (k_feature^2 max(tau, s_c(p), g_c(p)^2))
+ * Feature distances are per pixel, not per patch.  Where every feature weight is 1 (constant features of zero variance, or a
+ * k_feature whose square exceeds the f32 range) the output is rt_denoise_device's bit for bit.  Radii and bounds are those of
+ * RtDenoise: the features are read through the cache, not staged in shared memory.
+ *
+ * rt_render_features_device: the features of samples [sample_begin, sample_begin + count) of every pixel (count =
+ * sample_count, or samples_per_pixel - sample_begin when 0) into four device buffers of 3*W*H floats on the scene's device,
+ * [H][W][3], row 0 at the bottom; the outputs must not overlap.  Deterministic; asynchronous on `stream` unless stats is given
+ * (device_ms of the pass).
+ * rt_denoise_guided_device: rt_denoise_device with the four feature buffers; d_out_rgb must not overlap an input.
+ * rt_render_denoised_guided: rt_render_denoised, plus the features of samples [0, guide->feature_samples) of the same seed and
+ * the guided filter; stats->device_ms includes the feature pass.
+ */
+#define RT_GUIDE_DEFAULT_K_FEATURE 1.0 /* set by the sweep of DESIGN.md section 5f */
+#define RT_GUIDE_DEFAULT_TAU 1e-2
+#define RT_GUIDE_DEFAULT_FEATURE_SAMPLES 16
+typedef struct RtGuide {
+    double k_feature;        /* > 0: larger lets more across feature edges */
+    double tau;              /* > 0 and finite: the floor of the feature's normalisation */
+    int32_t feature_samples; /* >= 1; used by rt_render_denoised_guided only */
+    int32_t reserved;
+} RtGuide;
+int rt_render_features_device(const RtScene* scene, const RtCamera* cam, const RtParams* params, float* d_albedo,
+                              float* d_albedo_var, float* d_normal, float* d_normal_var, void* stream, RtStats* stats);
+int rt_denoise_guided_device(const float* d_mean_rgb, const float* d_var_rgb, const float* d_albedo, const float* d_albedo_var,
+                             const float* d_normal, const float* d_normal_var, int32_t width, int32_t height,
+                             const RtDenoise* opt, const RtGuide* guide, float* d_out_rgb, int device, void* stream);
+int rt_render_denoised_guided(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* adaptive,
+                              const RtDenoise* opt, const RtGuide* guide, int32_t* rgb, float* denoised_rgb, RtProgressFn cb,
+                              void* user, RtStats* stats);
+
+/*
  * rt_render over several GPUs of one process (the reference's row-parallel rayon loop, raytrace.rs:176-185, becomes
  * sample slices): scenes[g] is the same description created on a distinct device; device g renders every pixel for
  * the g-th slice of the sample range (rt_sample_slice), the float accumulation buffers are summed onto scenes[0]'s

@@ -168,6 +168,27 @@ impl Default for RtDenoise {
         }
     }
 }
+/// EXTENSION: feature-guided denoising (rt_render_features_device, rt_denoise_guided_device, rt_render_denoised_guided)
+#[repr(C)]
+pub struct RtGuide {
+    pub k_feature: f64,
+    pub tau: f64,
+    pub feature_samples: i32,
+    pub reserved: i32,
+}
+pub const RT_GUIDE_DEFAULT_K_FEATURE: f64 = 1.0;
+pub const RT_GUIDE_DEFAULT_TAU: f64 = 1e-2;
+pub const RT_GUIDE_DEFAULT_FEATURE_SAMPLES: i32 = 16;
+impl Default for RtGuide {
+    fn default() -> RtGuide {
+        RtGuide {
+            k_feature: RT_GUIDE_DEFAULT_K_FEATURE,
+            tau: RT_GUIDE_DEFAULT_TAU,
+            feature_samples: RT_GUIDE_DEFAULT_FEATURE_SAMPLES,
+            reserved: 0,
+        }
+    }
+}
 pub enum RtScene {}
 /// Called once per image row j = 0 .. total-1, in increasing order, on the calling thread (include/rt_b200.h).
 pub type RtProgressFn = Option<extern "C" fn(row: c_int, total: c_int, user: *mut c_void)>;
@@ -193,6 +214,14 @@ extern "C" {
                              device: c_int, stream: *mut c_void) -> c_int;
     pub fn rt_render_denoised(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive, opt: *const RtDenoise,
                               rgb: *mut i32, denoised_rgb: *mut f32, cb: RtProgressFn, user: *mut c_void, stats: *mut RtStats) -> c_int;
+    pub fn rt_render_features_device(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, d_albedo: *mut f32, d_albedo_var: *mut f32,
+                                     d_normal: *mut f32, d_normal_var: *mut f32, stream: *mut c_void, stats: *mut RtStats) -> c_int;
+    pub fn rt_denoise_guided_device(d_mean_rgb: *const f32, d_var_rgb: *const f32, d_albedo: *const f32, d_albedo_var: *const f32,
+                                    d_normal: *const f32, d_normal_var: *const f32, width: i32, height: i32, opt: *const RtDenoise,
+                                    guide: *const RtGuide, d_out_rgb: *mut f32, device: c_int, stream: *mut c_void) -> c_int;
+    pub fn rt_render_denoised_guided(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive,
+                                     opt: *const RtDenoise, guide: *const RtGuide, rgb: *mut i32, denoised_rgb: *mut f32, cb: RtProgressFn,
+                                     user: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_world_build(name: *const c_char, seed: u64, earth_rgb: *const u8, earth_w: i32, earth_h: i32, out: *mut *mut RtSceneDesc,
                           n_draws: *mut u64) -> c_int;
     pub fn rt_scene_desc_free(desc: *mut RtSceneDesc);

@@ -103,6 +103,13 @@ RT_DENOISE_DEFAULT_SEARCH_RADIUS, RT_DENOISE_DEFAULT_PATCH_RADIUS, RT_DENOISE_DE
 RT_DENOISE_MAX_SEARCH_RADIUS, RT_DENOISE_MAX_PATCH_RADIUS, RT_DENOISE_MAX_HEIGHT = 15, 7, 1048560
 
 
+class RtGuide(C.Structure):  # EXTENSION: feature-guided denoising (rt_denoise_guided_device, rt_render_denoised_guided)
+    _fields_ = [("k_feature", C.c_double), ("tau", C.c_double), ("feature_samples", C.c_int32), ("reserved", C.c_int32)]
+
+
+RT_GUIDE_DEFAULT_K_FEATURE, RT_GUIDE_DEFAULT_TAU, RT_GUIDE_DEFAULT_FEATURE_SAMPLES = 1.0, 1e-2, 16
+
+
 class RtWorldInfo(C.Structure):
     _fields_ = [("lookfrom", C.c_double * 3), ("lookat", C.c_double * 3), ("vfov_deg", C.c_double),
                 ("background_kind", C.c_int32), ("needs_earthmap", C.c_int32), ("uses_rng", C.c_int32)]
@@ -138,6 +145,13 @@ PROTOTYPES = {
     "rt_denoise_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(RtDenoise), C.c_void_p, C.c_int, C.c_void_p]),
     "rt_render_denoised": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtDenoise),
                                      C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
+    "rt_render_features_device": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.POINTER(RtStats)]),
+    "rt_denoise_guided_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                           C.POINTER(RtDenoise), C.POINTER(RtGuide), C.c_void_p, C.c_int, C.c_void_p]),
+    "rt_render_denoised_guided": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive),
+                                            C.POINTER(RtDenoise), C.POINTER(RtGuide), C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p,
+                                            C.POINTER(RtStats)]),
     "rt_tonemap_fixed_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int, C.c_void_p]),
     "rt_accum_fixed_to_float_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rt_release_cached_memory": (None, []),

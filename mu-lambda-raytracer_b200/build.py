@@ -67,7 +67,7 @@ def build(force=False, verbose=False):
             if verbose and out:
                 print(out)
         objs.append(o)
-    for src in ("rt_api.cu", "rt_wavefront.cu", "rt_persist.cu", "rt_multi.cu", "rt_peaks.cu", "rt_lbvh.cu", "dev_cache.cu", "rt_adaptive.cu", "rt_denoise.cu"):
+    for src in ("rt_api.cu", "rt_wavefront.cu", "rt_persist.cu", "rt_multi.cu", "rt_peaks.cu", "rt_lbvh.cu", "dev_cache.cu", "rt_adaptive.cu", "rt_denoise.cu", "rt_features.cu"):
         cu = os.path.join(CSRC, src)
         cuo = os.path.join(bdir, src + ".o")
         if force or _newer(cuo, [cu] + headers):

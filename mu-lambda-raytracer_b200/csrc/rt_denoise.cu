@@ -11,6 +11,12 @@
 // Two barriers per offset; no atomics, and every sum runs in a fixed order, so the output is reproducible bit for bit.
 // d = 0 has weight 1 and is not evaluated; an offset that puts every candidate of the tile outside the image is skipped.
 //
+// denoise_nlm_guided_kernel (rt_denoise_guided_device): the same body (nlm_body) with step 3's weight bounded by the feature
+// weight of the candidate (guide_weight).  Each thread keeps the features and per-channel scales of its two output pixels in
+// registers and reads the candidates' features through L1 (__ldg), so the shared memory and the radius bounds are those of
+// the colour-only filter.  The colour-only instances are compiled from the same body with the feature code removed at compile
+// time; their instructions are unchanged.
+//
 // rt_render_denoised renders through the moments family (rt_adaptive.cu), converts the sums (denoise_mean_var), filters and
 // tonemaps.
 #include <cuda_runtime.h>
@@ -24,6 +30,14 @@
 #include "scene_internal.h"
 
 using namespace rtb;
+
+namespace rtb {
+// The feature buffers of the guided filter (f32 [H][W][3] each) and its constants (a kernel parameter)
+struct GuideIn {
+    const float *albedo, *albedo_var, *normal, *normal_var;
+    float kf2_3, tau;  // 3 k_f^2, tau
+};
+}  // namespace rtb
 
 namespace {
 
@@ -40,13 +54,52 @@ size_t smem_bytes(int r, int f) {
 
 __device__ __forceinline__ int clampi(int x, int hi) { return x < 0 ? 0 : (x > hi ? hi : x); }
 
+// mean m, variance of the mean s and scale (guide_scale) of both features at pixel (x, y)
+struct GuideAt {
+    float m[2][3], s[2][3], scale[2][3];
+};
+
+__device__ __forceinline__ void guide_load(const GuideIn& g, size_t i, float m[2][3], float s[2][3]) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+        m[0][c] = __ldg(g.albedo + 3 * i + c), s[0][c] = __ldg(g.albedo_var + 3 * i + c), m[1][c] = __ldg(g.normal + 3 * i + c),
+        s[1][c] = __ldg(g.normal_var + 3 * i + c);
+}
+
+__device__ __forceinline__ GuideAt guide_at(const GuideIn& g, int W, int H, int x, int y) {
+    GuideAt a;
+    guide_load(g, (size_t)y * W + x, a.m, a.s);
+    const size_t xl = (size_t)y * W + clampi(x - 1, W - 1), xr = (size_t)y * W + clampi(x + 1, W - 1);
+    const size_t yd = (size_t)clampi(y - 1, H - 1) * W + x, yu = (size_t)clampi(y + 1, H - 1) * W + x;
+    const float* planes[2] = {g.albedo, g.normal};
+#pragma unroll
+    for (int j = 0; j < 2; ++j)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const float* m = planes[j];
+            const float gx = 0.5f * (__ldg(m + 3 * xr + c) - __ldg(m + 3 * xl + c)), gy = 0.5f * (__ldg(m + 3 * yu + c) - __ldg(m + 3 * yd + c));
+            a.scale[j][c] = guide_scale(a.s[j][c], gx, gy, g.kf2_3, g.tau);
+        }
+    return a;
+}
+
+// the feature weight of candidate q for the output pixel described by p: min over the features of exp(-max(0, d_j))
+__device__ __forceinline__ float guide_weight(const GuideIn& g, int W, const GuideAt& p, int qx, int qy) {
+    float m[2][3], s[2][3];
+    guide_load(g, (size_t)qy * W + qx, m, s);
+    const float d = fmaxf(guide_distance(p.m[0], p.s[0], p.scale[0], m[0], s[0]), guide_distance(p.m[1], p.s[1], p.scale[1], m[1], s[1]));
+    return __expf(-fmaxf(d, 0.0f));
+}
+
 }  // namespace
 
 namespace rtb {  // kernels with stable names (profiles)
 
-template <int NE>
-__global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const float* __restrict__ mean, const float* __restrict__ var, int W, int H, int r, int f,
-                                                               float k2, float alpha, float inv_norm, float* __restrict__ out) {
+// The body of both filters.  GUIDED adds the feature weight to step 3 and nothing else: the sums keep their order, so with
+// feature weights of 1 the output is the colour-only filter's bit for bit.
+template <int NE, bool GUIDED>
+__device__ __forceinline__ void nlm_body(const float* __restrict__ mean, const float* __restrict__ var, int W, int H, int r, int f, float k2, float alpha,
+                                         float inv_norm, float* __restrict__ out, const GuideIn& gd) {
     extern __shared__ float smem[];
     const int R = r + f;
     const int SW = kTileX + 2 * R, SH = kTileY + 2 * R, plane = SW * SH;
@@ -90,6 +143,11 @@ __global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const float* __re
 #pragma unroll
         for (int c = 0; c < 3; ++c) acc[m][c] = smem[c * plane + s];
     }
+    GuideAt gp[GUIDED ? 2 : 1];
+    if constexpr (GUIDED) {
+#pragma unroll
+        for (int m = 0; m < 2; ++m) gp[m] = guide_at(gd, W, H, clampi(px, W - 1), clampi(y0 + threadIdx.y + kThreadsY * m, H - 1));
+    }
 
     const int taps = 2 * f + 1;
     for (int dy = -r; dy <= r; ++dy) {
@@ -127,7 +185,8 @@ __global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const float* __re
                 const float* col = Hs + j * kTileX + threadIdx.x;
                 float D = 0.0f;
                 for (int b = 0; b < taps; ++b) D += col[b * kTileX];
-                const float w = __expf(-fmaxf(D * inv_norm, 0.0f));
+                float w = __expf(-fmaxf(D * inv_norm, 0.0f));
+                if constexpr (GUIDED) w = fminf(w, guide_weight(gd, W, gp[m], qx, qy));
                 const int s = (qy - sy0) * SW + (qx - sx0);
                 wsum[m] += w;
 #pragma unroll
@@ -143,6 +202,18 @@ __global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const float* __re
 #pragma unroll
         for (int c = 0; c < 3; ++c) out[g + c] = __fdiv_rn(acc[m][c], wsum[m]);
     }
+}
+
+template <int NE>
+__global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const float* __restrict__ mean, const float* __restrict__ var, int W, int H, int r, int f,
+                                                               float k2, float alpha, float inv_norm, float* __restrict__ out) {
+    nlm_body<NE, false>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, GuideIn{});
+}
+
+template <int NE>
+__global__ void __launch_bounds__(kThreads) denoise_nlm_guided_kernel(const float* __restrict__ mean, const float* __restrict__ var, int W, int H, int r,
+                                                                      int f, float k2, float alpha, float inv_norm, float* __restrict__ out, GuideIn g) {
+    nlm_body<NE, true>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, g);
 }
 
 // the sums of 3*W*H values over `counts` (per pixel) or `n` samples each -> mu, v (denoise_mean_var)
@@ -164,12 +235,14 @@ namespace {
 
 template <int NE>
 cudaError_t launch_nlm(const float* mean, const float* var, int W, int H, int r, int f, float k2, float alpha, float inv_norm, float* out,
-                       cudaStream_t stream) {
-    const size_t smem = smem_bytes(r, f);  // at most 116 KB (r = 15, f = 7)
-    cudaError_t e = cudaFuncSetAttribute(denoise_nlm_kernel<NE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                       const GuideIn* guide, cudaStream_t stream) {
+    const size_t smem = smem_bytes(r, f);  // at most 116 KB (r = 15, f = 7); the guided filter reads the features through L1
+    const void* kernel = guide ? (const void*)denoise_nlm_guided_kernel<NE> : (const void*)denoise_nlm_kernel<NE>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const dim3 grid((unsigned)((W + kTileX - 1) / kTileX), (unsigned)((H + kTileY - 1) / kTileY)), block(kTileX, kThreadsY);
-    denoise_nlm_kernel<NE><<<grid, block, smem, stream>>>(mean, var, W, H, r, f, k2, alpha, inv_norm, out);
+    if (guide) denoise_nlm_guided_kernel<NE><<<grid, block, smem, stream>>>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, *guide);
+    else denoise_nlm_kernel<NE><<<grid, block, smem, stream>>>(mean, var, W, H, r, f, k2, alpha, inv_norm, out);
     return cudaGetLastError();
 }
 
@@ -182,17 +255,25 @@ int check_denoise(const RtDenoise* opt, const char* who) {
     return RT_OK;
 }
 
-// the filter on device buffers of the current device (arguments checked)
-int denoise(const float* mean, const float* var, int W, int H, const RtDenoise* opt, float* out, cudaStream_t stream) {
+int check_guide(const RtGuide* guide, bool render, const char* who) {
+    if (!guide) return set_error(RT_ERR_INVALID, "%s: null RtGuide", who);
+    if (!(guide->k_feature > 0.0) || !(guide->tau > 0.0) || std::isinf(guide->tau))
+        return set_error(RT_ERR_INVALID, "%s: k_feature must be > 0 and tau finite and > 0", who);
+    if (render && guide->feature_samples < 1) return set_error(RT_ERR_INVALID, "%s: feature_samples must be >= 1", who);
+    return RT_OK;
+}
+
+// the filter on device buffers of the current device (arguments checked); guide: the feature-guided instance
+int denoise(const float* mean, const float* var, int W, int H, const RtDenoise* opt, float* out, cudaStream_t stream, const GuideIn* guide = nullptr) {
     const int r = opt->search_radius, f = opt->patch_radius;
     const float k2 = (float)(opt->k * opt->k), alpha = (float)opt->alpha, inv_norm = (float)(1.0 / (3.0 * (2 * f + 1) * (2 * f + 1)));
     cudaError_t e;
     switch (locations_per_thread(f)) {
-        case 2: e = launch_nlm<2>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
-        case 3: e = launch_nlm<3>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
-        case 4: e = launch_nlm<4>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
-        case 5: e = launch_nlm<5>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
-        default: e = launch_nlm<6>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, stream); break;
+        case 2: e = launch_nlm<2>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
+        case 3: e = launch_nlm<3>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
+        case 4: e = launch_nlm<4>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
+        case 5: e = launch_nlm<5>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
+        default: e = launch_nlm<6>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
     }
     static_assert(locations_per_thread(0) == 2 && locations_per_thread(RT_DENOISE_MAX_PATCH_RADIUS) == 6, "denoise_nlm_kernel instances");
     if (e != cudaSuccess) return set_error(RT_ERR_CUDA, "denoise: %s", cudaGetErrorString(e));
@@ -201,11 +282,16 @@ int denoise(const float* mean, const float* var, int W, int H, const RtDenoise* 
 
 bool overlaps(const float* a, const float* b, size_t n) { return a < b + n && b < a + n; }
 
+GuideIn guide_in(const float* albedo, const float* albedo_var, const float* normal, const float* normal_var, const RtGuide* guide) {
+    return GuideIn{albedo, albedo_var, normal, normal_var, (float)(3.0 * guide->k_feature * guide->k_feature), (float)guide->tau};
+}
+
 // device blocks of one denoised render, returned to the device cache on every exit
 struct DenoiseBuffers {
     AccumFx *accum = nullptr, *moment2 = nullptr;
     int32_t *samples = nullptr, *rgb = nullptr;
     float *mean = nullptr, *var = nullptr, *out = nullptr;
+    float* feat[4] = {nullptr, nullptr, nullptr, nullptr};  // albedo, albedo_var, normal, normal_var (guided)
     size_t n_pixels = 0;
     ~DenoiseBuffers() {
         cudaStreamSynchronize(0);
@@ -213,8 +299,99 @@ struct DenoiseBuffers {
         rtb::cache_free(accum, 3 * n * sizeof(AccumFx)), rtb::cache_free(moment2, 3 * n * sizeof(AccumFx));
         rtb::cache_free(samples, n * sizeof(int32_t)), rtb::cache_free(rgb, 3 * n * sizeof(int32_t));
         rtb::cache_free(mean, 3 * n * sizeof(float)), rtb::cache_free(var, 3 * n * sizeof(float)), rtb::cache_free(out, 3 * n * sizeof(float));
+        for (float* b : feat) rtb::cache_free(b, 3 * n * sizeof(float));
     }
 };
+
+// rt_render_denoised (guide == nullptr) and rt_render_denoised_guided
+int render_denoised(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt, const RtGuide* guide,
+                    int32_t* rgb, float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats, const char* who) {
+    int rc = have_device();
+    if (rc != RT_OK) return rc;
+    if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
+    if ((rc = check_denoise(opt, who)) != RT_OK) return rc;
+    if (guide && (rc = check_guide(guide, true, who)) != RT_OK) return rc;
+    if (ad) {
+        if ((rc = check_adaptive(params, ad, who)) != RT_OK) return rc;
+    } else {
+        if (params->sample_begin != 0 || params->sample_count != 0)
+            return set_error(RT_ERR_INVALID, "%s: sample_begin and sample_count must be 0 (the render owns the sample range)", who);
+        if (params->samples_per_pixel < 2) return set_error(RT_ERR_INVALID, "%s: a uniform render needs samples_per_pixel >= 2 (a variance)", who);
+    }
+    if ((rc = check_pipeline(params)) != RT_OK) return rc;
+    RtScene* scene = const_cast<RtScene*>(scene_);
+    DeviceGuard g(scene->device);
+    cudaStream_t stream = 0;
+    const int W = params->width, H = params->height;
+    const unsigned int npix = (unsigned int)W * (unsigned int)H;
+    const size_t n_values = 3 * (size_t)npix;
+
+    DenoiseBuffers b;
+    b.n_pixels = npix;
+    CU_TRY(rtb::cache_malloc((void**)&b.accum, n_values * sizeof(AccumFx)));
+    CU_TRY(rtb::cache_malloc((void**)&b.moment2, n_values * sizeof(AccumFx)));
+    if (ad) CU_TRY(rtb::cache_malloc((void**)&b.samples, npix * sizeof(int32_t)));
+    CU_TRY(rtb::cache_malloc((void**)&b.rgb, n_values * sizeof(int32_t)));
+    CU_TRY(rtb::cache_malloc((void**)&b.mean, n_values * sizeof(float)));
+    CU_TRY(rtb::cache_malloc((void**)&b.var, n_values * sizeof(float)));
+    CU_TRY(rtb::cache_malloc((void**)&b.out, n_values * sizeof(float)));
+    if (guide)
+        for (float*& f : b.feat) CU_TRY(rtb::cache_malloc((void**)&f, n_values * sizeof(float)));
+
+    rtb::RowProgress rows{cb, user, H, 0};
+    int launches = 0;
+    uint64_t paths = 0;
+    if (ad) {
+        rc = adaptive_rounds(scene, cam, params, ad, b.accum, b.moment2, b.samples, stream, &rows, &launches, &paths);
+        if (rc != RT_OK) return rc;
+    } else {
+        DCamera dc;
+        make_camera(*cam, dc);
+        CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
+        CU_TRY(cudaEventRecord(scene->ev0, stream));
+        CU_TRY(cudaMemsetAsync(b.accum, 0, n_values * sizeof(AccumFx), stream));
+        CU_TRY(cudaMemsetAsync(b.moment2, 0, n_values * sizeof(AccumFx), stream));
+        rc = launch_persist_moments(scene, dc, params, 0, params->samples_per_pixel, b.accum, b.moment2, nullptr, npix, stream, &launches);
+        if (rc != RT_OK) return rc;
+        paths = (uint64_t)npix * (uint64_t)params->samples_per_pixel;
+    }
+    if (guide) {
+        RtParams fp = *params;
+        fp.sample_begin = 0, fp.sample_count = guide->feature_samples;
+        if ((rc = launch_features(scene, cam, &fp, b.feat[0], b.feat[1], b.feat[2], b.feat[3], stream)) != RT_OK) return rc;
+        launches += 1;
+    }
+    const unsigned blocks = (unsigned)((n_values + 255) / 256);
+    denoise_convert_kernel<<<blocks, 256, 0, stream>>>(b.accum, b.moment2, b.samples, (uint32_t)params->samples_per_pixel, (long long)n_values, b.mean,
+                                                       b.var);
+    CU_TRY(cudaGetLastError());
+    if (guide) {
+        const GuideIn gi = guide_in(b.feat[0], b.feat[1], b.feat[2], b.feat[3], guide);
+        if ((rc = denoise(b.mean, b.var, W, H, opt, b.out, stream, &gi)) != RT_OK) return rc;
+    } else if ((rc = denoise(b.mean, b.var, W, H, opt, b.out, stream)) != RT_OK) {
+        return rc;
+    }
+    denoise_tonemap_kernel<<<blocks, 256, 0, stream>>>(b.out, b.rgb, (long long)n_values);
+    CU_TRY(cudaGetLastError());
+    launches += 3;
+    CU_TRY(cudaEventRecord(scene->ev1, stream));
+    if (rgb) CU_TRY(cudaMemcpyAsync(rgb, b.rgb, n_values * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    if (denoised_rgb) CU_TRY(cudaMemcpyAsync(denoised_rgb, b.out, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
+    CU_TRY(cudaStreamSynchronize(stream));
+    rtb::row_progress(1, 1, &rows);  // every row of a uniform render; whatever rows the rounds did not cover
+    if (stats) {
+        std::memset(stats, 0, sizeof *stats);
+        float ms = 0;
+        CU_TRY(cudaEventElapsedTime(&ms, scene->ev0, scene->ev1));
+        unsigned long long rays = 0;
+        CU_TRY(cudaMemcpy(&rays, scene->d_rays, sizeof rays, cudaMemcpyDeviceToHost));
+        stats->paths = paths, stats->rays = rays, stats->device_ms = ms;
+        stats->kernel_launches = launches;
+        stats->pipeline_used = RT_PIPELINE_PERSISTENT;
+        stats->bvh_layout_used = persist_layout_used(scene, params);
+    }
+    return RT_OK;
+}
 
 }  // namespace
 
@@ -236,79 +413,40 @@ int rt_denoise_device(const float* d_mean_rgb, const float* d_var_rgb, int32_t w
     return denoise(d_mean_rgb, d_var_rgb, width, height, opt, d_out_rgb, (cudaStream_t)stream);
 }
 
-int rt_render_denoised(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt, int32_t* rgb,
-                       float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats) {
+int rt_denoise_guided_device(const float* d_mean_rgb, const float* d_var_rgb, const float* d_albedo, const float* d_albedo_var, const float* d_normal,
+                             const float* d_normal_var, int32_t width, int32_t height, const RtDenoise* opt, const RtGuide* guide, float* d_out_rgb,
+                             int device, void* stream) {
     int rc = have_device();
     if (rc != RT_OK) return rc;
-    if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
-    if ((rc = check_denoise(opt, "rt_render_denoised")) != RT_OK) return rc;
-    if (ad) {
-        if ((rc = check_adaptive(params, ad, "rt_render_denoised")) != RT_OK) return rc;
-    } else {
-        if (params->sample_begin != 0 || params->sample_count != 0)
-            return set_error(RT_ERR_INVALID, "rt_render_denoised: sample_begin and sample_count must be 0 (the render owns the sample range)");
-        if (params->samples_per_pixel < 2) return set_error(RT_ERR_INVALID, "rt_render_denoised: a uniform render needs samples_per_pixel >= 2 (a variance)");
-    }
-    if ((rc = check_pipeline(params)) != RT_OK) return rc;
-    RtScene* scene = const_cast<RtScene*>(scene_);
-    DeviceGuard g(scene->device);
-    cudaStream_t stream = 0;
-    const int W = params->width, H = params->height;
-    const unsigned int npix = (unsigned int)W * (unsigned int)H;
-    const size_t n_values = 3 * (size_t)npix;
+    const float* in[6] = {d_mean_rgb, d_var_rgb, d_albedo, d_albedo_var, d_normal, d_normal_var};
+    for (const float* p : in)
+        if (!p) return set_error(RT_ERR_INVALID, "rt_denoise_guided_device: null buffer");
+    if (!d_out_rgb) return set_error(RT_ERR_INVALID, "rt_denoise_guided_device: null buffer");
+    if (width <= 0 || height <= 0 || height > RT_DENOISE_MAX_HEIGHT)
+        return set_error(RT_ERR_INVALID, "rt_denoise_guided_device: width must be > 0 and height in [1, %d]", RT_DENOISE_MAX_HEIGHT);
+    if ((rc = check_denoise(opt, "rt_denoise_guided_device")) != RT_OK) return rc;
+    if ((rc = check_guide(guide, false, "rt_denoise_guided_device")) != RT_OK) return rc;
+    const size_t n_values = 3 * (size_t)width * (size_t)height;
+    for (const float* p : in)
+        if (overlaps(d_out_rgb, p, n_values)) return set_error(RT_ERR_INVALID, "rt_denoise_guided_device: d_out_rgb overlaps an input");
+    if (device < 0) cudaGetDevice(&device);
+    DeviceGuard g(device);
+    const GuideIn gi = guide_in(d_albedo, d_albedo_var, d_normal, d_normal_var, guide);
+    return denoise(d_mean_rgb, d_var_rgb, width, height, opt, d_out_rgb, (cudaStream_t)stream, &gi);
+}
 
-    DenoiseBuffers b;
-    b.n_pixels = npix;
-    CU_TRY(rtb::cache_malloc((void**)&b.accum, n_values * sizeof(AccumFx)));
-    CU_TRY(rtb::cache_malloc((void**)&b.moment2, n_values * sizeof(AccumFx)));
-    if (ad) CU_TRY(rtb::cache_malloc((void**)&b.samples, npix * sizeof(int32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.rgb, n_values * sizeof(int32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.mean, n_values * sizeof(float)));
-    CU_TRY(rtb::cache_malloc((void**)&b.var, n_values * sizeof(float)));
-    CU_TRY(rtb::cache_malloc((void**)&b.out, n_values * sizeof(float)));
+int rt_render_denoised(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt, int32_t* rgb,
+                       float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats) {
+    return render_denoised(scene, cam, params, ad, opt, nullptr, rgb, denoised_rgb, cb, user, stats, "rt_render_denoised");
+}
 
-    rtb::RowProgress rows{cb, user, H, 0};
-    int launches = 0;
-    uint64_t paths = 0;
-    if (ad) {
-        rc = adaptive_rounds(scene, cam, params, ad, b.accum, b.moment2, b.samples, stream, &rows, &launches, &paths);
-        if (rc != RT_OK) return rc;
-    } else {
-        DCamera dc;
-        make_camera(*cam, dc);
-        CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
-        CU_TRY(cudaEventRecord(scene->ev0, stream));
-        CU_TRY(cudaMemsetAsync(b.accum, 0, n_values * sizeof(AccumFx), stream));
-        CU_TRY(cudaMemsetAsync(b.moment2, 0, n_values * sizeof(AccumFx), stream));
-        rc = launch_persist_moments(scene, dc, params, 0, params->samples_per_pixel, b.accum, b.moment2, nullptr, npix, stream, &launches);
-        if (rc != RT_OK) return rc;
-        paths = (uint64_t)npix * (uint64_t)params->samples_per_pixel;
+int rt_render_denoised_guided(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,
+                              const RtGuide* guide, int32_t* rgb, float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats) {
+    if (!guide) {  // (render_denoised takes a null guide for the colour-only filter)
+        const int rc = have_device();
+        return rc != RT_OK ? rc : set_error(RT_ERR_INVALID, "rt_render_denoised_guided: null RtGuide");
     }
-    const unsigned blocks = (unsigned)((n_values + 255) / 256);
-    denoise_convert_kernel<<<blocks, 256, 0, stream>>>(b.accum, b.moment2, b.samples, (uint32_t)params->samples_per_pixel, (long long)n_values, b.mean,
-                                                       b.var);
-    CU_TRY(cudaGetLastError());
-    if ((rc = denoise(b.mean, b.var, W, H, opt, b.out, stream)) != RT_OK) return rc;
-    denoise_tonemap_kernel<<<blocks, 256, 0, stream>>>(b.out, b.rgb, (long long)n_values);
-    CU_TRY(cudaGetLastError());
-    launches += 3;
-    CU_TRY(cudaEventRecord(scene->ev1, stream));
-    if (rgb) CU_TRY(cudaMemcpyAsync(rgb, b.rgb, n_values * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
-    if (denoised_rgb) CU_TRY(cudaMemcpyAsync(denoised_rgb, b.out, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
-    CU_TRY(cudaStreamSynchronize(stream));
-    rtb::row_progress(1, 1, &rows);  // every row of a uniform render; whatever rows the rounds did not cover
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        float ms = 0;
-        CU_TRY(cudaEventElapsedTime(&ms, scene->ev0, scene->ev1));
-        unsigned long long rays = 0;
-        CU_TRY(cudaMemcpy(&rays, scene->d_rays, sizeof rays, cudaMemcpyDeviceToHost));
-        stats->paths = paths, stats->rays = rays, stats->device_ms = ms;
-        stats->kernel_launches = launches;
-        stats->pipeline_used = RT_PIPELINE_PERSISTENT;
-        stats->bvh_layout_used = persist_layout_used(scene, params);
-    }
-    return RT_OK;
+    return render_denoised(scene, cam, params, ad, opt, guide, rgb, denoised_rgb, cb, user, stats, "rt_render_denoised_guided");
 }
 
 }  // extern "C"

@@ -16,7 +16,11 @@
 #define RTD_DDIV __ddiv_rn
 #define RTD_F32 __double2float_rn
 #define RTD_FDIV __fdividef  // x * MUFU.RCP(y): the library builds without --use_fast_math, so the approximation is explicit
+#define RTD_DADD __dadd_rn
+#define RTD_FRCP __frcp_rn
 #else
+#define RTD_DADD(a, b) ((double)(a) + (double)(b))
+#define RTD_FRCP(a) (1.0f / (a))
 #define RTD_DEV inline
 #define RTD_DMUL(a, b) ((double)(a) * (double)(b))
 #define RTD_DSUB(a, b) ((double)(a) - (double)(b))
@@ -55,6 +59,49 @@ RTD_DEV float denoise_term(float mu_x, float v_x, float ax, float cx, float mu_y
     const float d = mu_x - mu_y;
     const float num = fmaf(-alpha, fminf(v_x, v_y), fmaf(d, d, -ax));
     return RTD_FDIV(num, fmaf(k2, v_y, cx));
+}
+
+// ---- feature guidance (rt_features.cu, rt_denoise_guided_device)
+
+// One sample f of one feature channel added to its f64 sums: s1 += f, s2 += f^2 (each operation rounded on its own)
+RTD_DEV void feature_accumulate(double* s1, double* s2, float f) {
+    *s1 = RTD_DADD(*s1, (double)f);
+    *s2 = RTD_DADD(*s2, RTD_DMUL((double)f, (double)f));
+}
+
+// Mean and variance of the mean of one feature channel from its f64 sums over n >= 1 samples, each rounded once to f32:
+//   mu = s1 / n,   v = max(0, (s2 - n mu^2) / (n - 1)) / n,   v = 0 for n = 1
+RTD_DEV void feature_mean_var(double s1, double s2, uint32_t n, float* mu_out, float* v_out) {
+    const double dn = (double)n;
+    const double mu = RTD_DDIV(s1, dn);
+    double var = 0.0;
+    if (n > 1) {
+        var = RTD_DDIV(RTD_DSUB(s2, RTD_DMUL(dn, RTD_DMUL(mu, mu))), RTD_DSUB(dn, 1.0));
+        var = var > 0.0 ? var : 0.0;
+    }
+    *mu_out = RTD_F32(mu);
+    *v_out = RTD_F32(RTD_DDIV(var, dn));
+}
+
+// The per-pixel scale of one feature channel at p: 1 / (3 k_f^2 max(tau, s(p), g(p)^2)), with the central differences
+// gx, gy of the channel's mean and kf2_3 = 3 k_f^2 (a k_f^2 beyond the f32 range gives 0: the feature never matters)
+RTD_DEV float guide_scale(float s_p, float gx, float gy, float kf2_3, float tau) {
+    const float g2 = fmaf(gx, gx, gy * gy);
+    return RTD_FRCP(kf2_3 * fmaxf(tau, fmaxf(s_p, g2)));
+}
+
+// d_j(p, q) of one feature from the three channels' means m, variances of the mean s and scales (guide_scale) at p:
+//   sum_c [(m_c(p) - m_c(q))^2 - (s_c(p) + min(s_c(p), s_c(q)))] scale_c(p)
+RTD_DEV float guide_distance(const float m_p[3], const float s_p[3], const float scale_p[3], const float m_q[3], const float s_q[3]) {
+    float d = 0.0f;
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int c = 0; c < 3; ++c) {
+        const float e = m_p[c] - m_q[c];
+        d = fmaf(fmaf(e, e, -(s_p[c] + fminf(s_p[c], s_q[c]))), scale_p[c], d);
+    }
+    return d;
 }
 
 }  // namespace rtb

@@ -98,4 +98,8 @@ int check_adaptive(const RtParams* params, const RtAdaptive* ad, const char* who
 // `stream` after every round.  Adds to *launches and *paths.
 int adaptive_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, AccumFx* d_accum, AccumFx* d_moment2,
                     int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths);
+// rt_features.cu: the first-event features of samples [begin, begin + count) of the params' range (rt_render_features_device),
+// 3*W*H floats each, on a validated job; one launch
+int launch_features(RtScene* s, const RtCamera* cam, const RtParams* p, float* albedo, float* albedo_var, float* normal, float* normal_var,
+                    cudaStream_t stream);
 }  // namespace rtb

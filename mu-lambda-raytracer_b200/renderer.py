@@ -111,6 +111,7 @@ class Scene:
 
     def __init__(self, description, device=-1):
         self.description = description  # keep alive for sub-tree queries by the caller
+        self.device = int(device)  # -1: the current device
         h = C.c_void_p()
         abi.check(abi.load().rt_scene_create(description.ptr, int(device), C.byref(h)))
         self.handle = h
@@ -236,11 +237,13 @@ class Renderer:  # raytrace.rs:137-198
                       "bvh_layout": stats.bvh_layout_used}
         return rgb, samples, accum, moment2
 
-    def render_denoised(self, noise_threshold=None, min_samples=16, logger=None, **denoise_options):
+    def render_denoised(self, noise_threshold=None, min_samples=16, logger=None, guide=None, **denoise_options):
         """EXTENSION: a render through the moments family, then the variance-guided non-local-means filter (rt_render_denoised).
         noise_threshold None: a uniform render of parameters.samples_per_pixel (>= 2); else adaptive sampling as in
-        render_adaptive.  denoise_options: search_radius, patch_radius, k, alpha (see `denoise`).  Returns (rgb int32
-        [H,W,3], to_rgb of the filtered means; denoised float32 [H,W,3], the filtered means), row 0 at the bottom."""
+        render_adaptive.  denoise_options: search_radius, patch_radius, k, alpha (see `denoise`).  guide: None, or a dict of
+        k_feature, tau and feature_samples (each optional; defaults RT_GUIDE_DEFAULT_*) for the feature-guided filter
+        (rt_render_denoised_guided, see `denoise_guided`).  Returns (rgb int32 [H,W,3], to_rgb of the filtered means;
+        denoised float32 [H,W,3], the filtered means), row 0 at the bottom."""
         p = self._params()
         h, w = p.height, p.width
         rgb = np.empty((h, w, 3), dtype=np.int32)
@@ -251,13 +254,36 @@ class Renderer:  # raytrace.rs:137-198
             ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
         cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
         stats = abi.RtStats()
-        abi.check(abi.load().rt_render_denoised(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None,
-                                                C.byref(denoise_options_struct(**denoise_options)), rgb.ctypes.data, out.ctypes.data,
-                                                cb, None, C.byref(stats)))
+        if guide is None:
+            abi.check(abi.load().rt_render_denoised(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None,
+                                                    C.byref(denoise_options_struct(**denoise_options)), rgb.ctypes.data, out.ctypes.data,
+                                                    cb, None, C.byref(stats)))
+        else:
+            abi.check(abi.load().rt_render_denoised_guided(self.world.handle, C.byref(self.camera.c), C.byref(p),
+                                                           C.byref(ad) if ad else None, C.byref(denoise_options_struct(**denoise_options)),
+                                                           C.byref(guide_struct(**guide)), rgb.ctypes.data, out.ctypes.data, cb, None,
+                                                           C.byref(stats)))
         self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
                       "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
                       "bvh_layout": stats.bvh_layout_used}
         return rgb, out
+
+    def render_features(self, feature_samples=abi.RT_GUIDE_DEFAULT_FEATURE_SAMPLES):
+        """EXTENSION: the first-event features of samples [0, feature_samples) of every pixel (rt_render_features_device; the
+        definition is in include/rt_b200.h).  Returns numpy float32 (albedo, albedo_var, normal, normal_var), each [H, W, 3]
+        with row 0 at the bottom: per channel the mean over the samples and the variance of that mean."""
+        import torch
+        p = self._params()
+        p.sample_begin, p.sample_count = 0, int(feature_samples)
+        dev = torch.device("cuda", self.world.device) if self.world.device >= 0 else torch.device("cuda")
+        bufs = [torch.empty((p.height, p.width, 3), dtype=torch.float32, device=dev) for _ in range(4)]
+        stats = abi.RtStats()
+        abi.check(abi.load().rt_render_features_device(self.world.handle, C.byref(self.camera.c), C.byref(p),
+                                                           *[b.data_ptr() for b in bufs], None, C.byref(stats)))
+        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
+                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
+                      "bvh_layout": stats.bvh_layout_used}
+        return tuple(b.cpu().numpy() for b in bufs)
 
     def render(self, logger=None):
         """Renderer::render: H rows of W (r, g, b) tuples, row j = 0 at the BOTTOM; logger(j, H) called H times."""
@@ -292,6 +318,37 @@ def denoise(mean, var, search_radius=abi.RT_DENOISE_DEFAULT_SEARCH_RADIUS, patch
     abi.check(abi.load().rt_denoise_device(mean.data_ptr(), var.data_ptr(), mean.shape[1], mean.shape[0],
                                            C.byref(denoise_options_struct(search_radius, patch_radius, k, alpha)), out.data_ptr(),
                                            mean.device.index, stream))
+    return out
+
+
+def guide_struct(k_feature=abi.RT_GUIDE_DEFAULT_K_FEATURE, tau=abi.RT_GUIDE_DEFAULT_TAU, feature_samples=abi.RT_GUIDE_DEFAULT_FEATURE_SAMPLES):
+    """the RtGuide of the keyword arguments (defaults: the header's RT_GUIDE_DEFAULT_*)"""
+    g = abi.RtGuide()
+    g.k_feature, g.tau, g.feature_samples = float(k_feature), float(tau), int(feature_samples)
+    return g
+
+
+def denoise_guided(mean, var, albedo, albedo_var, normal, normal_var, k_feature=abi.RT_GUIDE_DEFAULT_K_FEATURE,
+                   tau=abi.RT_GUIDE_DEFAULT_TAU, **options):
+    """EXTENSION: the feature-guided non-local-means filter (rt_denoise_guided_device): `denoise` whose weights are also bounded by
+    the first-event albedo and normal features (Renderer.render_features; the definition is in include/rt_b200.h).  All six
+    inputs are contiguous CUDA float32 tensors [H, W, 3] on one device.  k_feature > 0: larger lets more across feature edges;
+    tau > 0: the floor of a feature's normalisation.  options: search_radius, patch_radius, k, alpha as in `denoise`.  Returns a
+    new tensor [H, W, 3], computed on the tensors' device and ordered on its current stream."""
+    import torch
+    ins = (mean, var, albedo, albedo_var, normal, normal_var)
+    if not all(isinstance(t, torch.Tensor) for t in ins):
+        raise TypeError("denoise_guided: every input must be a torch tensor")
+    if any(t.dtype != torch.float32 or not t.is_cuda or t.device != mean.device for t in ins):
+        raise ValueError("denoise_guided: every input must be a float32 CUDA tensor on one device")
+    if mean.dim() != 3 or mean.shape[2] != 3 or any(t.shape != mean.shape for t in ins):
+        raise ValueError("denoise_guided: every input must have the shape [H, W, 3]")
+    ins = [t.contiguous() for t in ins]
+    out = torch.empty_like(ins[0])
+    stream = torch.cuda.current_stream(mean.device).cuda_stream
+    abi.check(abi.load().rt_denoise_guided_device(*[t.data_ptr() for t in ins], mean.shape[1], mean.shape[0],
+                                                  C.byref(denoise_options_struct(**options)), C.byref(guide_struct(k_feature, tau)),
+                                                  out.data_ptr(), mean.device.index, stream))
     return out
 
 

@@ -397,6 +397,48 @@ int rt_render_denoised_guided(const RtScene* scene, const RtCamera* cam, const R
                               void* user, RtStats* stats);
 
 /*
+ * EXTENSION: dual-buffer cross-filtered denoising with a per-pixel error estimate, and adaptive sampling driven by that
+ * estimate.  The form follows Rousselle, Knaus & Zwicker, "Adaptive Rendering with Non-Local Means Filtering" (SIGGRAPH
+ * Asia 2012); it was not checked against the paper's text.
+ *
+ * Split: a job renders in ranges of samples (one for a uniform render, one per round for an adaptive one).  A range
+ * [b, b + c), c even, sends [b, b + c/2) to buffer A and [b + c/2, b + c) to buffer B; each holds the (S1, S2) sums of the
+ * moments family.  samples_per_pixel and min_samples (adaptive) must be even and >= 4, so every count n of the schedule of
+ * rt_render_adaptive is even and each half of a pixel holds n/2 >= 2 samples.  Per half, mu and v are those of
+ * rt_render_denoised with n/2.
+ * Cross filter: F_A is the filter of rt_denoise_device whose weights w(p, q) are computed from (mu_B, v_B), applied to
+ * mu_A; F_B is the same with A and B swapped.  With a guide each weight is also bounded by the feature weight of
+ * rt_denoise_guided_device (the same features for both halves).  out = (F_A + F_B) / 2 (f32).
+ * Error estimate: per channel, eps_c(p) = the mean over the 3 x 3 neighbourhood of p (neighbours clamped to the image, in
+ * row order from the bottom left) of ((F_A,c - F_B,c) / 2)^2, in f32 with every operation rounded on its own.  It estimates
+ * the VARIANCE of out_c(p), not its bias.
+ * Filtered stop rule: the rule of rt_render_adaptive on (out, eps) in place of (mu, se^2): per channel, in f64 with every
+ * operation rounded on its own, e = sqrt(eps) / (2 sqrt(max(out, 2^-16))); a pixel stops when n reaches the cap or when
+ * every channel has e <= noise_threshold or out - 3 sqrt(eps) >= 1.
+ * Exact reductions: with A = B, F_A = F_B = the output of rt_denoise_device (rt_denoise_guided_device with a guide) bit
+ * for bit, out equals it and eps = 0; swapping A and B gives the same out and eps bit for bit.
+ *
+ * rt_denoise_cross_device: the cross filter and the error estimate on device buffers of `device` (3*W*H floats each).
+ * guide NULL: colour-only, and the four feature pointers must be NULL; else all four are given.  d_err_rgb is optional;
+ * no output may overlap an input or the other output.  Asynchronous on `stream`.
+ * rt_render_denoised_dual: renders the two halves through the moments family — uniformly when `adaptive` is NULL, else in
+ * the rounds of rt_render_adaptive with the filtered stop rule (noise_threshold is its threshold) — cross-filters (guided
+ * when `guide` is given: the features of samples [0, guide->feature_samples), computed once before the first round) and
+ * tonemaps out with to_rgb.  In an adaptive render each round renders its half ranges for the active pixels, converts both
+ * halves of every pixel, filters the whole image and evaluates the active pixels.  Host buffers, each optional, row 0 at the
+ * bottom: rgb (3*W*H), denoised_rgb (out) and error_rgb (eps), 3*W*H floats each, samples (W*H counts).  Persistent
+ * pipeline only; sample_begin and sample_count must be 0.  cb as in rt_render_denoised.  stats: paths = the sum of the
+ * counts, device_ms from the first render launch (the feature pass) to the end of the tonemap.
+ */
+int rt_denoise_cross_device(const float* d_mean_a, const float* d_var_a, const float* d_mean_b, const float* d_var_b,
+                            const float* d_albedo, const float* d_albedo_var, const float* d_normal, const float* d_normal_var,
+                            int32_t width, int32_t height, const RtDenoise* opt, const RtGuide* guide, float* d_out_rgb,
+                            float* d_err_rgb, int device, void* stream);
+int rt_render_denoised_dual(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* adaptive,
+                            const RtDenoise* opt, const RtGuide* guide, int32_t* rgb, float* denoised_rgb, float* error_rgb,
+                            int32_t* samples, RtProgressFn cb, void* user, RtStats* stats);
+
+/*
  * rt_render over several GPUs of one process (the reference's row-parallel rayon loop, raytrace.rs:176-185, becomes
  * sample slices): scenes[g] is the same description created on a distinct device; device g renders every pixel for
  * the g-th slice of the sample range (rt_sample_slice), the float accumulation buffers are summed onto scenes[0]'s

@@ -222,6 +222,14 @@ extern "C" {
     pub fn rt_render_denoised_guided(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive,
                                      opt: *const RtDenoise, guide: *const RtGuide, rgb: *mut i32, denoised_rgb: *mut f32, cb: RtProgressFn,
                                      user: *mut c_void, stats: *mut RtStats) -> c_int;
+    // EXTENSION: dual-buffer cross-filtered denoising with an error estimate (guide null: colour-only)
+    pub fn rt_denoise_cross_device(d_mean_a: *const f32, d_var_a: *const f32, d_mean_b: *const f32, d_var_b: *const f32, d_albedo: *const f32,
+                                   d_albedo_var: *const f32, d_normal: *const f32, d_normal_var: *const f32, width: i32, height: i32,
+                                   opt: *const RtDenoise, guide: *const RtGuide, d_out_rgb: *mut f32, d_err_rgb: *mut f32, device: c_int,
+                                   stream: *mut c_void) -> c_int;
+    pub fn rt_render_denoised_dual(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive,
+                                   opt: *const RtDenoise, guide: *const RtGuide, rgb: *mut i32, denoised_rgb: *mut f32, error_rgb: *mut f32,
+                                   samples: *mut i32, cb: RtProgressFn, user: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_world_build(name: *const c_char, seed: u64, earth_rgb: *const u8, earth_w: i32, earth_h: i32, out: *mut *mut RtSceneDesc,
                           n_draws: *mut u64) -> c_int;
     pub fn rt_scene_desc_free(desc: *mut RtSceneDesc);

@@ -152,6 +152,11 @@ PROTOTYPES = {
     "rt_render_denoised_guided": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive),
                                             C.POINTER(RtDenoise), C.POINTER(RtGuide), C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p,
                                             C.POINTER(RtStats)]),
+    "rt_denoise_cross_device": (C.c_int, [C.c_void_p] * 8 + [C.c_int32, C.c_int32, C.POINTER(RtDenoise), C.POINTER(RtGuide), C.c_void_p, C.c_void_p,
+                                          C.c_int, C.c_void_p]),
+    "rt_render_denoised_dual": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtDenoise),
+                                          C.POINTER(RtGuide), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p,
+                                          C.POINTER(RtStats)]),
     "rt_tonemap_fixed_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int, C.c_void_p]),
     "rt_accum_fixed_to_float_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rt_release_cached_memory": (None, []),

@@ -15,7 +15,9 @@
 // (rt_render_adaptive; T = 0, the default, renders the fixed count; one GPU only), --denoise: the variance-guided
 // non-local-means filter with the library's default parameters after the render, uniform or adaptive (rt_render_denoised;
 // one GPU only; --stats then covers the render and the filter), --denoise_guided: the same with the feature-guided filter
-// and its default parameters (rt_render_denoised_guided; implies --denoise; --stats also covers the feature pass).
+// and its default parameters (rt_render_denoised_guided; implies --denoise; --stats also covers the feature pass),
+// --denoise_dual: dual-buffer cross filtering (rt_render_denoised_dual; implies --denoise, combines with --denoise_guided,
+// and with --noise_threshold the stop rule judges the filtered value; --samples_per_pixel and --min_samples must be even).
 // There is no CPU renderer here: without a CUDA device the program fails with the library's error.
 #include <unistd.h>
 
@@ -154,7 +156,7 @@ int main(int argc, char** argv) {
                             "aperture",     "focus_dist",  "world",             "seed",      "gpus",     "pipeline", "earthmap",
                             "noise_threshold", "min_samples"};
     std::map<std::string, std::string> opt = defaults;
-    bool randomized_rendering = false, want_stats = false, want_denoise = false, want_guided = false;
+    bool randomized_rendering = false, want_stats = false, want_denoise = false, want_guided = false, want_dual = false;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "--randomized_rendering" || a == "-r") {
@@ -173,8 +175,12 @@ int main(int argc, char** argv) {
             want_denoise = want_guided = true;
             continue;
         }
+        if (a == "--denoise_dual") {
+            want_denoise = want_dual = true;
+            continue;
+        }
         if (a == "--help" || a == "-h") {
-            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n        --denoise\n        --denoise_guided\n\nOPTIONS:\n");
+            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n        --denoise\n        --denoise_guided\n        --denoise_dual\n\nOPTIONS:\n");
             for (const char* v : valued) {
                 auto d = defaults.find(v);
                 printf("        --%s <%s>%s%s%s\n", v, v, d != defaults.end() ? " [default: " : "", d != defaults.end() ? d->second.c_str() : "",
@@ -245,7 +251,10 @@ int main(int argc, char** argv) {
     const long long min_samples = parse_int(opt["min_samples"], "min_samples");
     if (noise_threshold != 0.0 && gpus > 1) usage_error("--noise_threshold (adaptive sampling) renders on one GPU: it cannot be used with --gpus above 1");
     if (want_denoise && gpus > 1)
-        usage_error(std::string(want_guided ? "--denoise_guided" : "--denoise") + " renders and filters on one GPU: it cannot be used with --gpus above 1");
+        usage_error(std::string(want_dual ? "--denoise_dual" : want_guided ? "--denoise_guided" : "--denoise") +
+                    " renders and filters on one GPU: it cannot be used with --gpus above 1");
+    if (want_dual && (spp % 2 != 0 || min_samples % 2 != 0))
+        usage_error("--denoise_dual splits every range of samples into two halves: --samples_per_pixel and --min_samples must be even");
     static const std::map<std::string, int> pipelines = {{"auto", RT_PIPELINE_AUTO}, {"megakernel", RT_PIPELINE_MEGAKERNEL},
                                                          {"wavefront", RT_PIPELINE_WAVEFRONT},
                                                          {"persistent", RT_PIPELINE_PERSISTENT}};
@@ -306,10 +315,13 @@ int main(int argc, char** argv) {
         memset(&dn, 0, sizeof dn);
         dn.k = RT_DENOISE_DEFAULT_K, dn.alpha = RT_DENOISE_DEFAULT_ALPHA;
         dn.search_radius = RT_DENOISE_DEFAULT_SEARCH_RADIUS, dn.patch_radius = RT_DENOISE_DEFAULT_PATCH_RADIUS;
-        if (want_guided) {
-            RtGuide gd;
-            memset(&gd, 0, sizeof gd);
-            gd.k_feature = RT_GUIDE_DEFAULT_K_FEATURE, gd.tau = RT_GUIDE_DEFAULT_TAU, gd.feature_samples = RT_GUIDE_DEFAULT_FEATURE_SAMPLES;
+        RtGuide gd;
+        memset(&gd, 0, sizeof gd);
+        gd.k_feature = RT_GUIDE_DEFAULT_K_FEATURE, gd.tau = RT_GUIDE_DEFAULT_TAU, gd.feature_samples = RT_GUIDE_DEFAULT_FEATURE_SAMPLES;
+        if (want_dual) {
+            rc = rt_render_denoised_dual(scenes[0], &cam, &p, noise_threshold != 0.0 ? &ad : nullptr, &dn, want_guided ? &gd : nullptr, rgb.data(), nullptr,
+                                         nullptr, nullptr, progress_cb, &prog, &st);
+        } else if (want_guided) {
             rc = rt_render_denoised_guided(scenes[0], &cam, &p, noise_threshold != 0.0 ? &ad : nullptr, &dn, &gd, rgb.data(), nullptr, progress_cb, &prog,
                                            &st);
         } else {

@@ -116,8 +116,7 @@ int adaptive_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params,
 
     DCamera dc;
     make_camera(*cam, dc);
-    int n_rounds = 1;  // the schedule depends on (m, max) alone: the logger is paced by rounds
-    for (uint32_t n = m; n < n_max; n += std::min(n, n_max - n)) n_rounds += 1;
+    const int n_rounds = adaptive_round_total(m, n_max);  // the schedule depends on (m, max) alone: the logger is paced by rounds
 
     CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
     CU_TRY(cudaEventRecord(scene->ev0, stream));
@@ -130,7 +129,7 @@ int adaptive_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params,
     unsigned int n_list = npix;
     uint32_t n_done = 0;  // samples every active pixel holds
     for (int round = 0; n_list > 0u; ++round) {
-        const uint32_t count = round == 0 ? m : std::min(n_done, n_max - n_done);
+        const uint32_t count = adaptive_round_count(n_done, m, n_max);
         // round 0 covers every pixel: the list is the identity, which the kernel takes as a null list
         int rc = launch_persist_moments(scene, dc, params, (int)n_done, (int)count, d_accum, d_moment2, round == 0 ? nullptr : b.list_a, n_list, stream,
                                         &launches);

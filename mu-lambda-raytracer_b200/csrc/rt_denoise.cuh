@@ -18,7 +18,17 @@
 #define RTD_FDIV __fdividef  // x * MUFU.RCP(y): the library builds without --use_fast_math, so the approximation is explicit
 #define RTD_DADD __dadd_rn
 #define RTD_FRCP __frcp_rn
+#define RTD_FADD __fadd_rn
+#define RTD_FSUB __fsub_rn
+#define RTD_FMUL __fmul_rn
+#define RTD_FDIV_RN __fdiv_rn
+#define RTD_DSQRT __dsqrt_rn
 #else
+#define RTD_FADD(a, b) ((float)(a) + (float)(b))
+#define RTD_FSUB(a, b) ((float)(a) - (float)(b))
+#define RTD_FMUL(a, b) ((float)(a) * (float)(b))
+#define RTD_FDIV_RN(a, b) ((float)(a) / (float)(b))
+#define RTD_DSQRT(a) sqrt((double)(a))
 #define RTD_DADD(a, b) ((double)(a) + (double)(b))
 #define RTD_FRCP(a) (1.0f / (a))
 #define RTD_DEV inline
@@ -102,6 +112,40 @@ RTD_DEV float guide_distance(const float m_p[3], const float s_p[3], const float
         d = fmaf(fmaf(e, e, -(s_p[c] + fminf(s_p[c], s_q[c]))), scale_p[c], d);
     }
     return d;
+}
+
+// ---- dual buffers (rt_denoise_cross_device, rt_render_denoised_dual)
+
+// out of one channel from the two cross-filtered halves: (F_A + F_B) / 2
+RTD_DEV float dual_out(float fa, float fb) { return RTD_FMUL(RTD_FADD(fa, fb), 0.5f); }
+
+// eps of one channel from F_A and F_B at the nine neighbours of p (clamped to the image, in row order from the bottom left):
+// the mean of ((F_A - F_B) / 2)^2, every f32 operation rounded on its own (no contraction), so that the sum has one order
+RTD_DEV float dual_error(const float fa[9], const float fb[9]) {
+    float s = 0.0f;
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int k = 0; k < 9; ++k) {
+        const float d = RTD_FMUL(RTD_FSUB(fa[k], fb[k]), 0.5f);
+        s = RTD_FADD(s, RTD_FMUL(d, d));
+    }
+    return RTD_FDIV_RN(s, 9.0f);
+}
+
+// The filtered stop rule for a pixel that holds n of at most n_max samples, from its filtered value `out` and error estimate
+// `eps` per channel: the rule of adaptive_pixel_done with (out, eps) in place of (mu, se^2),
+//   e = sqrt(eps) / (2 sqrt(max(out, 2^-16))),
+// done when n == n_max or, for every channel, e <= threshold or out - 3 sqrt(eps) >= 1.  f64, every operation rounded on its own.
+RTD_DEV bool filtered_pixel_done(uint32_t n, uint32_t n_max, const float out[3], const float eps[3], double threshold) {
+    if (n >= n_max) return true;
+    for (int c = 0; c < 3; ++c) {
+        const double o = (double)out[c];
+        const double se = RTD_DSQRT((double)eps[c]);
+        const double e = RTD_DDIV(se, RTD_DMUL(2.0, RTD_DSQRT(o > 1.52587890625e-05 ? o : 1.52587890625e-05)));
+        if (!(e <= threshold || RTD_DSUB(o, RTD_DMUL(3.0, se)) >= 1.0)) return false;
+    }
+    return true;
 }
 
 }  // namespace rtb

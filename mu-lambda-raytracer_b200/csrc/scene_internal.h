@@ -2,6 +2,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <cstdint>
 #include <utility>
 #include <vector>
 
@@ -98,6 +100,14 @@ int check_adaptive(const RtParams* params, const RtAdaptive* ad, const char* who
 // `stream` after every round.  Adds to *launches and *paths.
 int adaptive_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, AccumFx* d_accum, AccumFx* d_moment2,
                     int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths);
+// the schedule of the rounds: the new samples of the round after every active pixel holds n_done (0 before round 0) of at
+// most n_max, with min_samples m: m, then as many as all earlier rounds together, the last one capped at n_max
+inline uint32_t adaptive_round_count(uint32_t n_done, uint32_t m, uint32_t n_max) { return n_done == 0 ? m : std::min(n_done, n_max - n_done); }
+inline int adaptive_round_total(uint32_t m, uint32_t n_max) {
+    int n_rounds = 0;
+    for (uint32_t n = 0; n < n_max; n += adaptive_round_count(n, m, n_max)) n_rounds += 1;
+    return n_rounds;
+}
 // rt_features.cu: the first-event features of samples [begin, begin + count) of the params' range (rt_render_features_device),
 // 3*W*H floats each, on a validated job; one launch
 int launch_features(RtScene* s, const RtCamera* cam, const RtParams* p, float* albedo, float* albedo_var, float* normal, float* normal_var,

@@ -268,6 +268,35 @@ class Renderer:  # raytrace.rs:137-198
                       "bvh_layout": stats.bvh_layout_used}
         return rgb, out
 
+    def render_denoised_dual(self, noise_threshold=None, min_samples=16, logger=None, guide=None, **denoise_options):
+        """EXTENSION: dual-buffer cross-filtered denoising with a per-pixel error estimate (rt_render_denoised_dual; the definition
+        is in include/rt_b200.h).  Each range of samples is split into two halves; each half is filtered with weights from the
+        other, and the two results give the output and an estimate of its variance.  noise_threshold None: a uniform render of
+        parameters.samples_per_pixel (even, >= 4); else adaptive sampling whose stop rule judges the FILTERED value and its error
+        estimate, with min_samples (even, >= 4).  guide and denoise_options as in render_denoised.  Returns (rgb int32 [H,W,3];
+        denoised float32 [H,W,3], the filtered means; error float32 [H,W,3], the error estimate eps (a variance); samples int32
+        [H,W], each pixel's count), row 0 at the bottom.  logger(j, H) as in render_adaptive."""
+        p = self._params()
+        h, w = p.height, p.width
+        rgb = np.empty((h, w, 3), dtype=np.int32)
+        out = np.empty((h, w, 3), dtype=np.float32)
+        err = np.empty((h, w, 3), dtype=np.float32)
+        samples = np.empty((h, w), dtype=np.int32)
+        ad = None
+        if noise_threshold is not None:
+            ad = abi.RtAdaptive()
+            ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
+        cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
+        stats = abi.RtStats()
+        abi.check(abi.load().rt_render_denoised_dual(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None,
+                                                     C.byref(denoise_options_struct(**denoise_options)),
+                                                     C.byref(guide_struct(**guide)) if guide is not None else None, rgb.ctypes.data,
+                                                     out.ctypes.data, err.ctypes.data, samples.ctypes.data, cb, None, C.byref(stats)))
+        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
+                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
+                      "bvh_layout": stats.bvh_layout_used}
+        return rgb, out, err, samples
+
     def render_features(self, feature_samples=abi.RT_GUIDE_DEFAULT_FEATURE_SAMPLES):
         """EXTENSION: the first-event features of samples [0, feature_samples) of every pixel (rt_render_features_device; the
         definition is in include/rt_b200.h).  Returns numpy float32 (albedo, albedo_var, normal, normal_var), each [H, W, 3]
@@ -350,6 +379,35 @@ def denoise_guided(mean, var, albedo, albedo_var, normal, normal_var, k_feature=
                                                   C.byref(denoise_options_struct(**options)), C.byref(guide_struct(k_feature, tau)),
                                                   out.data_ptr(), mean.device.index, stream))
     return out
+
+
+def denoise_cross(mean_a, var_a, mean_b, var_b, features=None, k_feature=abi.RT_GUIDE_DEFAULT_K_FEATURE, tau=abi.RT_GUIDE_DEFAULT_TAU,
+                  **options):
+    """EXTENSION: the dual-buffer cross filter (rt_denoise_cross_device; the definition is in include/rt_b200.h) of two
+    independent halves of a render, each a mean image and the variance of each mean.  Half A is filtered with weights computed
+    from B and B with weights from A.  features: None (colour-only), or (albedo, albedo_var, normal, normal_var) as in
+    `denoise_guided`, with k_feature and tau.  options: search_radius, patch_radius, k, alpha as in `denoise`.  Every input is
+    a contiguous CUDA float32 tensor [H, W, 3] on one device.  Returns new tensors (out, err): the mean of the two filtered
+    halves and the error estimate eps (an estimate of out's variance), computed on the tensors' device and ordered on its
+    current stream."""
+    import torch
+    ins = (mean_a, var_a, mean_b, var_b) + (tuple(features) if features is not None else ())
+    if features is not None and len(ins) != 8:
+        raise ValueError("denoise_cross: features must be (albedo, albedo_var, normal, normal_var)")
+    if not all(isinstance(t, torch.Tensor) for t in ins):
+        raise TypeError("denoise_cross: every input must be a torch tensor")
+    if any(t.dtype != torch.float32 or not t.is_cuda or t.device != mean_a.device for t in ins):
+        raise ValueError("denoise_cross: every input must be a float32 CUDA tensor on one device")
+    if mean_a.dim() != 3 or mean_a.shape[2] != 3 or any(t.shape != mean_a.shape for t in ins):
+        raise ValueError("denoise_cross: every input must have the shape [H, W, 3]")
+    ins = [t.contiguous() for t in ins]
+    ptrs = [t.data_ptr() for t in ins] + [None] * (8 - len(ins))
+    out, err = torch.empty_like(ins[0]), torch.empty_like(ins[0])
+    stream = torch.cuda.current_stream(mean_a.device).cuda_stream
+    guide = C.byref(guide_struct(k_feature, tau)) if features is not None else None
+    abi.check(abi.load().rt_denoise_cross_device(*ptrs, mean_a.shape[1], mean_a.shape[0], C.byref(denoise_options_struct(**options)), guide,
+                                                 out.data_ptr(), err.data_ptr(), mean_a.device.index, stream))
+    return out, err
 
 
 def to_ppm(rgb):

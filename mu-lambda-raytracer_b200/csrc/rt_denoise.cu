@@ -22,17 +22,17 @@
 // (at most 173 KB at r = 15, f = 7).  blockIdx.z picks the direction (F_A or F_B); colour-only and guided, every
 // locations-per-thread count.  dual_combine_kernel then writes out = (F_A + F_B) / 2 and the 3 x 3 error estimate.
 //
-// rt_render_denoised renders through the moments family (rt_adaptive.cu), converts the sums (denoise_mean_var), filters and
-// tonemaps.  rt_render_denoised_dual renders two halves of every range of samples, in the rounds of rt_render_adaptive's
-// schedule (adaptive_round_count), and cross-filters the whole image after each round; dual_eval_kernel applies the filtered
-// stop rule (filtered_pixel_done) to the active pixels.
+// Every filter launch goes through with_locations (the instance of the patch radius) and launch_tiles (one block per tile).
+//
+// Both renders run the round driver of rt_adaptive.cu (adaptive_rounds); a uniform render is its single round of
+// samples_per_pixel.  rt_render_denoised renders through the moments family (moments_rounds), converts the sums
+// (denoise_mean_var), filters and tonemaps.  rt_render_denoised_dual renders two halves of every range of samples in each
+// round and cross-filters the whole image; dual_eval_kernel applies the filtered stop rule (filtered_pixel_done) to the
+// active pixels.
 #include <cuda_runtime.h>
 
-#include <cub/device/device_select.cuh>
-
-#include <algorithm>
 #include <cmath>
-#include <cstring>
+#include <type_traits>
 
 #include "rt_denoise.cuh"
 #include "rt_device.cuh"
@@ -277,29 +277,26 @@ __global__ void denoise_tonemap_kernel(const float* __restrict__ x, int32_t* __r
 
 namespace {
 
-template <int NE>
-cudaError_t launch_nlm(const float* mean, const float* var, int W, int H, int r, int f, float k2, float alpha, float inv_norm, float* out,
-                       const GuideIn* guide, cudaStream_t stream) {
-    const size_t smem = smem_bytes(r, f);  // at most 116 KB (r = 15, f = 7); the guided filter reads the features through L1
-    const void* kernel = guide ? (const void*)denoise_nlm_guided_kernel<NE> : (const void*)denoise_nlm_kernel<NE>;
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    const dim3 grid((unsigned)((W + kTileX - 1) / kTileX), (unsigned)((H + kTileY - 1) / kTileY)), block(kTileX, kThreadsY);
-    if (guide) denoise_nlm_guided_kernel<NE><<<grid, block, smem, stream>>>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, *guide);
-    else denoise_nlm_kernel<NE><<<grid, block, smem, stream>>>(mean, var, W, H, r, f, k2, alpha, inv_norm, out);
-    return cudaGetLastError();
+// fn(std::integral_constant<int, NE>()) with NE the locations per thread of patch radius f: the filters' instances
+template <class Fn>
+cudaError_t with_locations(int f, Fn&& fn) {
+    static_assert(locations_per_thread(0) == 2 && locations_per_thread(RT_DENOISE_MAX_PATCH_RADIUS) == 6, "denoise_nlm_kernel instances");
+    switch (locations_per_thread(f)) {
+        case 2: return fn(std::integral_constant<int, 2>());
+        case 3: return fn(std::integral_constant<int, 3>());
+        case 4: return fn(std::integral_constant<int, 4>());
+        case 5: return fn(std::integral_constant<int, 5>());
+        default: return fn(std::integral_constant<int, 6>());
+    }
 }
 
-template <int NE>
-cudaError_t launch_nlm_cross(const float* ma, const float* va, const float* mb, const float* vb, int W, int H, int r, int f, float k2, float alpha,
-                             float inv_norm, float* fa, float* fb, const GuideIn* guide, cudaStream_t stream) {
-    const size_t smem = smem_bytes(r, f, 9);  // at most 173 KB (r = 15, f = 7)
-    const void* kernel = guide ? (const void*)denoise_nlm_cross_kernel<NE, true> : (const void*)denoise_nlm_cross_kernel<NE, false>;
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+// one filter kernel over the tiles of a W x H image (z: blockIdx.z's range) with smem bytes of dynamic shared memory
+template <class... P, class... A>
+cudaError_t launch_tiles(void (*kernel)(P...), int W, int H, unsigned z, size_t smem, cudaStream_t stream, A... args) {
+    const cudaError_t e = cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    const dim3 grid((unsigned)((W + kTileX - 1) / kTileX), (unsigned)((H + kTileY - 1) / kTileY), 2), block(kTileX, kThreadsY);
-    if (guide) denoise_nlm_cross_kernel<NE, true><<<grid, block, smem, stream>>>(ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, *guide);
-    else denoise_nlm_cross_kernel<NE, false><<<grid, block, smem, stream>>>(ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, GuideIn{});
+    const dim3 grid((unsigned)((W + kTileX - 1) / kTileX), (unsigned)((H + kTileY - 1) / kTileY), z), block(kTileX, kThreadsY);
+    kernel<<<grid, block, smem, stream>>>(args...);
     return cudaGetLastError();
 }
 
@@ -324,15 +321,12 @@ int check_guide(const RtGuide* guide, bool render, const char* who) {
 int denoise(const float* mean, const float* var, int W, int H, const RtDenoise* opt, float* out, cudaStream_t stream, const GuideIn* guide = nullptr) {
     const int r = opt->search_radius, f = opt->patch_radius;
     const float k2 = (float)(opt->k * opt->k), alpha = (float)opt->alpha, inv_norm = (float)(1.0 / (3.0 * (2 * f + 1) * (2 * f + 1)));
-    cudaError_t e;
-    switch (locations_per_thread(f)) {
-        case 2: e = launch_nlm<2>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
-        case 3: e = launch_nlm<3>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
-        case 4: e = launch_nlm<4>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
-        case 5: e = launch_nlm<5>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
-        default: e = launch_nlm<6>(mean, var, W, H, r, f, k2, alpha, inv_norm, out, guide, stream); break;
-    }
-    static_assert(locations_per_thread(0) == 2 && locations_per_thread(RT_DENOISE_MAX_PATCH_RADIUS) == 6, "denoise_nlm_kernel instances");
+    const size_t smem = smem_bytes(r, f);  // at most 116 KB (r = 15, f = 7); the guided filter reads the features through L1
+    const cudaError_t e = with_locations(f, [&](auto ne) {
+        constexpr int NE = decltype(ne)::value;
+        if (guide) return launch_tiles(denoise_nlm_guided_kernel<NE>, W, H, 1, smem, stream, mean, var, W, H, r, f, k2, alpha, inv_norm, out, *guide);
+        return launch_tiles(denoise_nlm_kernel<NE>, W, H, 1, smem, stream, mean, var, W, H, r, f, k2, alpha, inv_norm, out);
+    });
     if (e != cudaSuccess) return set_error(RT_ERR_CUDA, "denoise: %s", cudaGetErrorString(e));
     return RT_OK;
 }
@@ -343,14 +337,13 @@ int denoise_cross(const float* ma, const float* va, const float* mb, const float
                   float* fb, float* out, float* err, cudaStream_t stream) {
     const int r = opt->search_radius, f = opt->patch_radius;
     const float k2 = (float)(opt->k * opt->k), alpha = (float)opt->alpha, inv_norm = (float)(1.0 / (3.0 * (2 * f + 1) * (2 * f + 1)));
-    cudaError_t e;
-    switch (locations_per_thread(f)) {
-        case 2: e = launch_nlm_cross<2>(ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, guide, stream); break;
-        case 3: e = launch_nlm_cross<3>(ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, guide, stream); break;
-        case 4: e = launch_nlm_cross<4>(ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, guide, stream); break;
-        case 5: e = launch_nlm_cross<5>(ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, guide, stream); break;
-        default: e = launch_nlm_cross<6>(ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, guide, stream); break;
-    }
+    const size_t smem = smem_bytes(r, f, 9);  // at most 173 KB (r = 15, f = 7)
+    const GuideIn g = guide ? *guide : GuideIn{};
+    cudaError_t e = with_locations(f, [&](auto ne) {
+        constexpr int NE = decltype(ne)::value;
+        if (guide) return launch_tiles(denoise_nlm_cross_kernel<NE, true>, W, H, 2, smem, stream, ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, g);
+        return launch_tiles(denoise_nlm_cross_kernel<NE, false>, W, H, 2, smem, stream, ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, fa, fb, g);
+    });
     if (e != cudaSuccess) return set_error(RT_ERR_CUDA, "denoise_cross: %s", cudaGetErrorString(e));
     const long long n_values = 3LL * W * H;
     dual_combine_kernel<<<(unsigned)((n_values + 255) / 256), 256, 0, stream>>>(fa, fb, W, H, out, err);
@@ -364,24 +357,9 @@ GuideIn guide_in(const float* albedo, const float* albedo_var, const float* norm
     return GuideIn{albedo, albedo_var, normal, normal_var, (float)(3.0 * guide->k_feature * guide->k_feature), (float)guide->tau};
 }
 
-// device blocks of one denoised render, returned to the device cache on every exit
-struct DenoiseBuffers {
-    AccumFx *accum = nullptr, *moment2 = nullptr;
-    int32_t *samples = nullptr, *rgb = nullptr;
-    float *mean = nullptr, *var = nullptr, *out = nullptr;
-    float* feat[4] = {nullptr, nullptr, nullptr, nullptr};  // albedo, albedo_var, normal, normal_var (guided)
-    size_t n_pixels = 0;
-    ~DenoiseBuffers() {
-        cudaStreamSynchronize(0);
-        const size_t n = n_pixels;
-        rtb::cache_free(accum, 3 * n * sizeof(AccumFx)), rtb::cache_free(moment2, 3 * n * sizeof(AccumFx));
-        rtb::cache_free(samples, n * sizeof(int32_t)), rtb::cache_free(rgb, 3 * n * sizeof(int32_t));
-        rtb::cache_free(mean, 3 * n * sizeof(float)), rtb::cache_free(var, 3 * n * sizeof(float)), rtb::cache_free(out, 3 * n * sizeof(float));
-        for (float* b : feat) rtb::cache_free(b, 3 * n * sizeof(float));
-    }
-};
-
-// rt_render_denoised (guide == nullptr) and rt_render_denoised_guided
+// rt_render_denoised (guide == nullptr) and rt_render_denoised_guided: the rounds of moments_rounds (one round of
+// samples_per_pixel for a uniform render), then the feature pass (guided), the conversion of the sums, the filter and the
+// tonemapping
 int render_denoised(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt, const RtGuide* guide,
                     int32_t* rgb, float* denoised_rgb, RtProgressFn cb, void* user, RtStats* stats, const char* who) {
     int rc = have_device();
@@ -389,13 +367,9 @@ int render_denoised(const RtScene* scene_, const RtCamera* cam, const RtParams* 
     if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
     if ((rc = check_denoise(opt, who)) != RT_OK) return rc;
     if (guide && (rc = check_guide(guide, true, who)) != RT_OK) return rc;
-    if (ad) {
-        if ((rc = check_adaptive(params, ad, who)) != RT_OK) return rc;
-    } else {
-        if (params->sample_begin != 0 || params->sample_count != 0)
-            return set_error(RT_ERR_INVALID, "%s: sample_begin and sample_count must be 0 (the render owns the sample range)", who);
-        if (params->samples_per_pixel < 2) return set_error(RT_ERR_INVALID, "%s: a uniform render needs samples_per_pixel >= 2 (a variance)", who);
-    }
+    if ((rc = check_sample_range(params, ad, who)) != RT_OK) return rc;
+    if (!ad && params->samples_per_pixel < 2)
+        return set_error(RT_ERR_INVALID, "%s: a uniform render needs samples_per_pixel >= 2 (a variance)", who);
     if ((rc = check_pipeline(params)) != RT_OK) return rc;
     RtScene* scene = const_cast<RtScene*>(scene_);
     DeviceGuard g(scene->device);
@@ -403,81 +377,55 @@ int render_denoised(const RtScene* scene_, const RtCamera* cam, const RtParams* 
     const int W = params->width, H = params->height;
     const unsigned int npix = (unsigned int)W * (unsigned int)H;
     const size_t n_values = 3 * (size_t)npix;
+    const uint32_t n_max = (uint32_t)params->samples_per_pixel;
 
-    DenoiseBuffers b;
-    b.n_pixels = npix;
-    CU_TRY(rtb::cache_malloc((void**)&b.accum, n_values * sizeof(AccumFx)));
-    CU_TRY(rtb::cache_malloc((void**)&b.moment2, n_values * sizeof(AccumFx)));
-    if (ad) CU_TRY(rtb::cache_malloc((void**)&b.samples, npix * sizeof(int32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.rgb, n_values * sizeof(int32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.mean, n_values * sizeof(float)));
-    CU_TRY(rtb::cache_malloc((void**)&b.var, n_values * sizeof(float)));
-    CU_TRY(rtb::cache_malloc((void**)&b.out, n_values * sizeof(float)));
+    DeviceBlocks b(stream);
+    AccumFx *accum, *moment2;
+    int32_t *samples, *d_rgb;
+    float *mean, *var, *out;
+    float *albedo = nullptr, *albedo_var = nullptr, *normal = nullptr, *normal_var = nullptr;  // the features (guided)
+    CU_TRY(b.alloc(&accum, n_values));
+    CU_TRY(b.alloc(&moment2, n_values));
+    CU_TRY(b.alloc(&samples, npix));
+    CU_TRY(b.alloc(&d_rgb, n_values));
+    CU_TRY(b.alloc(&mean, n_values));
+    CU_TRY(b.alloc(&var, n_values));
+    CU_TRY(b.alloc(&out, n_values));
     if (guide)
-        for (float*& f : b.feat) CU_TRY(rtb::cache_malloc((void**)&f, n_values * sizeof(float)));
+        for (float** p : {&albedo, &albedo_var, &normal, &normal_var}) CU_TRY(b.alloc(p, n_values));
 
     rtb::RowProgress rows{cb, user, H, 0};
     int launches = 0;
     uint64_t paths = 0;
-    if (ad) {
-        rc = adaptive_rounds(scene, cam, params, ad, b.accum, b.moment2, b.samples, stream, &rows, &launches, &paths);
-        if (rc != RT_OK) return rc;
-    } else {
-        DCamera dc;
-        make_camera(*cam, dc);
-        CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
-        CU_TRY(cudaEventRecord(scene->ev0, stream));
-        CU_TRY(cudaMemsetAsync(b.accum, 0, n_values * sizeof(AccumFx), stream));
-        CU_TRY(cudaMemsetAsync(b.moment2, 0, n_values * sizeof(AccumFx), stream));
-        rc = launch_persist_moments(scene, dc, params, 0, params->samples_per_pixel, b.accum, b.moment2, nullptr, npix, stream, &launches);
-        if (rc != RT_OK) return rc;
-        paths = (uint64_t)npix * (uint64_t)params->samples_per_pixel;
-    }
+    rc = moments_rounds(scene, cam, params, ad ? (uint32_t)ad->min_samples : n_max, ad ? ad->noise_threshold : 0.0, accum, moment2, samples, stream, &rows,
+                        &launches, &paths);
+    if (rc != RT_OK) return rc;
     if (guide) {
         RtParams fp = *params;
         fp.sample_begin = 0, fp.sample_count = guide->feature_samples;
-        if ((rc = launch_features(scene, cam, &fp, b.feat[0], b.feat[1], b.feat[2], b.feat[3], stream)) != RT_OK) return rc;
+        if ((rc = launch_features(scene, cam, &fp, albedo, albedo_var, normal, normal_var, stream)) != RT_OK) return rc;
         launches += 1;
     }
     const unsigned blocks = (unsigned)((n_values + 255) / 256);
-    denoise_convert_kernel<<<blocks, 256, 0, stream>>>(b.accum, b.moment2, b.samples, (uint32_t)params->samples_per_pixel, (long long)n_values, b.mean,
-                                                       b.var);
+    denoise_convert_kernel<<<blocks, 256, 0, stream>>>(accum, moment2, samples, n_max, (long long)n_values, mean, var);
     CU_TRY(cudaGetLastError());
-    if (guide) {
-        const GuideIn gi = guide_in(b.feat[0], b.feat[1], b.feat[2], b.feat[3], guide);
-        if ((rc = denoise(b.mean, b.var, W, H, opt, b.out, stream, &gi)) != RT_OK) return rc;
-    } else if ((rc = denoise(b.mean, b.var, W, H, opt, b.out, stream)) != RT_OK) {
-        return rc;
-    }
-    denoise_tonemap_kernel<<<blocks, 256, 0, stream>>>(b.out, b.rgb, (long long)n_values);
+    const GuideIn gi = guide ? guide_in(albedo, albedo_var, normal, normal_var, guide) : GuideIn{};
+    if ((rc = denoise(mean, var, W, H, opt, out, stream, guide ? &gi : nullptr)) != RT_OK) return rc;
+    denoise_tonemap_kernel<<<blocks, 256, 0, stream>>>(out, d_rgb, (long long)n_values);
     CU_TRY(cudaGetLastError());
     launches += 3;
     CU_TRY(cudaEventRecord(scene->ev1, stream));
-    if (rgb) CU_TRY(cudaMemcpyAsync(rgb, b.rgb, n_values * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
-    if (denoised_rgb) CU_TRY(cudaMemcpyAsync(denoised_rgb, b.out, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
+    if (rgb) CU_TRY(cudaMemcpyAsync(rgb, d_rgb, n_values * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    if (denoised_rgb) CU_TRY(cudaMemcpyAsync(denoised_rgb, out, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
     CU_TRY(cudaStreamSynchronize(stream));
-    rtb::row_progress(1, 1, &rows);  // every row of a uniform render; whatever rows the rounds did not cover
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        float ms = 0;
-        CU_TRY(cudaEventElapsedTime(&ms, scene->ev0, scene->ev1));
-        unsigned long long rays = 0;
-        CU_TRY(cudaMemcpy(&rays, scene->d_rays, sizeof rays, cudaMemcpyDeviceToHost));
-        stats->paths = paths, stats->rays = rays, stats->device_ms = ms;
-        stats->kernel_launches = launches;
-        stats->pipeline_used = RT_PIPELINE_PERSISTENT;
-        stats->bvh_layout_used = persist_layout_used(scene, params);
-    }
-    return RT_OK;
+    rtb::row_progress(1, 1, &rows);  // whatever rows the rounds did not cover
+    return render_stats(scene, params, paths, launches, stats);
 }
 
-// the active pixels after a dual round: (list non-null) the identity list of round 0 and the half count of each pixel
-__global__ void dual_count_kernel(uint32_t* __restrict__ identity, unsigned int n_list, const uint32_t* __restrict__ list, int32_t half,
-                                  int32_t* __restrict__ d_half) {
+// the half count of the active pixels after a dual round
+__global__ void dual_count_kernel(const uint32_t* __restrict__ list, unsigned int n_list, int32_t half, int32_t* __restrict__ d_half) {
     const unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_list) return;
-    if (identity) identity[i] = i;
-    d_half[identity ? i : list[i]] = half;
+    if (i < n_list) d_half[list[i]] = half;
 }
 
 // the active pixels after a dual round that brought each of them to n samples: whether they go on (filtered_pixel_done)
@@ -489,29 +437,6 @@ __global__ void dual_eval_kernel(const uint32_t* __restrict__ list, unsigned int
     keep[i] = filtered_pixel_done(n, n_max, out + 3 * p, err + 3 * p, threshold) ? 0 : 1;
 }
 
-// device blocks of one dual render, returned to the device cache on every exit
-struct DualBuffers {
-    AccumFx* sums[4] = {nullptr, nullptr, nullptr, nullptr};  // S1 and S2 of A, S1 and S2 of B
-    float* planes[8] = {};                                    // mu_A, v_A, mu_B, v_B, F_A, F_B, out, eps
-    float* feat[4] = {nullptr, nullptr, nullptr, nullptr};   // albedo, albedo_var, normal, normal_var (guided)
-    int32_t *half = nullptr, *rgb = nullptr;
-    uint32_t *list_a = nullptr, *list_b = nullptr;
-    unsigned char* keep = nullptr;
-    int* n_sel = nullptr;
-    void* temp = nullptr;
-    size_t n_pixels = 0, temp_bytes = 0;
-    ~DualBuffers() {
-        cudaStreamSynchronize(0);
-        const size_t n = n_pixels;
-        for (AccumFx* b : sums) rtb::cache_free(b, 3 * n * sizeof(AccumFx));
-        for (float* b : planes) rtb::cache_free(b, 3 * n * sizeof(float));
-        for (float* b : feat) rtb::cache_free(b, 3 * n * sizeof(float));
-        rtb::cache_free(half, n * sizeof(int32_t)), rtb::cache_free(rgb, 3 * n * sizeof(int32_t));
-        rtb::cache_free(list_a, n * sizeof(uint32_t)), rtb::cache_free(list_b, n * sizeof(uint32_t));
-        rtb::cache_free(keep, n), rtb::cache_free(n_sel, sizeof(int)), rtb::cache_free(temp, temp_bytes);
-    }
-};
-
 int check_dual_counts(const RtParams* params, const RtAdaptive* ad, const char* who) {
     const int32_t spp = params->samples_per_pixel;
     if (spp < 4 || spp % 2 != 0) return set_error(RT_ERR_INVALID, "%s: samples_per_pixel must be even and >= 4 (two halves with a variance each)", who);
@@ -520,9 +445,9 @@ int check_dual_counts(const RtParams* params, const RtAdaptive* ad, const char* 
     return RT_OK;
 }
 
-// rt_render_denoised_dual: the rounds of adaptive_rounds' schedule (one round of samples_per_pixel for a uniform render), each
-// rendering its two half ranges, converting both halves of every pixel, cross-filtering, combining and evaluating the active
-// pixels with the filtered rule
+// rt_render_denoised_dual: the rounds of adaptive_rounds (one round of samples_per_pixel for a uniform render), each rendering
+// its two half ranges, converting both halves of every pixel, cross-filtering, combining and evaluating the active pixels
+// with the filtered rule
 int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,
                          const RtGuide* guide, int32_t* rgb, float* denoised_rgb, float* error_rgb, int32_t* samples, RtProgressFn cb, void* user,
                          RtStats* stats) {
@@ -532,11 +457,7 @@ int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtPar
     if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
     if ((rc = check_denoise(opt, who)) != RT_OK) return rc;
     if (guide && (rc = check_guide(guide, true, who)) != RT_OK) return rc;
-    if (ad) {
-        if ((rc = check_adaptive(params, ad, who)) != RT_OK) return rc;
-    } else if (params->sample_begin != 0 || params->sample_count != 0) {
-        return set_error(RT_ERR_INVALID, "%s: sample_begin and sample_count must be 0 (the render owns the sample range)", who);
-    }
+    if ((rc = check_sample_range(params, ad, who)) != RT_OK) return rc;
     if ((rc = check_dual_counts(params, ad, who)) != RT_OK) return rc;
     if ((rc = check_pipeline(params)) != RT_OK) return rc;
     RtScene* scene = const_cast<RtScene*>(scene_);
@@ -548,99 +469,71 @@ int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtPar
     const uint32_t n_max = (uint32_t)params->samples_per_pixel, m = ad ? (uint32_t)ad->min_samples : n_max;
     const double threshold = ad ? ad->noise_threshold : 0.0;
 
-    DualBuffers b;
-    b.n_pixels = npix;
-    for (AccumFx*& p : b.sums) CU_TRY(rtb::cache_malloc((void**)&p, n_values * sizeof(AccumFx)));
-    for (float*& p : b.planes) CU_TRY(rtb::cache_malloc((void**)&p, n_values * sizeof(float)));
+    DeviceBlocks b(stream);
+    AccumFx *s1_a, *s2_a, *s1_b, *s2_b;                      // the sums of the halves A and B
+    float *mu_a, *v_a, *mu_b, *v_b, *f_a, *f_b, *out, *err;  // their means and variances, F_A, F_B, out and eps
+    float *albedo = nullptr, *albedo_var = nullptr, *normal = nullptr, *normal_var = nullptr;  // the features (guided)
+    int32_t *half, *d_rgb;
+    for (AccumFx** p : {&s1_a, &s2_a, &s1_b, &s2_b}) CU_TRY(b.alloc(p, n_values));
+    for (float** p : {&mu_a, &v_a, &mu_b, &v_b, &f_a, &f_b, &out, &err}) CU_TRY(b.alloc(p, n_values));
     if (guide)
-        for (float*& p : b.feat) CU_TRY(rtb::cache_malloc((void**)&p, n_values * sizeof(float)));
-    CU_TRY(rtb::cache_malloc((void**)&b.half, npix * sizeof(int32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.rgb, n_values * sizeof(int32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.list_a, npix * sizeof(uint32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.list_b, npix * sizeof(uint32_t)));
-    CU_TRY(rtb::cache_malloc((void**)&b.keep, npix));
-    CU_TRY(rtb::cache_malloc((void**)&b.n_sel, sizeof(int)));
-    CU_TRY(cub::DeviceSelect::Flagged(nullptr, b.temp_bytes, b.list_a, b.keep, b.list_b, b.n_sel, (int)npix, stream));
-    CU_TRY(rtb::cache_malloc(&b.temp, b.temp_bytes));
-    float *mu_a = b.planes[0], *v_a = b.planes[1], *mu_b = b.planes[2], *v_b = b.planes[3], *out = b.planes[6], *err = b.planes[7];
+        for (float** p : {&albedo, &albedo_var, &normal, &normal_var}) CU_TRY(b.alloc(p, n_values));
+    CU_TRY(b.alloc(&half, npix));
+    CU_TRY(b.alloc(&d_rgb, n_values));
+    const GuideIn gi = guide ? guide_in(albedo, albedo_var, normal, normal_var, guide) : GuideIn{};
 
     rtb::RowProgress rows{cb, user, H, 0};
     DCamera dc;
     make_camera(*cam, dc);
-    CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
-    CU_TRY(cudaEventRecord(scene->ev0, stream));
     int launches = 0;
-    if (guide) {
-        RtParams fp = *params;
-        fp.sample_begin = 0, fp.sample_count = guide->feature_samples;
-        if ((rc = launch_features(scene, cam, &fp, b.feat[0], b.feat[1], b.feat[2], b.feat[3], stream)) != RT_OK) return rc;
-        launches += 1;
-    }
-    const GuideIn gi = guide ? guide_in(b.feat[0], b.feat[1], b.feat[2], b.feat[3], guide) : GuideIn{};
-    for (AccumFx* p : b.sums) CU_TRY(cudaMemsetAsync(p, 0, n_values * sizeof(AccumFx), stream));
-    const int n_rounds = adaptive_round_total(m, n_max);
-    const unsigned blocks = (unsigned)((n_values + 255) / 256);
     uint64_t paths = 0;
-    unsigned int n_list = npix;
-    uint32_t n_done = 0;  // samples every active pixel holds
-    for (int round = 0; n_list > 0u; ++round) {
-        const uint32_t count = adaptive_round_count(n_done, m, n_max), h = count / 2;
-        // round 0 covers every pixel: the list is the identity, which the render takes as a null list
-        const uint32_t* list = round == 0 ? nullptr : b.list_a;
-        rc = launch_persist_moments(scene, dc, params, (int)n_done, (int)h, b.sums[0], b.sums[1], list, n_list, stream, &launches);
-        if (rc != RT_OK) return rc;
-        rc = launch_persist_moments(scene, dc, params, (int)(n_done + h), (int)h, b.sums[2], b.sums[3], list, n_list, stream, &launches);
-        if (rc != RT_OK) return rc;
-        paths += (uint64_t)n_list * count;
-        n_done += count;
-        const unsigned list_blocks = (n_list + 255) / 256;
-        dual_count_kernel<<<list_blocks, 256, 0, stream>>>(round == 0 ? b.list_a : nullptr, n_list, b.list_a, (int32_t)(n_done / 2), b.half);
-        CU_TRY(cudaGetLastError());
-        // every pixel: stopped pixels still feed their neighbours
-        denoise_convert_kernel<<<blocks, 256, 0, stream>>>(b.sums[0], b.sums[1], b.half, 0, (long long)n_values, mu_a, v_a);
-        CU_TRY(cudaGetLastError());
-        denoise_convert_kernel<<<blocks, 256, 0, stream>>>(b.sums[2], b.sums[3], b.half, 0, (long long)n_values, mu_b, v_b);
-        CU_TRY(cudaGetLastError());
-        rc = denoise_cross(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, b.planes[4], b.planes[5], out, err, stream);
-        if (rc != RT_OK) return rc;
-        dual_eval_kernel<<<list_blocks, 256, 0, stream>>>(b.list_a, n_list, n_done, n_max, threshold, out, err, b.keep);
-        CU_TRY(cudaGetLastError());
-        launches += 6;
-        int n_next = 0;
-        if (n_done < n_max) {
-            CU_TRY(cub::DeviceSelect::Flagged(b.temp, b.temp_bytes, b.list_a, b.keep, b.list_b, b.n_sel, (int)n_list, stream));
-            CU_TRY(cudaMemcpyAsync(&n_next, b.n_sel, sizeof(int), cudaMemcpyDeviceToHost, stream));
+    const unsigned blocks = (unsigned)((n_values + 255) / 256);
+    const auto start = [&]() -> int {
+        CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
+        CU_TRY(cudaEventRecord(scene->ev0, stream));
+        if (guide) {
+            RtParams fp = *params;
+            fp.sample_begin = 0, fp.sample_count = guide->feature_samples;
+            if ((rc = launch_features(scene, cam, &fp, albedo, albedo_var, normal, normal_var, stream)) != RT_OK) return rc;
             launches += 1;
         }
-        CU_TRY(cudaStreamSynchronize(stream));
-        std::swap(b.list_a, b.list_b);
-        n_list = (unsigned int)n_next;
-        rtb::row_progress(round + 1, n_rounds, &rows);
-    }
-    denoise_tonemap_kernel<<<blocks, 256, 0, stream>>>(out, b.rgb, (long long)n_values);
+        for (AccumFx* p : {s1_a, s2_a, s1_b, s2_b}) CU_TRY(cudaMemsetAsync(p, 0, n_values * sizeof(AccumFx), stream));
+        return RT_OK;
+    };
+    const auto round = [&](const AdaptiveRound& r) -> int {
+        const uint32_t h = r.count / 2, n = r.first + r.count;
+        int rc = launch_persist_moments(scene, dc, params, (int)r.first, (int)h, s1_a, s2_a, r.render_list, r.n_list, stream, &launches);
+        if (rc != RT_OK) return rc;
+        rc = launch_persist_moments(scene, dc, params, (int)(r.first + h), (int)h, s1_b, s2_b, r.render_list, r.n_list, stream, &launches);
+        if (rc != RT_OK) return rc;
+        const unsigned list_blocks = (r.n_list + 255) / 256;
+        dual_count_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, (int32_t)(n / 2), half);
+        CU_TRY(cudaGetLastError());
+        // every pixel: stopped pixels still feed their neighbours
+        denoise_convert_kernel<<<blocks, 256, 0, stream>>>(s1_a, s2_a, half, 0, (long long)n_values, mu_a, v_a);
+        CU_TRY(cudaGetLastError());
+        denoise_convert_kernel<<<blocks, 256, 0, stream>>>(s1_b, s2_b, half, 0, (long long)n_values, mu_b, v_b);
+        CU_TRY(cudaGetLastError());
+        if ((rc = denoise_cross(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, f_a, f_b, out, err, stream)) != RT_OK) return rc;
+        dual_eval_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, n, n_max, threshold, out, err, r.keep);
+        CU_TRY(cudaGetLastError());
+        launches += 6;
+        return RT_OK;
+    };
+    if ((rc = adaptive_rounds(npix, m, n_max, stream, &rows, &launches, &paths, start, round)) != RT_OK) return rc;
+    denoise_tonemap_kernel<<<blocks, 256, 0, stream>>>(out, d_rgb, (long long)n_values);
     CU_TRY(cudaGetLastError());
     launches += 1;
     CU_TRY(cudaEventRecord(scene->ev1, stream));
-    if (rgb) CU_TRY(cudaMemcpyAsync(rgb, b.rgb, n_values * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    if (rgb) CU_TRY(cudaMemcpyAsync(rgb, d_rgb, n_values * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
     if (denoised_rgb) CU_TRY(cudaMemcpyAsync(denoised_rgb, out, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
     if (error_rgb) CU_TRY(cudaMemcpyAsync(error_rgb, err, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
-    if (samples) CU_TRY(cudaMemcpyAsync(samples, b.half, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    if (samples) CU_TRY(cudaMemcpyAsync(samples, half, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
     CU_TRY(cudaStreamSynchronize(stream));
     if (samples)
         for (size_t i = 0; i < npix; ++i) samples[i] *= 2;  // (the device holds the count of each half)
     rtb::row_progress(1, 1, &rows);  // whatever rows the rounds did not cover
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        float ms = 0;
-        CU_TRY(cudaEventElapsedTime(&ms, scene->ev0, scene->ev1));
-        unsigned long long rays = 0;
-        CU_TRY(cudaMemcpy(&rays, scene->d_rays, sizeof rays, cudaMemcpyDeviceToHost));
-        stats->paths = paths, stats->rays = rays, stats->device_ms = ms;
-        stats->kernel_launches = launches;
-        stats->pipeline_used = RT_PIPELINE_PERSISTENT;
-        stats->bvh_layout_used = persist_layout_used(scene, params);
-    }
-    return RT_OK;
+    return render_stats(scene, params, paths, launches, stats);
 }
 
 }  // namespace

@@ -4,6 +4,7 @@
 
 #include <algorithm>
 #include <cstdint>
+#include <functional>
 #include <utility>
 #include <vector>
 
@@ -92,14 +93,56 @@ int launch_persist_moments(RtScene* s, const DCamera& cam, const RtParams* p, in
                            const uint32_t* d_list, unsigned int n_list, cudaStream_t stream, int* launches);
 int have_device();  // RT_OK, or RT_ERR_NO_DEVICE with the message set
 int validate_render(const RtScene* scene, const RtCamera* cam, const RtParams* p);
-// rt_adaptive.cu: RT_ERR_UNSUPPORTED unless the persistent pipeline; the checks of an RtAdaptive and the sample range
+// Device blocks of one call from the device cache.  Each block is returned with the byte count it was allocated with (the
+// cache is keyed by size) when the owner goes out of scope, after `stream` is synchronised: an error return may leave work
+// in flight, and the cache hands blocks on without a free.
+class DeviceBlocks {
+  public:
+    explicit DeviceBlocks(cudaStream_t stream) : stream_(stream) {}
+    DeviceBlocks(const DeviceBlocks&) = delete;
+    DeviceBlocks& operator=(const DeviceBlocks&) = delete;
+    ~DeviceBlocks() {
+        cudaStreamSynchronize(stream_);
+        for (const auto& [p, bytes] : blocks_) cache_free(p, bytes);
+    }
+    template <class T>
+    cudaError_t alloc(T** p, size_t n) {  // n elements of T
+        const cudaError_t e = cache_malloc((void**)p, n * sizeof(T));
+        if (e == cudaSuccess) blocks_.emplace_back(*p, n * sizeof(T));
+        return e;
+    }
+
+  private:
+    cudaStream_t stream_;
+    std::vector<std::pair<void*, size_t>> blocks_;
+};
+
+// rt_adaptive.cu: RT_ERR_UNSUPPORTED unless the persistent pipeline; the sample range a render owns (sample_begin and
+// sample_count 0), then with an RtAdaptive its min_samples and noise_threshold
 int check_pipeline(const RtParams* p);
-int check_adaptive(const RtParams* params, const RtAdaptive* ad, const char* who);
-// the rounds of rt_render_adaptive on a validated job: zeroes d_accum / d_moment2 (3*W*H) and leaves each pixel's sums and its
-// count (d_samples, W*H) on the device; records scene->ev0 before the first launch, reports rows through `rows`, synchronises
-// `stream` after every round.  Adds to *launches and *paths.
-int adaptive_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, AccumFx* d_accum, AccumFx* d_moment2,
-                    int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths);
+int check_sample_range(const RtParams* params, const RtAdaptive* ad, const char* who);
+// one round of adaptive_rounds: samples [first, first + count) of the n_list active pixels
+struct AdaptiveRound {
+    uint32_t first, count;
+    const uint32_t* list;         // the active pixels, ascending; the identity in round 0
+    const uint32_t* render_list;  // the same for launch_persist_moments: nullptr (every pixel) in round 0
+    unsigned int n_list;
+    unsigned char* keep;          // to be written by the round: 1 where the pixel goes on, 0 where it stops
+};
+// The rounds of adaptive sampling on a validated job of npix pixels, in the schedule of adaptive_round_count.  Allocates the
+// lists, then calls `start` (the caller resets scene->d_rays, records scene->ev0 and zeroes its sums, so that no allocation
+// is timed), builds the identity list and runs `round` for every round.  After each round it compacts the kept pixels into
+// the next list (cub::DeviceSelect::Flagged, stable), synchronises `stream` once and reports rows through `rows`.  Adds its
+// own launches and the paths of every round to *launches and *paths; `round` adds the launches it makes.
+int adaptive_rounds(unsigned int npix, uint32_t m, uint32_t n_max, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths,
+                    const std::function<int()>& start, const std::function<int(const AdaptiveRound&)>& round);
+// the rounds of rt_render_adaptive (uniform: m = n_max): zeroes d_accum / d_moment2 (3*W*H), renders every round through the
+// moments family and applies the stop rule (adaptive_pixel_done) with `threshold`; leaves each pixel's sums and its count
+// (d_samples, W*H) on the device.  Timing starts at scene->ev0, recorded before the first launch.
+int moments_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, uint32_t m, double threshold, AccumFx* d_accum, AccumFx* d_moment2,
+                   int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths);
+// fills *stats (if non-null) of a persistent-pipeline render timed from scene->ev0 to scene->ev1 (both recorded)
+int render_stats(const RtScene* scene, const RtParams* params, uint64_t paths, int launches, RtStats* stats);
 // the schedule of the rounds: the new samples of the round after every active pixel holds n_done (0 before round 0) of at
 // most n_max, with min_samples m: m, then as many as all earlier rounds together, the last one capped at n_max
 inline uint32_t adaptive_round_count(uint32_t n_done, uint32_t m, uint32_t n_max) { return n_done == 0 ? m : std::min(n_done, n_max - n_done); }

@@ -46,6 +46,35 @@ def load_earthmap(path=None):
     return np.frombuffer(data, dtype=np.uint8, offset=pos + 1, count=w * h * 3).reshape(h, w, 3).copy()
 
 
+def _stats_dict(stats):
+    """Renderer.stats of the RtStats of one call"""
+    return {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms, "kernel_launches": stats.kernel_launches,
+            "pipeline": stats.pipeline_used, "bvh_layout": stats.bvh_layout_used}
+
+
+def _adaptive(noise_threshold, min_samples):
+    """the RtAdaptive of an adaptive render, or None (a uniform render) when noise_threshold is None"""
+    if noise_threshold is None:
+        return None
+    ad = abi.RtAdaptive()
+    ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
+    return ad
+
+
+def _image_inputs(who, ins, subject="every input", plural=False):
+    """the inputs of a denoise function, checked and made contiguous: torch tensors, float32 on one CUDA device, each of the
+    shape [H, W, 3].  Errors read "<who>: <subject> must be ...", in the plural for a subject that names several inputs."""
+    import torch
+    a, s = ("", "s") if plural else ("a ", "")
+    if not all(isinstance(t, torch.Tensor) for t in ins):
+        raise TypeError(f"{who}: {subject} must be {a}torch tensor{s}")
+    if any(t.dtype != torch.float32 or not t.is_cuda or t.device != ins[0].device for t in ins):
+        raise ValueError(f"{who}: {subject} must be {a}float32 CUDA tensor{s} on one device")
+    if ins[0].dim() != 3 or ins[0].shape[2] != 3 or any(t.shape != ins[0].shape for t in ins):
+        raise ValueError(f"{who}: {subject} must have the shape [H, W, 3]")
+    return [t.contiguous() for t in ins]
+
+
 class GradientBackground:  # raytrace.rs:12-35
     kind = abi.RT_BG_GRADIENT
 
@@ -208,9 +237,7 @@ class Renderer:  # raytrace.rs:137-198
         abi.check(abi.load().rt_render(self.world.handle, C.byref(self.camera.c), C.byref(p),
                                        accum.ctypes.data_as(C.c_void_p) if want_accum else None,
                                        rgb.ctypes.data_as(C.c_void_p), cb, None, C.byref(stats)))
-        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
-                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
-                      "bvh_layout": stats.bvh_layout_used}
+        self.stats = _stats_dict(stats)
         return rgb, accum
 
     def render_adaptive(self, noise_threshold, min_samples=16, logger=None):
@@ -225,16 +252,13 @@ class Renderer:  # raytrace.rs:137-198
         samples = np.empty((h, w), dtype=np.int32)
         accum = np.empty((h, w, 3), dtype=np.uint64)
         moment2 = np.empty((h, w, 3), dtype=np.uint64)
-        ad = abi.RtAdaptive()
-        ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
+        ad = _adaptive(noise_threshold, min_samples)
         cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
         stats = abi.RtStats()
         abi.check(abi.load().rt_render_adaptive(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad),
                                                 rgb.ctypes.data, samples.ctypes.data, accum.ctypes.data, moment2.ctypes.data,
                                                 cb, None, C.byref(stats)))
-        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
-                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
-                      "bvh_layout": stats.bvh_layout_used}
+        self.stats = _stats_dict(stats)
         return rgb, samples, accum, moment2
 
     def render_denoised(self, noise_threshold=None, min_samples=16, logger=None, guide=None, **denoise_options):
@@ -248,10 +272,7 @@ class Renderer:  # raytrace.rs:137-198
         h, w = p.height, p.width
         rgb = np.empty((h, w, 3), dtype=np.int32)
         out = np.empty((h, w, 3), dtype=np.float32)
-        ad = None
-        if noise_threshold is not None:
-            ad = abi.RtAdaptive()
-            ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
+        ad = _adaptive(noise_threshold, min_samples)
         cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
         stats = abi.RtStats()
         if guide is None:
@@ -263,9 +284,7 @@ class Renderer:  # raytrace.rs:137-198
                                                            C.byref(ad) if ad else None, C.byref(denoise_options_struct(**denoise_options)),
                                                            C.byref(guide_struct(**guide)), rgb.ctypes.data, out.ctypes.data, cb, None,
                                                            C.byref(stats)))
-        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
-                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
-                      "bvh_layout": stats.bvh_layout_used}
+        self.stats = _stats_dict(stats)
         return rgb, out
 
     def render_denoised_dual(self, noise_threshold=None, min_samples=16, logger=None, guide=None, **denoise_options):
@@ -282,19 +301,14 @@ class Renderer:  # raytrace.rs:137-198
         out = np.empty((h, w, 3), dtype=np.float32)
         err = np.empty((h, w, 3), dtype=np.float32)
         samples = np.empty((h, w), dtype=np.int32)
-        ad = None
-        if noise_threshold is not None:
-            ad = abi.RtAdaptive()
-            ad.noise_threshold, ad.min_samples = float(noise_threshold), int(min_samples)
+        ad = _adaptive(noise_threshold, min_samples)
         cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
         stats = abi.RtStats()
         abi.check(abi.load().rt_render_denoised_dual(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None,
                                                      C.byref(denoise_options_struct(**denoise_options)),
                                                      C.byref(guide_struct(**guide)) if guide is not None else None, rgb.ctypes.data,
                                                      out.ctypes.data, err.ctypes.data, samples.ctypes.data, cb, None, C.byref(stats)))
-        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
-                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
-                      "bvh_layout": stats.bvh_layout_used}
+        self.stats = _stats_dict(stats)
         return rgb, out, err, samples
 
     def render_features(self, feature_samples=abi.RT_GUIDE_DEFAULT_FEATURE_SAMPLES):
@@ -309,9 +323,7 @@ class Renderer:  # raytrace.rs:137-198
         stats = abi.RtStats()
         abi.check(abi.load().rt_render_features_device(self.world.handle, C.byref(self.camera.c), C.byref(p),
                                                            *[b.data_ptr() for b in bufs], None, C.byref(stats)))
-        self.stats = {"paths": stats.paths, "rays": stats.rays, "device_ms": stats.device_ms,
-                      "kernel_launches": stats.kernel_launches, "pipeline": stats.pipeline_used,
-                      "bvh_layout": stats.bvh_layout_used}
+        self.stats = _stats_dict(stats)
         return tuple(b.cpu().numpy() for b in bufs)
 
     def render(self, logger=None):
@@ -335,13 +347,7 @@ def denoise(mean, var, search_radius=abi.RT_DENOISE_DEFAULT_SEARCH_RADIUS, patch
     patch_radius f: patches of (2f + 1)^2 pixels; k > 0: strength; alpha >= 0: how much of the variance the patch distance
     cancels.  Returns a new tensor [H, W, 3], computed on the tensors' device and ordered on its current stream."""
     import torch
-    if not (isinstance(mean, torch.Tensor) and isinstance(var, torch.Tensor)):
-        raise TypeError("denoise: mean and var must be torch tensors")
-    if mean.dtype != torch.float32 or var.dtype != torch.float32 or not mean.is_cuda or var.device != mean.device:
-        raise ValueError("denoise: mean and var must be float32 CUDA tensors on one device")
-    if mean.dim() != 3 or mean.shape[2] != 3 or var.shape != mean.shape:
-        raise ValueError("denoise: mean and var must have the shape [H, W, 3]")
-    mean, var = mean.contiguous(), var.contiguous()
+    mean, var = _image_inputs("denoise", (mean, var), "mean and var", plural=True)
     out = torch.empty_like(mean)
     stream = torch.cuda.current_stream(mean.device).cuda_stream
     abi.check(abi.load().rt_denoise_device(mean.data_ptr(), var.data_ptr(), mean.shape[1], mean.shape[0],
@@ -365,14 +371,7 @@ def denoise_guided(mean, var, albedo, albedo_var, normal, normal_var, k_feature=
     tau > 0: the floor of a feature's normalisation.  options: search_radius, patch_radius, k, alpha as in `denoise`.  Returns a
     new tensor [H, W, 3], computed on the tensors' device and ordered on its current stream."""
     import torch
-    ins = (mean, var, albedo, albedo_var, normal, normal_var)
-    if not all(isinstance(t, torch.Tensor) for t in ins):
-        raise TypeError("denoise_guided: every input must be a torch tensor")
-    if any(t.dtype != torch.float32 or not t.is_cuda or t.device != mean.device for t in ins):
-        raise ValueError("denoise_guided: every input must be a float32 CUDA tensor on one device")
-    if mean.dim() != 3 or mean.shape[2] != 3 or any(t.shape != mean.shape for t in ins):
-        raise ValueError("denoise_guided: every input must have the shape [H, W, 3]")
-    ins = [t.contiguous() for t in ins]
+    ins = _image_inputs("denoise_guided", (mean, var, albedo, albedo_var, normal, normal_var))
     out = torch.empty_like(ins[0])
     stream = torch.cuda.current_stream(mean.device).cuda_stream
     abi.check(abi.load().rt_denoise_guided_device(*[t.data_ptr() for t in ins], mean.shape[1], mean.shape[0],
@@ -394,13 +393,7 @@ def denoise_cross(mean_a, var_a, mean_b, var_b, features=None, k_feature=abi.RT_
     ins = (mean_a, var_a, mean_b, var_b) + (tuple(features) if features is not None else ())
     if features is not None and len(ins) != 8:
         raise ValueError("denoise_cross: features must be (albedo, albedo_var, normal, normal_var)")
-    if not all(isinstance(t, torch.Tensor) for t in ins):
-        raise TypeError("denoise_cross: every input must be a torch tensor")
-    if any(t.dtype != torch.float32 or not t.is_cuda or t.device != mean_a.device for t in ins):
-        raise ValueError("denoise_cross: every input must be a float32 CUDA tensor on one device")
-    if mean_a.dim() != 3 or mean_a.shape[2] != 3 or any(t.shape != mean_a.shape for t in ins):
-        raise ValueError("denoise_cross: every input must have the shape [H, W, 3]")
-    ins = [t.contiguous() for t in ins]
+    ins = _image_inputs("denoise_cross", ins)
     ptrs = [t.data_ptr() for t in ins] + [None] * (8 - len(ins))
     out, err = torch.empty_like(ins[0]), torch.empty_like(ins[0])
     stream = torch.cuda.current_stream(mean_a.device).cuda_stream

@@ -336,8 +336,8 @@ int rt_render_adaptive(const RtScene* scene, const RtCamera* cam, const RtParams
 #define RT_DENOISE_MAX_PATCH_RADIUS 7
 #define RT_DENOISE_MAX_HEIGHT 1048560
 typedef struct RtDenoise {
-    double k;              /* strength, > 0: larger blurs more */
-    double alpha;          /* variance cancellation, >= 0 */
+    double k;              /* strength, > 0 with (float)(k * k) finite (k^2 at most FLT_MAX): larger blurs more */
+    double alpha;          /* variance cancellation, >= 0 with (float)alpha finite (at most FLT_MAX) */
     int32_t search_radius; /* r in [0, RT_DENOISE_MAX_SEARCH_RADIUS]; 0 returns the input */
     int32_t patch_radius;  /* f in [0, RT_DENOISE_MAX_PATCH_RADIUS] */
 } RtDenoise;
@@ -384,6 +384,9 @@ int rt_render_denoised(const RtScene* scene, const RtCamera* cam, const RtParams
 typedef struct RtGuide {
     double k_feature;        /* > 0: larger lets more across feature edges */
     double tau;              /* > 0 and finite: the floor of the feature's normalisation */
+    /* The filter computes 1 / (3 k_feature^2 max(tau, s, g^2)) in f32 with subnormals flushed to zero, so (float)(3 k_feature^2),
+     * (float)tau and their f32 product must each be at least FLT_MIN; (float)(3 k_feature^2) may be +inf (k_feature above about
+     * 1.07e19: the feature is ignored).  Smaller values are RT_ERR_INVALID. */
     int32_t feature_samples; /* >= 1; used by rt_render_denoised_guided only */
     int32_t reserved;
 } RtGuide;

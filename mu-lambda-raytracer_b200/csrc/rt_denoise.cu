@@ -31,6 +31,7 @@
 // active pixels.
 #include <cuda_runtime.h>
 
+#include <cfloat>
 #include <cmath>
 #include <type_traits>
 
@@ -306,6 +307,9 @@ int check_denoise(const RtDenoise* opt, const char* who) {
         return set_error(RT_ERR_INVALID, "%s: search_radius must lie in [0, %d] and patch_radius in [0, %d]", who, RT_DENOISE_MAX_SEARCH_RADIUS,
                          RT_DENOISE_MAX_PATCH_RADIUS);
     if (!(opt->k > 0.0) || !(opt->alpha >= 0.0)) return set_error(RT_ERR_INVALID, "%s: k must be > 0 and alpha >= 0", who);
+    // the kernels take k^2 and alpha as f32: an infinite one makes the term of a zero-variance pixel NaN, and its weight 1
+    if (!std::isfinite((float)(opt->k * opt->k)) || !std::isfinite((float)opt->alpha))
+        return set_error(RT_ERR_INVALID, "%s: k^2 and alpha must be finite in f32 (k^2 and alpha at most FLT_MAX)", who);
     return RT_OK;
 }
 
@@ -313,6 +317,12 @@ int check_guide(const RtGuide* guide, bool render, const char* who) {
     if (!guide) return set_error(RT_ERR_INVALID, "%s: null RtGuide", who);
     if (!(guide->k_feature > 0.0) || !(guide->tau > 0.0) || std::isinf(guide->tau))
         return set_error(RT_ERR_INVALID, "%s: k_feature must be > 0 and tau finite and > 0", who);
+    // guide_scale, 1 / (3 k_f^2 max(tau, s, g^2)) in f32, must be finite, else a zero feature difference gives 0 * inf = NaN and
+    // the feature weight 1.  The kernels flush subnormal f32 values to zero, so 3 k_f^2, tau and their product must be normal
+    // numbers; 3 k_f^2 may be +inf (the feature is ignored).
+    const float kf2_3 = (float)(3.0 * guide->k_feature * guide->k_feature), tau = (float)guide->tau;
+    if (!(kf2_3 >= FLT_MIN) || !(tau >= FLT_MIN) || !(kf2_3 * tau >= FLT_MIN))
+        return set_error(RT_ERR_INVALID, "%s: 3 k_feature^2, tau and 3 k_feature^2 tau must be at least FLT_MIN in f32", who);
     if (render && guide->feature_samples < 1) return set_error(RT_ERR_INVALID, "%s: feature_samples must be >= 1", who);
     return RT_OK;
 }

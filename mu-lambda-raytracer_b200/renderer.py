@@ -345,7 +345,7 @@ def denoise(mean, var, search_radius=abi.RT_DENOISE_DEFAULT_SEARCH_RADIUS, patch
     """EXTENSION: the variance-guided non-local-means filter (rt_denoise_device) of a mean image and the variance of each mean,
     both contiguous CUDA float32 tensors [H, W, 3] on one device.  search_radius r: the window of candidates [-r, r]^2;
     patch_radius f: patches of (2f + 1)^2 pixels; k > 0: strength; alpha >= 0: how much of the variance the patch distance
-    cancels.  Returns a new tensor [H, W, 3], computed on the tensors' device and ordered on its current stream."""
+    cancels.  The kernel computes in f32, so k^2 and alpha must be at most FLT_MAX (about 3.4e38).  Returns a new tensor [H, W, 3], computed on the tensors' device and ordered on its current stream."""
     import torch
     mean, var = _image_inputs("denoise", (mean, var), "mean and var", plural=True)
     out = torch.empty_like(mean)
@@ -368,7 +368,9 @@ def denoise_guided(mean, var, albedo, albedo_var, normal, normal_var, k_feature=
     """EXTENSION: the feature-guided non-local-means filter (rt_denoise_guided_device): `denoise` whose weights are also bounded by
     the first-event albedo and normal features (Renderer.render_features; the definition is in include/rt_b200.h).  All six
     inputs are contiguous CUDA float32 tensors [H, W, 3] on one device.  k_feature > 0: larger lets more across feature edges;
-    tau > 0: the floor of a feature's normalisation.  options: search_radius, patch_radius, k, alpha as in `denoise`.  Returns a
+    tau > 0: the floor of a feature's normalisation.  The kernel forms 1 / (3 k_feature^2 tau) in f32 without subnormals, so
+    3 k_feature^2, tau and their product must each be at least FLT_MIN (about 1.18e-38); 3 k_feature^2 beyond the f32 range
+    ignores the feature.  options: search_radius, patch_radius, k, alpha as in `denoise`.  Returns a
     new tensor [H, W, 3], computed on the tensors' device and ordered on its current stream."""
     import torch
     ins = _image_inputs("denoise_guided", (mean, var, albedo, albedo_var, normal, normal_var))

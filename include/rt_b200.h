@@ -157,13 +157,17 @@ typedef struct RtCamera {
  */
 enum { RT_PIPELINE_AUTO = 0, RT_PIPELINE_MEGAKERNEL = 1, RT_PIPELINE_WAVEFRONT = 2, RT_PIPELINE_WAVEFRONT_SMEM = 3 /* retired: RT_ERR_UNSUPPORTED */, RT_PIPELINE_PERSISTENT = 4 };
 
+/* the largest end, sample_begin + sample_count, of a sample range: sample indices are 32-bit signed integers */
+#define RT_MAX_SAMPLE_END 2147483647
+
 /* RenderingParams (raytrace.rs:50-55) + max_depth (main.rs:72) + device-side knobs */
 typedef struct RtParams {
     int32_t width, height;
     int32_t samples_per_pixel; /* spp of the WHOLE image (used by the tonemap divisor) */
     int32_t max_depth;
     uint64_t seed;             /* key of the Philox render streams */
-    int32_t sample_begin;      /* this call renders samples [sample_begin, sample_begin+sample_count) */
+    int32_t sample_begin;      /* this call renders samples [sample_begin, sample_begin+sample_count), which must end at or
+                                  before RT_MAX_SAMPLE_END (RT_ERR_INVALID otherwise) */
     int32_t sample_count;      /* 0 = all of samples_per_pixel */
     int32_t pipeline;          /* RT_PIPELINE_* */
     int32_t device;            /* ignored: a scene lives on the device it was created on */
@@ -276,7 +280,7 @@ int rt_accum_fixed_to_float_device(const uint64_t* d_accum_fixed, float* d_accum
  *
  * Second moments are kept beside the radiance sums as unsigned 64-bit fixed-point sums of the SQUARED samples: every
  * sample q of the accumulation (in RT_ACCUM_FIXED_ONE units) adds (min(q, 2^44))^2 >> 40, i.e. radiance^2 in units of
- * 1 / RT_MOMENT2_FIXED_ONE, exactly.  A sample above 4096 is capped in the square; the sum holds 2^16 such extremes.
+ * 1 / RT_MOMENT2_FIXED_ONE, exactly.  A sample above 4096 is capped in the square; the sum holds 2^16 - 1 such extremes.
  * Both entry points run on the persistent pipeline only (RT_ERR_UNSUPPORTED for another pipeline).
  *
  * rt_render_moments_fixed_device: rt_render_accumulate_fixed_device plus d_moment2_fixed (3*W*H uint64 on the scene's

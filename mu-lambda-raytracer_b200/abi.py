@@ -176,6 +176,7 @@ PROTOTYPES = {
 }
 
 RT_ACCUM_FIXED_ONE = 4294967296.0
+RT_MAX_SAMPLE_END = 2 ** 31 - 1  # the largest sample_begin + sample_count
 RT_MOMENT2_FIXED_ONE = 16777216.0
 
 _HERE = os.path.dirname(os.path.abspath(__file__))

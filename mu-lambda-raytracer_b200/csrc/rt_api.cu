@@ -265,6 +265,8 @@ int validate_render(const RtScene* scene, const RtCamera* cam, const RtParams* p
     if ((long long)p->width * p->height > (1ll << 31) / 3) return set_error(RT_ERR_INVALID, "render: image too large");
     if (p->samples_per_pixel <= 0 || p->max_depth < 0) return set_error(RT_ERR_INVALID, "render: samples_per_pixel must be > 0 and max_depth >= 0");
     if (p->sample_begin < 0 || p->sample_count < 0) return set_error(RT_ERR_INVALID, "render: negative sample range");
+    // sample indices are int on the host (accumulate_fixed, the launch loops) and uint32 on the device
+    if ((long long)p->sample_begin + p->sample_count > RT_MAX_SAMPLE_END) return set_error(RT_ERR_INVALID, "render: sample range ends beyond 2^31 - 1");
     if (p->pipeline < RT_PIPELINE_AUTO || p->pipeline > RT_PIPELINE_PERSISTENT) return set_error(RT_ERR_INVALID, "render: unknown pipeline");
     return RT_OK;
 }

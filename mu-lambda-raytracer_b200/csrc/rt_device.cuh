@@ -1066,7 +1066,7 @@ RTB_DEV AccumFx radiance_fixed(float x) {
 
 // EXTENSION: the square of one fixed-point sample q = radiance_fixed(x), exactly, in 2^-24 units of radiance^2
 // (RT_MOMENT2_FIXED_ONE): (min(q, 2^44))^2 >> 40.  A sample above 4096 is capped in the square, so one sample adds at
-// most 2^48 and a 64-bit sum holds 2^16 such extremes (about 2^40 ordinary ones).
+// most 2^48 and a 64-bit sum holds 2^16 - 1 such extremes (about 2^40 ordinary ones).
 RTB_DEV AccumFx moment2_fixed(AccumFx q) {
     q = q < (1ull << 44) ? q : (1ull << 44);
 #if defined(__CUDACC__) && !defined(RTB_HOST_EMULATION)

@@ -142,6 +142,8 @@ int rt_render_multi(RtScene* const* scenes, int32_t n_scenes, const RtCamera* ca
     }
     if (params->width < 2 || params->height < 2 || params->samples_per_pixel <= 0 || params->sample_begin < 0 || params->sample_count < 0)
         return rtb::set_error(RT_ERR_INVALID, "rt_render_multi: bad image size or sample range");
+    if ((long long)params->sample_begin + params->sample_count > RT_MAX_SAMPLE_END)
+        return rtb::set_error(RT_ERR_INVALID, "rt_render_multi: sample range ends beyond 2^31 - 1");
     int begin = params->sample_begin;
     int count = params->sample_count > 0 ? params->sample_count : params->samples_per_pixel - begin;
     if (count <= 0) return rtb::set_error(RT_ERR_INVALID, "render: empty sample range");

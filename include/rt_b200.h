@@ -446,6 +446,62 @@ int rt_render_denoised_dual(const RtScene* scene, const RtCamera* cam, const RtP
                             int32_t* samples, RtProgressFn cb, void* user, RtStats* stats);
 
 /*
+ * EXTENSION: per-pixel selection among three strengths of the cross filter by Stein's unbiased risk estimate (SURE), with a
+ * bias-aware error estimate that drives adaptive sampling.  In the spirit of Li, Wu & Chuang, "SURE-based optimization for
+ * adaptive sampling and reconstruction" (SIGGRAPH Asia 2012) and Rousselle, Knaus & Zwicker, "Robust Denoising using Feature
+ * and Color Information" (Pacific Graphics 2013); the form was not checked against the papers' text.
+ *
+ * Inputs: those of rt_denoise_cross_device.  Candidates j = 0, 1, 2 with strengths s = (1, ratio^2, ratio^-2), computed in f64
+ * and each rounded once to f32: s_1 = (float)(ratio * ratio), s_2 = (float)(1 / (ratio * ratio)).
+ *   Weights: with D(p, q) the patch distance of rt_denoise_device, w_j(p, q) = exp(-s_j max(0, D(p, q))); with a guide,
+ *   min(w_j, the feature weight of rt_denoise_guided_device).  w = 1 at d = 0; candidates outside the image are skipped.
+ *   j = 0 is the cross filter; j = 1 blurs less (about k / ratio), j = 2 more (about k ratio).
+ *   Filters: F_A,j takes its weights from (mu_B, v_B) and its values from mu_A, with weight sum W_A,j(p) = sum_q w_j(p, q) >= 1;
+ *   F_B,j is the same with A and B swapped.  F_A,j is a linear smoother of mu_A whose derivative in mu_A(p) is 1 / W_A,j(p).
+ *   Risk of one half, per channel (f32, every operation rounded on its own, in this order; W = 1 gives exactly v_A):
+ *     R_A,j,c(p) = (F_A,j,c(p) - mu_A,c(p))^2 + v_A,c(p) (2 / W_A,j(p) - 1)
+ *   an unbiased estimate of E[(F_A,j,c(p) - t_c(p))^2] (t the expected value) for independent pixels and an unbiased v; R_B is
+ *   the same with A and B swapped.
+ *   Risk of the output: s_hat_j,c(p) = (R_A,j,c + R_B,j,c) / 2, an estimate of an upper bound of E[(out_j - t)^2] with
+ *   out_j = (F_A,j + F_B,j) / 2, since ((a + b) / 2)^2 <= (a^2 + b^2) / 2.
+ *   Selection: S_j(p) = the mean over the (2b + 1)^2 window around p (b = smooth_radius; neighbours clamped to the image, in row
+ *   order from the bottom left) of (s_hat_j,0 + s_hat_j,1) + s_hat_j,2, the sum and the division by (2b + 1)^2 in f32 with every
+ *   operation rounded on its own; j*(p) = argmin_j S_j(p), ties to the smaller j.
+ *   Outputs: out(p) = (F_A,j* + F_B,j*) / 2 as in rt_denoise_cross_device; err_c(p) = max(0, the window mean, in the same order,
+ *   of s_hat_j*(p),c); choice(p) = j*(p).
+ *   SURE stop rule: the filtered stop rule of rt_render_denoised_dual with (out, err) in place of (out, eps).
+ * Exact reductions: ratio = 1 gives rt_denoise_cross_device's out bit for bit (colour-only and guided) and choice 0 everywhere;
+ * r = 0 gives every W = 1, out = (mu_A + mu_B) / 2 and err the window mean of (v_A + v_B) / 2; swapping A and B gives the same
+ * out, err and choice bit for bit.
+ * Caveat: with a guide, the features come from samples [0, feature_samples), which overlap half A of the first range, so the
+ * weights of F_A are not independent of A and the estimate is approximate in guided mode.
+ *
+ * RtSure: ratio >= 1, with (float)(ratio^2) finite and (float)(ratio^-2) at least FLT_MIN; smooth_radius in
+ * [0, RT_SURE_MAX_SMOOTH_RADIUS].  Other values are RT_ERR_INVALID.
+ * rt_denoise_sure_device: rt_denoise_cross_device with the selection: out and the optional err (3*W*H floats each) and choice
+ * (W*H int32); no output may overlap an input or another output.  Deterministic; asynchronous on `stream`.  It allocates
+ * 11 x 3*W*H floats of stream-ordered scratch (F and W of the three candidates in both directions, and s_hat), against
+ * 2 x 3*W*H for rt_denoise_cross_device: about 1.9 GB at 3840 x 3840.  rt_render_denoised_sure holds the same scratch.
+ * rt_render_denoised_sure: rt_render_denoised_dual with the SURE filter in place of the cross filter and the SURE stop rule in
+ * adaptive renders; error_rgb receives err and choice (optional, W*H) the final choice of every pixel.
+ */
+#define RT_SURE_DEFAULT_RATIO 1.5         /* set by the sweep of DESIGN.md section 5h */
+#define RT_SURE_DEFAULT_SMOOTH_RADIUS 5
+#define RT_SURE_MAX_SMOOTH_RADIUS 7
+typedef struct RtSure {
+    double ratio;          /* >= 1: the strengths of the candidates are 1, ratio^2 and ratio^-2 */
+    int32_t smooth_radius; /* b in [0, RT_SURE_MAX_SMOOTH_RADIUS]: the window of the selection is (2b + 1)^2 */
+    int32_t reserved;
+} RtSure;
+int rt_denoise_sure_device(const float* d_mean_a, const float* d_var_a, const float* d_mean_b, const float* d_var_b,
+                           const float* d_albedo, const float* d_albedo_var, const float* d_normal, const float* d_normal_var,
+                           int32_t width, int32_t height, const RtDenoise* opt, const RtGuide* guide, const RtSure* sure,
+                           float* d_out_rgb, float* d_err_rgb, int32_t* d_choice, int device, void* stream);
+int rt_render_denoised_sure(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* adaptive,
+                            const RtDenoise* opt, const RtGuide* guide, const RtSure* sure, int32_t* rgb, float* denoised_rgb,
+                            float* error_rgb, int32_t* samples, int32_t* choice, RtProgressFn cb, void* user, RtStats* stats);
+
+/*
  * rt_render over several GPUs of one process (the reference's row-parallel rayon loop, raytrace.rs:176-185, becomes
  * sample slices): scenes[g] is the same description created on a distinct device; device g renders every pixel for
  * the g-th slice of the sample range (rt_sample_slice), the float accumulation buffers are summed onto scenes[0]'s

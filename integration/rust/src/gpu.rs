@@ -189,6 +189,21 @@ impl Default for RtGuide {
         }
     }
 }
+/// EXTENSION: SURE selection among three strengths of the cross filter (rt_denoise_sure_device, rt_render_denoised_sure)
+#[repr(C)]
+pub struct RtSure {
+    pub ratio: f64,
+    pub smooth_radius: i32,
+    pub reserved: i32,
+}
+pub const RT_SURE_DEFAULT_RATIO: f64 = 1.5;
+pub const RT_SURE_DEFAULT_SMOOTH_RADIUS: i32 = 5;
+pub const RT_SURE_MAX_SMOOTH_RADIUS: i32 = 7;
+impl Default for RtSure {
+    fn default() -> RtSure {
+        RtSure { ratio: RT_SURE_DEFAULT_RATIO, smooth_radius: RT_SURE_DEFAULT_SMOOTH_RADIUS, reserved: 0 }
+    }
+}
 pub enum RtScene {}
 /// Called once per image row j = 0 .. total-1, in increasing order, on the calling thread (include/rt_b200.h).
 pub type RtProgressFn = Option<extern "C" fn(row: c_int, total: c_int, user: *mut c_void)>;
@@ -230,6 +245,15 @@ extern "C" {
     pub fn rt_render_denoised_dual(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive,
                                    opt: *const RtDenoise, guide: *const RtGuide, rgb: *mut i32, denoised_rgb: *mut f32, error_rgb: *mut f32,
                                    samples: *mut i32, cb: RtProgressFn, user: *mut c_void, stats: *mut RtStats) -> c_int;
+    // EXTENSION: SURE selection among three strengths of the cross filter, with a risk estimate (guide null: colour-only)
+    pub fn rt_denoise_sure_device(d_mean_a: *const f32, d_var_a: *const f32, d_mean_b: *const f32, d_var_b: *const f32, d_albedo: *const f32,
+                                  d_albedo_var: *const f32, d_normal: *const f32, d_normal_var: *const f32, width: i32, height: i32,
+                                  opt: *const RtDenoise, guide: *const RtGuide, sure: *const RtSure, d_out_rgb: *mut f32, d_err_rgb: *mut f32,
+                                  d_choice: *mut i32, device: c_int, stream: *mut c_void) -> c_int;
+    pub fn rt_render_denoised_sure(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive,
+                                   opt: *const RtDenoise, guide: *const RtGuide, sure: *const RtSure, rgb: *mut i32, denoised_rgb: *mut f32,
+                                   error_rgb: *mut f32, samples: *mut i32, choice: *mut i32, cb: RtProgressFn, user: *mut c_void,
+                                   stats: *mut RtStats) -> c_int;
     pub fn rt_world_build(name: *const c_char, seed: u64, earth_rgb: *const u8, earth_w: i32, earth_h: i32, out: *mut *mut RtSceneDesc,
                           n_draws: *mut u64) -> c_int;
     pub fn rt_scene_desc_free(desc: *mut RtSceneDesc);

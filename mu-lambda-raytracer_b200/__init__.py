@@ -8,4 +8,4 @@ package is the thin Python host layer over that ABI, mirroring the reference's o
 from . import abi  # noqa: F401
 from .renderer import (BlackBackground, Camera, GradientBackground, RecursiveRayTracer, Renderer,  # noqa: F401
                        RenderingParams, Scene, SceneDescription, SeedableRngator, World, denoise, denoise_cross,
-                       denoise_guided, load_earthmap, to_ppm, worlds)
+                       denoise_guided, denoise_sure, load_earthmap, to_ppm, worlds)

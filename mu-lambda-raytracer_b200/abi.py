@@ -110,6 +110,13 @@ class RtGuide(C.Structure):  # EXTENSION: feature-guided denoising (rt_denoise_g
 RT_GUIDE_DEFAULT_K_FEATURE, RT_GUIDE_DEFAULT_TAU, RT_GUIDE_DEFAULT_FEATURE_SAMPLES = 1.0, 1e-2, 16
 
 
+class RtSure(C.Structure):  # EXTENSION: SURE selection among three cross-filter strengths (rt_denoise_sure_device, rt_render_denoised_sure)
+    _fields_ = [("ratio", C.c_double), ("smooth_radius", C.c_int32), ("reserved", C.c_int32)]
+
+
+RT_SURE_DEFAULT_RATIO, RT_SURE_DEFAULT_SMOOTH_RADIUS, RT_SURE_MAX_SMOOTH_RADIUS = 1.5, 5, 7
+
+
 class RtWorldInfo(C.Structure):
     _fields_ = [("lookfrom", C.c_double * 3), ("lookat", C.c_double * 3), ("vfov_deg", C.c_double),
                 ("background_kind", C.c_int32), ("needs_earthmap", C.c_int32), ("uses_rng", C.c_int32)]
@@ -157,6 +164,11 @@ PROTOTYPES = {
     "rt_render_denoised_dual": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtDenoise),
                                           C.POINTER(RtGuide), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p,
                                           C.POINTER(RtStats)]),
+    "rt_denoise_sure_device": (C.c_int, [C.c_void_p] * 8 + [C.c_int32, C.c_int32, C.POINTER(RtDenoise), C.POINTER(RtGuide), C.POINTER(RtSure),
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "rt_render_denoised_sure": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtDenoise),
+                                          C.POINTER(RtGuide), C.POINTER(RtSure), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
     "rt_tonemap_fixed_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int, C.c_void_p]),
     "rt_accum_fixed_to_float_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rt_release_cached_memory": (None, []),

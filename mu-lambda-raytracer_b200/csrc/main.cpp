@@ -17,7 +17,9 @@
 // one GPU only; --stats then covers the render and the filter), --denoise_guided: the same with the feature-guided filter
 // and its default parameters (rt_render_denoised_guided; implies --denoise; --stats also covers the feature pass),
 // --denoise_dual: dual-buffer cross filtering (rt_render_denoised_dual; implies --denoise, combines with --denoise_guided,
-// and with --noise_threshold the stop rule judges the filtered value; --samples_per_pixel and --min_samples must be even).
+// and with --noise_threshold the stop rule judges the filtered value; --samples_per_pixel and --min_samples must be even),
+// --denoise_sure: per-pixel selection among three strengths of the cross filter by a risk estimate, which also drives the stop
+// rule with --noise_threshold (rt_render_denoised_sure with the library's default RtSure; implies --denoise_dual).
 // There is no CPU renderer here: without a CUDA device the program fails with the library's error.
 #include <unistd.h>
 
@@ -156,7 +158,7 @@ int main(int argc, char** argv) {
                             "aperture",     "focus_dist",  "world",             "seed",      "gpus",     "pipeline", "earthmap",
                             "noise_threshold", "min_samples"};
     std::map<std::string, std::string> opt = defaults;
-    bool randomized_rendering = false, want_stats = false, want_denoise = false, want_guided = false, want_dual = false;
+    bool randomized_rendering = false, want_stats = false, want_denoise = false, want_guided = false, want_dual = false, want_sure = false;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "--randomized_rendering" || a == "-r") {
@@ -179,8 +181,12 @@ int main(int argc, char** argv) {
             want_denoise = want_dual = true;
             continue;
         }
+        if (a == "--denoise_sure") {
+            want_denoise = want_dual = want_sure = true;
+            continue;
+        }
         if (a == "--help" || a == "-h") {
-            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n        --denoise\n        --denoise_guided\n        --denoise_dual\n\nOPTIONS:\n");
+            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n        --denoise\n        --denoise_guided\n        --denoise_dual\n        --denoise_sure\n\nOPTIONS:\n");
             for (const char* v : valued) {
                 auto d = defaults.find(v);
                 printf("        --%s <%s>%s%s%s\n", v, v, d != defaults.end() ? " [default: " : "", d != defaults.end() ? d->second.c_str() : "",
@@ -251,10 +257,11 @@ int main(int argc, char** argv) {
     const long long min_samples = parse_int(opt["min_samples"], "min_samples");
     if (noise_threshold != 0.0 && gpus > 1) usage_error("--noise_threshold (adaptive sampling) renders on one GPU: it cannot be used with --gpus above 1");
     if (want_denoise && gpus > 1)
-        usage_error(std::string(want_dual ? "--denoise_dual" : want_guided ? "--denoise_guided" : "--denoise") +
+        usage_error(std::string(want_sure ? "--denoise_sure" : want_dual ? "--denoise_dual" : want_guided ? "--denoise_guided" : "--denoise") +
                     " renders and filters on one GPU: it cannot be used with --gpus above 1");
     if (want_dual && (spp % 2 != 0 || min_samples % 2 != 0))
-        usage_error("--denoise_dual splits every range of samples into two halves: --samples_per_pixel and --min_samples must be even");
+        usage_error(std::string(want_sure ? "--denoise_sure" : "--denoise_dual") +
+                    " splits every range of samples into two halves: --samples_per_pixel and --min_samples must be even");
     static const std::map<std::string, int> pipelines = {{"auto", RT_PIPELINE_AUTO}, {"megakernel", RT_PIPELINE_MEGAKERNEL},
                                                          {"wavefront", RT_PIPELINE_WAVEFRONT},
                                                          {"persistent", RT_PIPELINE_PERSISTENT}};
@@ -318,7 +325,13 @@ int main(int argc, char** argv) {
         RtGuide gd;
         memset(&gd, 0, sizeof gd);
         gd.k_feature = RT_GUIDE_DEFAULT_K_FEATURE, gd.tau = RT_GUIDE_DEFAULT_TAU, gd.feature_samples = RT_GUIDE_DEFAULT_FEATURE_SAMPLES;
-        if (want_dual) {
+        RtSure su;
+        memset(&su, 0, sizeof su);
+        su.ratio = RT_SURE_DEFAULT_RATIO, su.smooth_radius = RT_SURE_DEFAULT_SMOOTH_RADIUS;
+        if (want_sure) {
+            rc = rt_render_denoised_sure(scenes[0], &cam, &p, noise_threshold != 0.0 ? &ad : nullptr, &dn, want_guided ? &gd : nullptr, &su, rgb.data(),
+                                         nullptr, nullptr, nullptr, nullptr, progress_cb, &prog, &st);
+        } else if (want_dual) {
             rc = rt_render_denoised_dual(scenes[0], &cam, &p, noise_threshold != 0.0 ? &ad : nullptr, &dn, want_guided ? &gd : nullptr, rgb.data(), nullptr,
                                          nullptr, nullptr, progress_cb, &prog, &st);
         } else if (want_guided) {

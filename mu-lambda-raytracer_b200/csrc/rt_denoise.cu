@@ -22,12 +22,17 @@
 // (at most 173 KB at r = 15, f = 7).  blockIdx.z picks the direction (F_A or F_B); colour-only and guided, every
 // locations-per-thread count.  dual_combine_kernel then writes out = (F_A + F_B) / 2 and the 3 x 3 error estimate.
 //
+// denoise_nlm_sure_kernel (rt_denoise_sure_device): the cross body with two more sets of accumulators, for the candidates of
+// strengths ratio^2 and ratio^-2, from the same patch distance; it writes F_j and the weight sums W_j of the three candidates in
+// both directions.  sure_risk_kernel then writes the risk estimate s_hat of every pixel, candidate and channel, and
+// sure_select_kernel picks the candidate of least windowed risk per pixel and writes out, err and the choice.
+//
 // Every filter launch goes through with_locations (the instance of the patch radius) and launch_tiles (one block per tile).
 //
 // Both renders run the round driver of rt_adaptive.cu (adaptive_rounds); a uniform render is its single round of
 // samples_per_pixel.  rt_render_denoised renders through the moments family (moments_rounds), converts the sums
 // (denoise_mean_var), filters and tonemaps.  rt_render_denoised_dual renders two halves of every range of samples in each
-// round and cross-filters the whole image; dual_eval_kernel applies the filtered stop rule (filtered_pixel_done) to the
+// round and cross-filters (or SURE-filters, rt_render_denoised_sure) the whole image; dual_eval_kernel applies the filtered stop rule (filtered_pixel_done) to the
 // active pixels.
 #include <cuda_runtime.h>
 
@@ -108,10 +113,14 @@ namespace rtb {  // kernels with stable names (profiles)
 
 // The body of all filters.  GUIDED adds the feature weight to step 3 and nothing else: the sums keep their order, so with
 // feature weights of 1 the output is the colour-only filter's bit for bit.  CROSS computes the weights from (mean, var) and
-// averages `values` (a third mu, staged as planes 6-8): with values == mean the output is the filter's bit for bit.
-template <int NE, bool GUIDED, bool CROSS = false>
+// averages `values` (a third mu, staged as planes 6-8): with values == mean the output is the filter's bit for bit.  SURE (with
+// CROSS) also accumulates the candidates j = 1, 2 of weights exp(-s_j max(0, D)) from the same D (j = 0 is the weight of CROSS,
+// computed as before): F_j goes to out + 3*W*H*j and the weight sum W_j to wsum_out + W*H*j.
+template <int NE, bool GUIDED, bool CROSS = false, bool SURE = false>
 __device__ __forceinline__ void nlm_body(const float* __restrict__ mean, const float* __restrict__ var, const float* __restrict__ values, int W, int H, int r,
-                                         int f, float k2, float alpha, float inv_norm, float* __restrict__ out, const GuideIn& gd) {
+                                         int f, float k2, float alpha, float inv_norm, float* __restrict__ out, const GuideIn& gd, float s1 = 1.0f,
+                                         float s2 = 1.0f, float* __restrict__ wsum_out = nullptr) {
+    static_assert(CROSS || !SURE, "the SURE candidates are cross filters");
     extern __shared__ float smem[];
     constexpr int V = CROSS ? 6 : 0;  // the first plane of the averaged mu
     const int R = r + f;
@@ -158,6 +167,17 @@ __device__ __forceinline__ void nlm_body(const float* __restrict__ mean, const f
 #pragma unroll
         for (int c = 0; c < 3; ++c) acc[m][c] = smem[(V + c) * plane + s];
     }
+    float xsum[SURE ? 2 : 1][2], xacc[SURE ? 2 : 1][2][3];  // the candidates j = 1, 2 (SURE)
+    if constexpr (SURE) {
+#pragma unroll
+        for (int j = 0; j < 2; ++j)
+#pragma unroll
+            for (int m = 0; m < 2; ++m) {
+                xsum[j][m] = wsum[m];
+#pragma unroll
+                for (int c = 0; c < 3; ++c) xacc[j][m][c] = acc[m][c];
+            }
+    }
     GuideAt gp[GUIDED ? 2 : 1];
     if constexpr (GUIDED) {
 #pragma unroll
@@ -201,7 +221,23 @@ __device__ __forceinline__ void nlm_body(const float* __restrict__ mean, const f
                 float D = 0.0f;
                 for (int b = 0; b < taps; ++b) D += col[b * kTileX];
                 float w = __expf(-fmaxf(D * inv_norm, 0.0f));
-                if constexpr (GUIDED) w = fminf(w, guide_weight(gd, W, gp[m], qx, qy));
+                if constexpr (SURE) {
+                    const int s = (qy - sy0) * SW + (qx - sx0);
+                    const float x = fmaxf(D * inv_norm, 0.0f);
+                    float wj[2] = {__expf(-(x * s1)), __expf(-(x * s2))};
+                    if constexpr (GUIDED) {
+                        const float gw = guide_weight(gd, W, gp[m], qx, qy);
+                        w = fminf(w, gw), wj[0] = fminf(wj[0], gw), wj[1] = fminf(wj[1], gw);
+                    }
+#pragma unroll
+                    for (int i = 0; i < 2; ++i) {
+                        xsum[i][m] += wj[i];
+#pragma unroll
+                        for (int c = 0; c < 3; ++c) xacc[i][m][c] = fmaf(wj[i], smem[(V + c) * plane + s], xacc[i][m][c]);
+                    }
+                } else if constexpr (GUIDED) {
+                    w = fminf(w, guide_weight(gd, W, gp[m], qx, qy));
+                }
                 const int s = (qy - sy0) * SW + (qx - sx0);
                 wsum[m] += w;
 #pragma unroll
@@ -216,6 +252,16 @@ __device__ __forceinline__ void nlm_body(const float* __restrict__ mean, const f
         const size_t g = 3 * ((size_t)py * W + px);
 #pragma unroll
         for (int c = 0; c < 3; ++c) out[g + c] = __fdiv_rn(acc[m][c], wsum[m]);
+        if constexpr (SURE) {
+            const size_t n_values = 3 * (size_t)W * H, p = (size_t)py * W + px;
+            wsum_out[p] = wsum[m];
+#pragma unroll
+            for (int j = 0; j < 2; ++j) {
+                wsum_out[(j + 1) * (n_values / 3) + p] = xsum[j][m];
+#pragma unroll
+                for (int c = 0; c < 3; ++c) out[(j + 1) * n_values + g + c] = __fdiv_rn(xacc[j][m][c], xsum[j][m]);
+            }
+        }
     }
 }
 
@@ -259,6 +305,55 @@ __global__ void dual_combine_kernel(const float* __restrict__ fa, const float* _
         a[k] = fa[j], b[k] = fb[j];
     }
     err[i] = dual_error(a, b);
+}
+
+// The SURE candidates j = 0, 1, 2 of the cross filter, both directions in one launch (blockIdx.z as in denoise_nlm_cross_kernel):
+// F_A,j into fa + 3*W*H*j and W_A,j into wa + W*H*j; F_B,j and W_B,j likewise into fb and wb.  s1, s2: the strengths of j = 1, 2.
+// Two blocks per SM for the colour-only instances, and for the guided ones up to 4 locations per thread (f <= 3): this holds
+// the guided instances at 128 registers (at 4 locations with a 24-byte spill) where they would need 128-154; at 5 and 6
+// locations (128-172 unbounded) they would spill 96-144 bytes, so they keep one block per SM.
+template <int NE, bool GUIDED>
+__global__ void __launch_bounds__(kThreads, !GUIDED || NE <= 4 ? 2 : 1) denoise_nlm_sure_kernel(const float* __restrict__ mean_a, const float* __restrict__ var_a,
+                                                                    const float* __restrict__ mean_b, const float* __restrict__ var_b, int W, int H, int r,
+                                                                    int f, float k2, float alpha, float inv_norm, float s1, float s2,
+                                                                    float* __restrict__ fa, float* __restrict__ fb, float* __restrict__ wa,
+                                                                    float* __restrict__ wb, GuideIn g) {
+    const bool b = blockIdx.z != 0;
+    nlm_body<NE, GUIDED, true, true>(b ? mean_a : mean_b, b ? var_a : var_b, b ? mean_b : mean_a, W, H, r, f, k2, alpha, inv_norm, b ? fb : fa, g, s1, s2,
+                                     b ? wb : wa);
+}
+
+// s_hat of every pixel, candidate and channel into risk ([H][W][9], candidate-major) from F, W, mu and v of both halves
+// (sure_risk, sure_out_risk)
+__global__ void sure_risk_kernel(const float* __restrict__ fa, const float* __restrict__ fb, const float* __restrict__ wa, const float* __restrict__ wb,
+                                 const float* __restrict__ mean_a, const float* __restrict__ var_a, const float* __restrict__ mean_b,
+                                 const float* __restrict__ var_b, int W, int H, float* __restrict__ risk) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t npix = (size_t)W * H;
+    if (i >= 9LL * (long long)npix) return;
+    const size_t p = (size_t)i / 9;
+    const int j = (int)(i % 9) / 3, c = (int)(i % 3);
+    const size_t v = 3 * p + c, fj = 3 * npix * j + v, wj = npix * j + p;
+    risk[i] = sure_out_risk(sure_risk(fa[fj], mean_a[v], var_a[v], wa[wj]), sure_risk(fb[fj], mean_b[v], var_b[v], wb[wj]));
+}
+
+// out, err (optional) and choice (optional) of every pixel: sure_select over the (2b + 1)^2 window of s_hat, then dual_out of
+// the chosen candidate's F_A and F_B
+__global__ void sure_select_kernel(const float* __restrict__ risk, const float* __restrict__ fa, const float* __restrict__ fb, int W, int H, int b,
+                                   float* __restrict__ out, float* __restrict__ err, int32_t* __restrict__ choice) {
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t npix = (size_t)W * H;
+    if (p >= (long long)npix) return;
+    const int x = (int)(p % W), y = (int)(p / W), side = 2 * b + 1;
+    float e[3];
+    const int j = sure_select(side * side, [&](int k) { return risk + 9 * ((size_t)clampi(y + k / side - b, H - 1) * W + clampi(x + k % side - b, W - 1)); }, e);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const size_t v = 3 * (size_t)p + c;
+        out[v] = dual_out(fa[3 * npix * j + v], fb[3 * npix * j + v]);
+        if (err) err[v] = e[c];
+    }
+    if (choice) choice[p] = j;
 }
 
 // the sums of 3*W*H values over `counts` (per pixel) or `n` samples each -> mu, v (denoise_mean_var)
@@ -361,7 +456,53 @@ int denoise_cross(const float* ma, const float* va, const float* mb, const float
     return RT_OK;
 }
 
+int check_sure(const RtSure* sure, const char* who) {
+    if (!sure) return set_error(RT_ERR_INVALID, "%s: null RtSure", who);
+    // the strengths ratio^2 and ratio^-2 are f32 kernel parameters: the first must be finite, the second a normal number
+    const double q = sure->ratio * sure->ratio;
+    if (!(sure->ratio >= 1.0) || !std::isfinite((float)q) || !((float)(1.0 / q) >= FLT_MIN))
+        return set_error(RT_ERR_INVALID, "%s: ratio must be >= 1 with (float)ratio^2 finite and (float)ratio^-2 at least FLT_MIN", who);
+    if (sure->smooth_radius < 0 || sure->smooth_radius > RT_SURE_MAX_SMOOTH_RADIUS)
+        return set_error(RT_ERR_INVALID, "%s: smooth_radius must lie in [0, %d]", who, RT_SURE_MAX_SMOOTH_RADIUS);
+    return RT_OK;
+}
+
+// floats of scratch of denoise_sure per value of the image (3*W*H): F_A,j and F_B,j (3 each), W_A,j and W_B,j (1 each), s_hat (3)
+constexpr size_t kSureScratchPerValue = 11;
+
+// the SURE filter of the halves A and B (arguments checked) with kSureScratchPerValue * 3*W*H floats of scratch: the three
+// candidates of the cross filter in both directions, s_hat, then out, err and choice (each of the last two optional); guide:
+// the feature-guided instances
+int denoise_sure(const float* ma, const float* va, const float* mb, const float* vb, int W, int H, const RtDenoise* opt, const GuideIn* guide,
+                 const RtSure* sure, float* scratch, float* out, float* err, int32_t* choice, cudaStream_t stream) {
+    const int r = opt->search_radius, f = opt->patch_radius;
+    const float k2 = (float)(opt->k * opt->k), alpha = (float)opt->alpha, inv_norm = (float)(1.0 / (3.0 * (2 * f + 1) * (2 * f + 1)));
+    const float s1 = (float)(sure->ratio * sure->ratio), s2 = (float)(1.0 / (sure->ratio * sure->ratio));
+    const size_t npix = (size_t)W * H, n_values = 3 * npix;
+    float *fa = scratch, *fb = fa + 3 * n_values, *wa = fb + 3 * n_values, *wb = wa + 3 * npix, *risk = wb + 3 * npix;
+    const size_t smem = smem_bytes(r, f, 9);  // as denoise_cross
+    const GuideIn g = guide ? *guide : GuideIn{};
+    cudaError_t e = with_locations(f, [&](auto ne) {
+        constexpr int NE = decltype(ne)::value;
+        if (guide)
+            return launch_tiles(denoise_nlm_sure_kernel<NE, true>, W, H, 2, smem, stream, ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, s1, s2, fa, fb, wa,
+                                wb, g);
+        return launch_tiles(denoise_nlm_sure_kernel<NE, false>, W, H, 2, smem, stream, ma, va, mb, vb, W, H, r, f, k2, alpha, inv_norm, s1, s2, fa, fb, wa, wb,
+                            g);
+    });
+    if (e != cudaSuccess) return set_error(RT_ERR_CUDA, "denoise_sure: %s", cudaGetErrorString(e));
+    sure_risk_kernel<<<(unsigned)((3 * n_values + 255) / 256), 256, 0, stream>>>(fa, fb, wa, wb, ma, va, mb, vb, W, H, risk);
+    if ((e = cudaGetLastError()) != cudaSuccess) return set_error(RT_ERR_CUDA, "denoise_sure: %s", cudaGetErrorString(e));
+    sure_select_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, stream>>>(risk, fa, fb, W, H, sure->smooth_radius, out, err, choice);
+    if ((e = cudaGetLastError()) != cudaSuccess) return set_error(RT_ERR_CUDA, "denoise_sure: %s", cudaGetErrorString(e));
+    return RT_OK;
+}
+
 bool overlaps(const float* a, const float* b, size_t n) { return a < b + n && b < a + n; }
+// the choice plane (W*H int32) against a buffer of n_values floats
+bool overlaps_choice(const int32_t* choice, const float* b, size_t n_values) {
+    return (const void*)choice < (const void*)(b + n_values) && (const void*)b < (const void*)(choice + n_values / 3);
+}
 
 GuideIn guide_in(const float* albedo, const float* albedo_var, const float* normal, const float* normal_var, const RtGuide* guide) {
     return GuideIn{albedo, albedo_var, normal, normal_var, (float)(3.0 * guide->k_feature * guide->k_feature), (float)guide->tau};
@@ -455,18 +596,19 @@ int check_dual_counts(const RtParams* params, const RtAdaptive* ad, const char* 
     return RT_OK;
 }
 
-// rt_render_denoised_dual: the rounds of adaptive_rounds (one round of samples_per_pixel for a uniform render), each rendering
-// its two half ranges, converting both halves of every pixel, cross-filtering, combining and evaluating the active pixels
-// with the filtered rule
+// rt_render_denoised_dual (sure == nullptr) and rt_render_denoised_sure: the rounds of adaptive_rounds (one round of
+// samples_per_pixel for a uniform render), each rendering its two half ranges, converting both halves of every pixel,
+// filtering (the cross filter and eps, or the SURE filter and its risk estimate) and evaluating the active pixels with the
+// filtered rule
 int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,
-                         const RtGuide* guide, int32_t* rgb, float* denoised_rgb, float* error_rgb, int32_t* samples, RtProgressFn cb, void* user,
-                         RtStats* stats) {
-    const char* who = "rt_render_denoised_dual";
+                         const RtGuide* guide, const RtSure* sure, int32_t* rgb, float* denoised_rgb, float* error_rgb, int32_t* samples,
+                         int32_t* choice, RtProgressFn cb, void* user, RtStats* stats, const char* who) {
     int rc = have_device();
     if (rc != RT_OK) return rc;
     if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
     if ((rc = check_denoise(opt, who)) != RT_OK) return rc;
     if (guide && (rc = check_guide(guide, true, who)) != RT_OK) return rc;
+    if (sure && (rc = check_sure(sure, who)) != RT_OK) return rc;
     if ((rc = check_sample_range(params, ad, who)) != RT_OK) return rc;
     if ((rc = check_dual_counts(params, ad, who)) != RT_OK) return rc;
     if ((rc = check_pipeline(params)) != RT_OK) return rc;
@@ -481,11 +623,18 @@ int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtPar
 
     DeviceBlocks b(stream);
     AccumFx *s1_a, *s2_a, *s1_b, *s2_b;                      // the sums of the halves A and B
-    float *mu_a, *v_a, *mu_b, *v_b, *f_a, *f_b, *out, *err;  // their means and variances, F_A, F_B, out and eps
+    float *mu_a, *v_a, *mu_b, *v_b, *f_a = nullptr, *f_b = nullptr, *out, *err;  // their means and variances, F_A, F_B (cross), out, eps or err
     float *albedo = nullptr, *albedo_var = nullptr, *normal = nullptr, *normal_var = nullptr;  // the features (guided)
-    int32_t *half, *d_rgb;
+    float* scratch = nullptr;                                                                  // of denoise_sure (SURE)
+    int32_t *half, *d_rgb, *d_choice = nullptr;
     for (AccumFx** p : {&s1_a, &s2_a, &s1_b, &s2_b}) CU_TRY(b.alloc(p, n_values));
-    for (float** p : {&mu_a, &v_a, &mu_b, &v_b, &f_a, &f_b, &out, &err}) CU_TRY(b.alloc(p, n_values));
+    if (sure) {
+        for (float** p : {&mu_a, &v_a, &mu_b, &v_b, &out, &err}) CU_TRY(b.alloc(p, n_values));
+        CU_TRY(b.alloc(&scratch, kSureScratchPerValue * n_values));
+        CU_TRY(b.alloc(&d_choice, npix));
+    } else {
+        for (float** p : {&mu_a, &v_a, &mu_b, &v_b, &f_a, &f_b, &out, &err}) CU_TRY(b.alloc(p, n_values));
+    }
     if (guide)
         for (float** p : {&albedo, &albedo_var, &normal, &normal_var}) CU_TRY(b.alloc(p, n_values));
     CU_TRY(b.alloc(&half, npix));
@@ -524,10 +673,14 @@ int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtPar
         CU_TRY(cudaGetLastError());
         denoise_convert_kernel<<<blocks, 256, 0, stream>>>(s1_b, s2_b, half, 0, (long long)n_values, mu_b, v_b);
         CU_TRY(cudaGetLastError());
-        if ((rc = denoise_cross(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, f_a, f_b, out, err, stream)) != RT_OK) return rc;
+        if (sure)
+            rc = denoise_sure(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, sure, scratch, out, err, d_choice, stream);
+        else
+            rc = denoise_cross(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, f_a, f_b, out, err, stream);
+        if (rc != RT_OK) return rc;
         dual_eval_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, n, n_max, threshold, out, err, r.keep);
         CU_TRY(cudaGetLastError());
-        launches += 6;
+        launches += sure ? 7 : 6;
         return RT_OK;
     };
     if ((rc = adaptive_rounds(npix, m, n_max, stream, &rows, &launches, &paths, start, round)) != RT_OK) return rc;
@@ -539,6 +692,7 @@ int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtPar
     if (denoised_rgb) CU_TRY(cudaMemcpyAsync(denoised_rgb, out, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
     if (error_rgb) CU_TRY(cudaMemcpyAsync(error_rgb, err, n_values * sizeof(float), cudaMemcpyDeviceToHost, stream));
     if (samples) CU_TRY(cudaMemcpyAsync(samples, half, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    if (choice) CU_TRY(cudaMemcpyAsync(choice, d_choice, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
     CU_TRY(cudaStreamSynchronize(stream));
     if (samples)
         for (size_t i = 0; i < npix; ++i) samples[i] *= 2;  // (the device holds the count of each half)
@@ -631,7 +785,56 @@ int rt_denoise_cross_device(const float* d_mean_a, const float* d_var_a, const f
 int rt_render_denoised_dual(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,
                             const RtGuide* guide, int32_t* rgb, float* denoised_rgb, float* error_rgb, int32_t* samples, RtProgressFn cb, void* user,
                             RtStats* stats) {
-    return render_denoised_dual(scene, cam, params, ad, opt, guide, rgb, denoised_rgb, error_rgb, samples, cb, user, stats);
+    return render_denoised_dual(scene, cam, params, ad, opt, guide, nullptr, rgb, denoised_rgb, error_rgb, samples, nullptr, cb, user, stats,
+                                "rt_render_denoised_dual");
+}
+
+int rt_denoise_sure_device(const float* d_mean_a, const float* d_var_a, const float* d_mean_b, const float* d_var_b, const float* d_albedo,
+                           const float* d_albedo_var, const float* d_normal, const float* d_normal_var, int32_t width, int32_t height, const RtDenoise* opt,
+                           const RtGuide* guide, const RtSure* sure, float* d_out_rgb, float* d_err_rgb, int32_t* d_choice, int device, void* stream_) {
+    const char* who = "rt_denoise_sure_device";
+    int rc = have_device();
+    if (rc != RT_OK) return rc;
+    const float* in[8] = {d_mean_a, d_var_a, d_mean_b, d_var_b, d_albedo, d_albedo_var, d_normal, d_normal_var};
+    for (int i = 0; i < 4; ++i)
+        if (!in[i]) return set_error(RT_ERR_INVALID, "%s: null buffer", who);
+    for (int i = 4; i < 8; ++i)
+        if (!in[i] != !guide) return set_error(RT_ERR_INVALID, "%s: the four feature buffers must be given with a guide and NULL without one", who);
+    if (!d_out_rgb) return set_error(RT_ERR_INVALID, "%s: null buffer", who);
+    if (width <= 0 || height <= 0 || height > RT_DENOISE_MAX_HEIGHT)
+        return set_error(RT_ERR_INVALID, "%s: width must be > 0 and height in [1, %d]", who, RT_DENOISE_MAX_HEIGHT);
+    if ((rc = check_denoise(opt, who)) != RT_OK) return rc;
+    if (guide && (rc = check_guide(guide, false, who)) != RT_OK) return rc;
+    if ((rc = check_sure(sure, who)) != RT_OK) return rc;
+    const size_t n_values = 3 * (size_t)width * (size_t)height;
+    for (const float* p : in)
+        if (p && (overlaps(d_out_rgb, p, n_values) || (d_err_rgb && overlaps(d_err_rgb, p, n_values)) || (d_choice && overlaps_choice(d_choice, p, n_values))))
+            return set_error(RT_ERR_INVALID, "%s: an output overlaps an input", who);
+    if ((d_err_rgb && overlaps(d_out_rgb, d_err_rgb, n_values)) || (d_choice && overlaps_choice(d_choice, d_out_rgb, n_values)) ||
+        (d_choice && d_err_rgb && overlaps_choice(d_choice, d_err_rgb, n_values)))
+        return set_error(RT_ERR_INVALID, "%s: the outputs overlap", who);
+    if (device < 0) cudaGetDevice(&device);
+    DeviceGuard g(device);
+    cudaStream_t stream = (cudaStream_t)stream_;
+    float* scratch = nullptr;  // stream-ordered so that the call stays asynchronous
+    CU_TRY(cudaMallocAsync((void**)&scratch, kSureScratchPerValue * n_values * sizeof(float), stream));
+    const GuideIn gi = guide ? guide_in(d_albedo, d_albedo_var, d_normal, d_normal_var, guide) : GuideIn{};
+    rc = denoise_sure(d_mean_a, d_var_a, d_mean_b, d_var_b, width, height, opt, guide ? &gi : nullptr, sure, scratch, d_out_rgb, d_err_rgb, d_choice, stream);
+    const cudaError_t e = cudaFreeAsync(scratch, stream);
+    if (rc != RT_OK) return rc;
+    if (e != cudaSuccess) return set_error(RT_ERR_CUDA, "%s: cudaFreeAsync: %s", who, cudaGetErrorString(e));
+    return RT_OK;
+}
+
+int rt_render_denoised_sure(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,
+                            const RtGuide* guide, const RtSure* sure, int32_t* rgb, float* denoised_rgb, float* error_rgb, int32_t* samples, int32_t* choice,
+                            RtProgressFn cb, void* user, RtStats* stats) {
+    if (!sure) {  // (render_denoised_dual takes a null RtSure for the cross filter)
+        const int rc = have_device();
+        return rc != RT_OK ? rc : set_error(RT_ERR_INVALID, "rt_render_denoised_sure: null RtSure");
+    }
+    return render_denoised_dual(scene, cam, params, ad, opt, guide, sure, rgb, denoised_rgb, error_rgb, samples, choice, cb, user, stats,
+                                "rt_render_denoised_sure");
 }
 
 int rt_render_denoised_guided(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,

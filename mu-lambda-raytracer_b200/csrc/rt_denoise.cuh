@@ -148,4 +148,56 @@ RTD_DEV bool filtered_pixel_done(uint32_t n, uint32_t n_max, const float out[3],
     return true;
 }
 
+// ---- SURE selection (rt_denoise_sure_device, rt_render_denoised_sure)
+
+// R of one half, candidate and channel from its filtered value f, its own mean mu and variance of the mean v, and its weight
+// sum w >= 1: (f - mu)^2 + v (2 / w - 1), every f32 operation rounded on its own (w = 1 and f = mu give v exactly)
+RTD_DEV float sure_risk(float f, float mu, float v, float w) {
+    const float d = RTD_FSUB(f, mu);
+    return RTD_FADD(RTD_FMUL(d, d), RTD_FMUL(v, RTD_FSUB(RTD_FDIV_RN(2.0f, w), 1.0f)));
+}
+
+// s_hat of one candidate and channel from the risks of the two halves: (R_A + R_B) / 2
+RTD_DEV float sure_out_risk(float ra, float rb) { return RTD_FMUL(RTD_FADD(ra, rb), 0.5f); }
+
+// The selection at p from s_hat at the n neighbours of its window (clamped to the image, in row order from the bottom left):
+// risk(k) points to the nine s_hat of neighbour k, candidate-major ([j][c]).  S_j = sum_k ((s_j,0 + s_j,1) + s_j,2) / n and
+// the per-channel window means, in f32 with every operation rounded on its own; returns j* = argmin S_j (ties to the smaller
+// j) and err_c = max(0, the window mean of s_hat_j*,c).
+template <class Risk>
+RTD_DEV int sure_select(int n, Risk risk, float err[3]) {
+    float S[3] = {0.0f, 0.0f, 0.0f}, E[3][3] = {{0.0f, 0.0f, 0.0f}, {0.0f, 0.0f, 0.0f}, {0.0f, 0.0f, 0.0f}};
+    for (int k = 0; k < n; ++k) {
+        const float* s = risk(k);
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+        for (int j = 0; j < 3; ++j) {
+            S[j] = RTD_FADD(S[j], RTD_FADD(RTD_FADD(s[3 * j], s[3 * j + 1]), s[3 * j + 2]));
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+            for (int c = 0; c < 3; ++c) E[j][c] = RTD_FADD(E[j][c], s[3 * j + c]);
+        }
+    }
+    const float fn = (float)n;
+    int best = 0;
+    float s_best = RTD_FDIV_RN(S[0], fn);
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int j = 1; j < 3; ++j) {
+        const float s = RTD_FDIV_RN(S[j], fn);
+        if (s < s_best) best = j, s_best = s;
+    }
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int c = 0; c < 3; ++c) {
+        const float e = RTD_FDIV_RN(best == 0 ? E[0][c] : best == 1 ? E[1][c] : E[2][c], fn);
+        err[c] = e > 0.0f ? e : 0.0f;
+    }
+    return best;
+}
+
 }  // namespace rtb

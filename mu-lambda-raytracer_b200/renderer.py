@@ -311,6 +311,32 @@ class Renderer:  # raytrace.rs:137-198
         self.stats = _stats_dict(stats)
         return rgb, out, err, samples
 
+    def render_denoised_sure(self, noise_threshold=None, min_samples=16, logger=None, guide=None, ratio=abi.RT_SURE_DEFAULT_RATIO,
+                             smooth_radius=abi.RT_SURE_DEFAULT_SMOOTH_RADIUS, **denoise_options):
+        """EXTENSION: render_denoised_dual with the SURE filter (rt_render_denoised_sure; the definition is in include/rt_b200.h):
+        per pixel, the cross filter of strength 1, ratio^2 or ratio^-2 with the least risk estimate over a (2 smooth_radius + 1)^2
+        window, and that risk estimate (bias included) as the error, which also drives the stop rule of an adaptive render.
+        Arguments as in render_denoised_dual; ratio >= 1, smooth_radius in [0, RT_SURE_MAX_SMOOTH_RADIUS].  Returns (rgb int32
+        [H,W,3]; denoised float32 [H,W,3]; err float32 [H,W,3], the risk estimate of each channel; samples int32 [H,W]; choice int32
+        [H,W], the candidate each pixel took: 0 strength 1, 1 blurs less, 2 blurs more), row 0 at the bottom."""
+        p = self._params()
+        h, w = p.height, p.width
+        rgb = np.empty((h, w, 3), dtype=np.int32)
+        out = np.empty((h, w, 3), dtype=np.float32)
+        err = np.empty((h, w, 3), dtype=np.float32)
+        samples = np.empty((h, w), dtype=np.int32)
+        choice = np.empty((h, w), dtype=np.int32)
+        ad = _adaptive(noise_threshold, min_samples)
+        cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
+        stats = abi.RtStats()
+        abi.check(abi.load().rt_render_denoised_sure(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None,
+                                                     C.byref(denoise_options_struct(**denoise_options)),
+                                                     C.byref(guide_struct(**guide)) if guide is not None else None,
+                                                     C.byref(sure_struct(ratio, smooth_radius)), rgb.ctypes.data, out.ctypes.data, err.ctypes.data,
+                                                     samples.ctypes.data, choice.ctypes.data, cb, None, C.byref(stats)))
+        self.stats = _stats_dict(stats)
+        return rgb, out, err, samples, choice
+
     def render_features(self, feature_samples=abi.RT_GUIDE_DEFAULT_FEATURE_SAMPLES):
         """EXTENSION: the first-event features of samples [0, feature_samples) of every pixel (rt_render_features_device; the
         definition is in include/rt_b200.h).  Returns numpy float32 (albedo, albedo_var, normal, normal_var), each [H, W, 3]
@@ -403,6 +429,37 @@ def denoise_cross(mean_a, var_a, mean_b, var_b, features=None, k_feature=abi.RT_
     abi.check(abi.load().rt_denoise_cross_device(*ptrs, mean_a.shape[1], mean_a.shape[0], C.byref(denoise_options_struct(**options)), guide,
                                                  out.data_ptr(), err.data_ptr(), mean_a.device.index, stream))
     return out, err
+
+
+def sure_struct(ratio=abi.RT_SURE_DEFAULT_RATIO, smooth_radius=abi.RT_SURE_DEFAULT_SMOOTH_RADIUS):
+    """the RtSure of the arguments (defaults: the header's RT_SURE_DEFAULT_*)"""
+    sure = abi.RtSure()
+    sure.ratio, sure.smooth_radius = float(ratio), int(smooth_radius)
+    return sure
+
+
+def denoise_sure(mean_a, var_a, mean_b, var_b, features=None, k_feature=abi.RT_GUIDE_DEFAULT_K_FEATURE, tau=abi.RT_GUIDE_DEFAULT_TAU,
+                 ratio=abi.RT_SURE_DEFAULT_RATIO, smooth_radius=abi.RT_SURE_DEFAULT_SMOOTH_RADIUS, **options):
+    """EXTENSION: the SURE filter (rt_denoise_sure_device; the definition is in include/rt_b200.h) of two independent halves of a
+    render: the cross filter of `denoise_cross` at the strengths 1, ratio^2 and ratio^-2, and per pixel the one whose Stein's
+    unbiased risk estimate, averaged over a (2 smooth_radius + 1)^2 window, is least.  Inputs, features, k_feature, tau and options
+    as in `denoise_cross`; ratio >= 1, smooth_radius in [0, RT_SURE_MAX_SMOOTH_RADIUS].  Returns new tensors (out [H, W, 3], err
+    [H, W, 3], the risk estimate of out, bias included; choice int32 [H, W], 0 strength 1, 1 blurs less, 2 blurs more), computed on
+    the tensors' device and ordered on its current stream."""
+    import torch
+    ins = (mean_a, var_a, mean_b, var_b) + (tuple(features) if features is not None else ())
+    if features is not None and len(ins) != 8:
+        raise ValueError("denoise_sure: features must be (albedo, albedo_var, normal, normal_var)")
+    ins = _image_inputs("denoise_sure", ins)
+    ptrs = [t.data_ptr() for t in ins] + [None] * (8 - len(ins))
+    out, err = torch.empty_like(ins[0]), torch.empty_like(ins[0])
+    choice = torch.empty(ins[0].shape[:2], dtype=torch.int32, device=ins[0].device)
+    stream = torch.cuda.current_stream(mean_a.device).cuda_stream
+    guide = C.byref(guide_struct(k_feature, tau)) if features is not None else None
+    abi.check(abi.load().rt_denoise_sure_device(*ptrs, mean_a.shape[1], mean_a.shape[0], C.byref(denoise_options_struct(**options)), guide,
+                                                C.byref(sure_struct(ratio, smooth_radius)), out.data_ptr(), err.data_ptr(), choice.data_ptr(),
+                                                mean_a.device.index, stream))
+    return out, err, choice
 
 
 def to_ppm(rgb):

@@ -502,6 +502,56 @@ int rt_render_denoised_sure(const RtScene* scene, const RtCamera* cam, const RtP
                             float* error_rgb, int32_t* samples, int32_t* choice, RtProgressFn cb, void* user, RtStats* stats);
 
 /*
+ * EXTENSION: a neighbourhood prior on each pixel's per-sample variance (empirical Bayes), for the stop rules of
+ * rt_render_adaptive and rt_render_denoised_sure.  A pixel whose first samples found no light has mu = 0 and s^2 = 0, so its
+ * error estimate is 0 and it stops in round 0; the prior lends it the variance of the pixels around it.
+ *
+ * Term of a pixel q holding n_q >= 2 samples, per channel c, with mu as in the rule of rt_render_adaptive (f64, every
+ * operation rounded on its own): N_q,c = max(0, S2 2^-24 - n_q mu^2) (that is (n_q - 1) s^2) and d_q = n_q - 1.  Stored as
+ * four f64 per pixel (N_r, N_g, N_b, d).
+ * Pool of p: the window is the (2b + 1)^2 square around p WITHOUT p; neighbours outside the image are skipped (not clamped).
+ * sum N_c and sum d in f64 over the window in row order from the bottom left (dy = -b..b, then dx = -b..b), every addition
+ * rounded on its own; P_c(p) = sum N_c / sum d (f64).  Every pixel takes part with its current sums: a stopped pixel keeps
+ * feeding its neighbours.
+ * Posterior per-sample variance, n0 = prior_samples (f64, every operation rounded on its own, in this form):
+ *   s~^2_c = (N_p,c + n0 P_c) / ((n_p - 1) + n0)
+ * and, when the window holds no pixel (a 1 x 1 image), s~^2_c = N_p,c / (n_p - 1) = s^2 (no prior).  n0 = 0 gives s^2 bit for
+ * bit.  There is no prior on the mean.
+ * Prior rule: the rule of rt_render_adaptive with s~^2 in place of s^2 (mu, the slope, the saturation test and the cap as
+ * there).  A mu = 0 pixel with noisy neighbours keeps sampling; one whose neighbours are all noise-free still stops.
+ * SURE prior rule (rt_render_denoised_sure_prior): the same pool and posterior per half, from the half's own sums with
+ * n = n_p / 2 and the neighbours' sums of the same half: v~_A = s~^2_A / (n_p / 2) (f64, rounded once to f32), v~_B likewise.
+ * s_hat'_j,c = (R'_A + R'_B) / 2 with R' the risk of rt_render_denoised_sure with v~ in place of v; err'_c(p) = max(0, the
+ * window mean of s_hat'_j*(p),c) with j*(p), the window and the order of the selection.  The stop rule is the filtered rule on
+ * (out, err').  out and the choice are those of rt_render_denoised_sure: the prior only decides which pixels go on.
+ * Exact reductions: n0 = 0 at any radius gives rt_render_adaptive and rt_render_denoised_sure bit for bit (every output, the
+ * counts and stats->paths); so does a window without pixels at any n0 in the per-pixel functions (an image of one pixel,
+ * which the renders, at least 2 x 2, do not take).
+ *
+ * RtPrior: prior_samples finite and >= 0, radius in [1, RT_PRIOR_MAX_RADIUS]; other values, or a NULL RtPrior, are
+ * RT_ERR_INVALID.
+ * rt_render_adaptive_prior: rt_render_adaptive with the prior rule.  It holds 4 f64 of terms per pixel of scratch.
+ * rt_render_denoised_sure_prior: rt_render_denoised_sure with the SURE prior rule; `adaptive` must be given (a uniform render
+ * has no stop rule).  error_rgb receives err'.  It holds 8 f64 of terms and 6 f32 of v~ per pixel beside the scratch of
+ * rt_render_denoised_sure.
+ */
+#define RT_PRIOR_DEFAULT_SAMPLES 16.0 /* set by the sweep of DESIGN.md section 5i */
+#define RT_PRIOR_DEFAULT_RADIUS 7
+#define RT_PRIOR_MAX_RADIUS 7
+typedef struct RtPrior {
+    double prior_samples; /* n0 >= 0 and finite: the weight of the neighbourhood's variance, in samples */
+    int32_t radius;       /* b in [1, RT_PRIOR_MAX_RADIUS]: the window is (2b + 1)^2 without the pixel */
+    int32_t reserved;
+} RtPrior;
+int rt_render_adaptive_prior(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* adaptive,
+                             const RtPrior* prior, int32_t* rgb, int32_t* samples, uint64_t* accum_fixed, uint64_t* moment2_fixed,
+                             RtProgressFn cb, void* user, RtStats* stats);
+int rt_render_denoised_sure_prior(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* adaptive,
+                                  const RtDenoise* opt, const RtGuide* guide, const RtSure* sure, const RtPrior* prior, int32_t* rgb,
+                                  float* denoised_rgb, float* error_rgb, int32_t* samples, int32_t* choice, RtProgressFn cb,
+                                  void* user, RtStats* stats);
+
+/*
  * rt_render over several GPUs of one process (the reference's row-parallel rayon loop, raytrace.rs:176-185, becomes
  * sample slices): scenes[g] is the same description created on a distinct device; device g renders every pixel for
  * the g-th slice of the sample range (rt_sample_slice), the float accumulation buffers are summed onto scenes[0]'s

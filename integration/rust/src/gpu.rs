@@ -204,6 +204,21 @@ impl Default for RtSure {
         RtSure { ratio: RT_SURE_DEFAULT_RATIO, smooth_radius: RT_SURE_DEFAULT_SMOOTH_RADIUS, reserved: 0 }
     }
 }
+/// EXTENSION: neighbourhood variance prior of the stop rules (rt_render_adaptive_prior, rt_render_denoised_sure_prior)
+#[repr(C)]
+pub struct RtPrior {
+    pub prior_samples: f64,
+    pub radius: i32,
+    pub reserved: i32,
+}
+pub const RT_PRIOR_DEFAULT_SAMPLES: f64 = 16.0;
+pub const RT_PRIOR_DEFAULT_RADIUS: i32 = 7;
+pub const RT_PRIOR_MAX_RADIUS: i32 = 7;
+impl Default for RtPrior {
+    fn default() -> RtPrior {
+        RtPrior { prior_samples: RT_PRIOR_DEFAULT_SAMPLES, radius: RT_PRIOR_DEFAULT_RADIUS, reserved: 0 }
+    }
+}
 pub enum RtScene {}
 /// Called once per image row j = 0 .. total-1, in increasing order, on the calling thread (include/rt_b200.h).
 pub type RtProgressFn = Option<extern "C" fn(row: c_int, total: c_int, user: *mut c_void)>;
@@ -254,6 +269,14 @@ extern "C" {
                                    opt: *const RtDenoise, guide: *const RtGuide, sure: *const RtSure, rgb: *mut i32, denoised_rgb: *mut f32,
                                    error_rgb: *mut f32, samples: *mut i32, choice: *mut i32, cb: RtProgressFn, user: *mut c_void,
                                    stats: *mut RtStats) -> c_int;
+    // EXTENSION: the stop rules with a neighbourhood variance prior (adaptive must be non-null)
+    pub fn rt_render_adaptive_prior(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive,
+                                    prior: *const RtPrior, rgb: *mut i32, samples: *mut i32, accum_fixed: *mut u64, moment2_fixed: *mut u64,
+                                    cb: RtProgressFn, user: *mut c_void, stats: *mut RtStats) -> c_int;
+    pub fn rt_render_denoised_sure_prior(scene: *const RtScene, cam: *const RtCamera, params: *const RtParams, adaptive: *const RtAdaptive,
+                                         opt: *const RtDenoise, guide: *const RtGuide, sure: *const RtSure, prior: *const RtPrior, rgb: *mut i32,
+                                         denoised_rgb: *mut f32, error_rgb: *mut f32, samples: *mut i32, choice: *mut i32, cb: RtProgressFn,
+                                         user: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_world_build(name: *const c_char, seed: u64, earth_rgb: *const u8, earth_w: i32, earth_h: i32, out: *mut *mut RtSceneDesc,
                           n_draws: *mut u64) -> c_int;
     pub fn rt_scene_desc_free(desc: *mut RtSceneDesc);

@@ -117,6 +117,13 @@ class RtSure(C.Structure):  # EXTENSION: SURE selection among three cross-filter
 RT_SURE_DEFAULT_RATIO, RT_SURE_DEFAULT_SMOOTH_RADIUS, RT_SURE_MAX_SMOOTH_RADIUS = 1.5, 5, 7
 
 
+class RtPrior(C.Structure):  # EXTENSION: neighbourhood variance prior of the stop rules (rt_render_adaptive_prior, rt_render_denoised_sure_prior)
+    _fields_ = [("prior_samples", C.c_double), ("radius", C.c_int32), ("reserved", C.c_int32)]
+
+
+RT_PRIOR_DEFAULT_SAMPLES, RT_PRIOR_DEFAULT_RADIUS, RT_PRIOR_MAX_RADIUS = 16.0, 7, 7
+
+
 class RtWorldInfo(C.Structure):
     _fields_ = [("lookfrom", C.c_double * 3), ("lookat", C.c_double * 3), ("vfov_deg", C.c_double),
                 ("background_kind", C.c_int32), ("needs_earthmap", C.c_int32), ("uses_rng", C.c_int32)]
@@ -169,6 +176,11 @@ PROTOTYPES = {
     "rt_render_denoised_sure": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtDenoise),
                                           C.POINTER(RtGuide), C.POINTER(RtSure), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                           RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
+    "rt_render_adaptive_prior": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtPrior),
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
+    "rt_render_denoised_sure_prior": (C.c_int, [C.c_void_p, C.POINTER(RtCamera), C.POINTER(RtParams), C.POINTER(RtAdaptive), C.POINTER(RtDenoise),
+                                                C.POINTER(RtGuide), C.POINTER(RtSure), C.POINTER(RtPrior), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                C.c_void_p, C.c_void_p, RtProgressFn, C.c_void_p, C.POINTER(RtStats)]),
     "rt_tonemap_fixed_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int, C.c_void_p]),
     "rt_accum_fixed_to_float_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rt_release_cached_memory": (None, []),

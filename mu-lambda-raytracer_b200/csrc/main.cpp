@@ -19,7 +19,10 @@
 // --denoise_dual: dual-buffer cross filtering (rt_render_denoised_dual; implies --denoise, combines with --denoise_guided,
 // and with --noise_threshold the stop rule judges the filtered value; --samples_per_pixel and --min_samples must be even),
 // --denoise_sure: per-pixel selection among three strengths of the cross filter by a risk estimate, which also drives the stop
-// rule with --noise_threshold (rt_render_denoised_sure with the library's default RtSure; implies --denoise_dual).
+// rule with --noise_threshold (rt_render_denoised_sure with the library's default RtSure; implies --denoise_dual),
+// --noise_prior: the stop rule of --noise_threshold with each pixel's variance pooled with its neighbourhood's (the library's
+// default RtPrior: rt_render_adaptive_prior, or rt_render_denoised_sure_prior with --denoise_sure; needs --noise_threshold, and
+// of the filters only --denoise_sure).
 // There is no CPU renderer here: without a CUDA device the program fails with the library's error.
 #include <unistd.h>
 
@@ -158,7 +161,8 @@ int main(int argc, char** argv) {
                             "aperture",     "focus_dist",  "world",             "seed",      "gpus",     "pipeline", "earthmap",
                             "noise_threshold", "min_samples"};
     std::map<std::string, std::string> opt = defaults;
-    bool randomized_rendering = false, want_stats = false, want_denoise = false, want_guided = false, want_dual = false, want_sure = false;
+    bool randomized_rendering = false, want_stats = false, want_denoise = false, want_guided = false, want_dual = false, want_sure = false,
+         want_prior = false;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "--randomized_rendering" || a == "-r") {
@@ -185,8 +189,12 @@ int main(int argc, char** argv) {
             want_denoise = want_dual = want_sure = true;
             continue;
         }
+        if (a == "--noise_prior") {
+            want_prior = true;
+            continue;
+        }
         if (a == "--help" || a == "-h") {
-            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n        --denoise\n        --denoise_guided\n        --denoise_dual\n        --denoise_sure\n\nOPTIONS:\n");
+            printf("mulambda raytracer 0.1 (B200)\n\nUSAGE:\n    rt_main [FLAGS] [OPTIONS]\n\nFLAGS:\n    -r, --randomized_rendering\n        --stats\n        --denoise\n        --denoise_guided\n        --denoise_dual\n        --denoise_sure\n        --noise_prior\n\nOPTIONS:\n");
             for (const char* v : valued) {
                 auto d = defaults.find(v);
                 printf("        --%s <%s>%s%s%s\n", v, v, d != defaults.end() ? " [default: " : "", d != defaults.end() ? d->second.c_str() : "",
@@ -255,6 +263,11 @@ int main(int argc, char** argv) {
     long long gpus = parse_int(opt["gpus"], "gpus");
     const double noise_threshold = parse_f64(opt["noise_threshold"], "noise_threshold");
     const long long min_samples = parse_int(opt["min_samples"], "min_samples");
+    if (want_prior && noise_threshold == 0.0) usage_error("--noise_prior is a prior of the stop rule: it needs --noise_threshold");
+    if (want_prior && gpus > 1) usage_error("--noise_prior (adaptive sampling) renders on one GPU: it cannot be used with --gpus above 1");
+    if (want_prior && want_denoise && !want_sure)
+        usage_error(std::string("--noise_prior drives the plain or the SURE stop rule: it cannot be used with ") +
+                    (want_dual ? "--denoise_dual" : want_guided ? "--denoise_guided" : "--denoise") + " unless --denoise_sure is also given");
     if (noise_threshold != 0.0 && gpus > 1) usage_error("--noise_threshold (adaptive sampling) renders on one GPU: it cannot be used with --gpus above 1");
     if (want_denoise && gpus > 1)
         usage_error(std::string(want_sure ? "--denoise_sure" : want_dual ? "--denoise_dual" : want_guided ? "--denoise_guided" : "--denoise") +
@@ -317,6 +330,9 @@ int main(int argc, char** argv) {
     RtAdaptive ad;
     memset(&ad, 0, sizeof ad);
     ad.noise_threshold = noise_threshold, ad.min_samples = (int32_t)min_samples;
+    RtPrior pr;
+    memset(&pr, 0, sizeof pr);
+    pr.prior_samples = RT_PRIOR_DEFAULT_SAMPLES, pr.radius = RT_PRIOR_DEFAULT_RADIUS;
     if (want_denoise) {
         RtDenoise dn;
         memset(&dn, 0, sizeof dn);
@@ -328,7 +344,10 @@ int main(int argc, char** argv) {
         RtSure su;
         memset(&su, 0, sizeof su);
         su.ratio = RT_SURE_DEFAULT_RATIO, su.smooth_radius = RT_SURE_DEFAULT_SMOOTH_RADIUS;
-        if (want_sure) {
+        if (want_sure && want_prior) {
+            rc = rt_render_denoised_sure_prior(scenes[0], &cam, &p, &ad, &dn, want_guided ? &gd : nullptr, &su, &pr, rgb.data(), nullptr, nullptr,
+                                               nullptr, nullptr, progress_cb, &prog, &st);
+        } else if (want_sure) {
             rc = rt_render_denoised_sure(scenes[0], &cam, &p, noise_threshold != 0.0 ? &ad : nullptr, &dn, want_guided ? &gd : nullptr, &su, rgb.data(),
                                          nullptr, nullptr, nullptr, nullptr, progress_cb, &prog, &st);
         } else if (want_dual) {
@@ -340,6 +359,8 @@ int main(int argc, char** argv) {
         } else {
             rc = rt_render_denoised(scenes[0], &cam, &p, noise_threshold != 0.0 ? &ad : nullptr, &dn, rgb.data(), nullptr, progress_cb, &prog, &st);
         }
+    } else if (want_prior) {
+        rc = rt_render_adaptive_prior(scenes[0], &cam, &p, &ad, &pr, rgb.data(), nullptr, nullptr, nullptr, progress_cb, &prog, &st);
     } else if (noise_threshold != 0.0) {
         rc = rt_render_adaptive(scenes[0], &cam, &p, &ad, rgb.data(), nullptr, nullptr, nullptr, progress_cb, &prog, &st);
     } else {

@@ -11,6 +11,10 @@
 // stop rule (rt_device.cuh: adaptive_pixel_done) to the active pixels, cub::DeviceSelect::Flagged (stable) compacts the
 // rest into the next list, and one host synchronisation reads its length.  adaptive_rounds runs this loop for every render
 // of the family (rt_denoise.cu too) with the work of one round passed in; a uniform render is its single round, m = max.
+//
+// With a neighbourhood prior (rt_render_adaptive_prior; the definition is in include/rt_b200.h) the evaluation is two
+// launches: prior_term_kernel updates the terms (N, d) of the pixels rendered this round, then prior_eval_kernel pools the
+// window of every active pixel (one thread per pixel, the terms read through L1) and applies the prior rule.
 #include <cuda_runtime.h>
 
 #include <cub/device/device_select.cuh>
@@ -19,6 +23,7 @@
 #include <cmath>
 #include <cstring>
 
+#include "rt_denoise.cuh"
 #include "rt_device.cuh"
 #include "scene_internal.h"
 
@@ -42,6 +47,13 @@ int check_sample_range(const RtParams* params, const RtAdaptive* ad, const char*
     return RT_OK;
 }
 
+int check_prior(const RtPrior* prior, const char* who) {
+    if (!prior) return set_error(RT_ERR_INVALID, "%s: null RtPrior", who);
+    if (!std::isfinite(prior->prior_samples) || !(prior->prior_samples >= 0.0)) return set_error(RT_ERR_INVALID, "%s: prior_samples must be finite and >= 0", who);
+    if (prior->radius < 1 || prior->radius > RT_PRIOR_MAX_RADIUS) return set_error(RT_ERR_INVALID, "%s: radius must lie in [1, %d]", who, RT_PRIOR_MAX_RADIUS);
+    return RT_OK;
+}
+
 }  // namespace rtb
 
 namespace {
@@ -60,6 +72,35 @@ __global__ void adaptive_eval_kernel(const uint32_t* __restrict__ list, unsigned
     const uint32_t p = list[i];
     samples[p] = (int32_t)n;
     keep[i] = adaptive_pixel_done(n, n_max, accum + 3 * (size_t)p, moment2 + 3 * (size_t)p, threshold) ? 0 : 1;
+}
+
+// the active pixels after a round that brought each of them to n samples: their count and their terms (prior_term)
+__global__ void prior_term_kernel(const uint32_t* __restrict__ list, unsigned int n_list, uint32_t n, const AccumFx* __restrict__ accum,
+                                  const AccumFx* __restrict__ moment2, int32_t* __restrict__ samples, double* __restrict__ terms) {
+    const unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_list) return;
+    const uint32_t p = list[i];
+    samples[p] = (int32_t)n;
+    prior_term((const uint64_t*)accum + 3 * (size_t)p, (const uint64_t*)moment2 + 3 * (size_t)p, n, terms + 4 * (size_t)p);
+}
+
+// the active pixels after prior_term_kernel: the pool of each one's window, its posterior variances and the prior rule
+__global__ void prior_eval_kernel(const uint32_t* __restrict__ list, unsigned int n_list, uint32_t n, uint32_t n_max, double threshold, int W,
+                                  int H, int b, double n0, const AccumFx* __restrict__ accum, const double* __restrict__ terms,
+                                  unsigned char* __restrict__ keep) {
+    const unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_list) return;
+    if (n >= n_max) {
+        keep[i] = 0;
+        return;
+    }
+    const uint32_t p = list[i];
+    double sum[4], var[3];
+    prior_pool((int)(p % (uint32_t)W), (int)(p / (uint32_t)W), W, H, b, [&](size_t q) { return terms + 4 * q; }, sum);
+    const double* t = terms + 4 * (size_t)p;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) var[c] = prior_posterior(t[c], t[3], sum[c], sum[3], n0);
+    keep[i] = prior_pixel_done(n, n_max, (const uint64_t*)accum + 3 * (size_t)p, var, threshold) ? 0 : 1;
 }
 
 // every pixel tonemapped with its own sample count (to_rgb of raytrace.rs:59-68)
@@ -115,12 +156,15 @@ int adaptive_rounds(unsigned int npix, uint32_t m, uint32_t n_max, cudaStream_t 
 }
 
 int moments_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, uint32_t m, double threshold, AccumFx* d_accum, AccumFx* d_moment2,
-                   int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths) {
+                   int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths, const RtPrior* prior) {
     const unsigned int npix = (unsigned int)params->width * (unsigned int)params->height;
     const size_t n_values = 3 * (size_t)npix;
     const uint32_t n_max = (uint32_t)params->samples_per_pixel;
     DCamera dc;
     make_camera(*cam, dc);
+    DeviceBlocks b(stream);
+    double* terms = nullptr;  // (prior) N_r, N_g, N_b, d of every pixel
+    if (prior) CU_TRY(b.alloc(&terms, 4 * (size_t)npix));
     const auto start = [&]() -> int {
         CU_TRY(cudaMemsetAsync(scene->d_rays, 0, sizeof(unsigned long long), stream));
         CU_TRY(cudaEventRecord(scene->ev0, stream));
@@ -131,8 +175,18 @@ int moments_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, 
     const auto round = [&](const AdaptiveRound& r) -> int {
         const int rc = launch_persist_moments(scene, dc, params, (int)r.first, (int)r.count, d_accum, d_moment2, r.render_list, r.n_list, stream, launches);
         if (rc != RT_OK) return rc;
-        adaptive_eval_kernel<<<(r.n_list + 255) / 256, 256, 0, stream>>>(r.list, r.n_list, r.first + r.count, n_max, threshold, d_accum, d_moment2,
-                                                                         d_samples, r.keep);
+        const unsigned list_blocks = (r.n_list + 255) / 256;
+        if (prior) {
+            prior_term_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, r.first + r.count, d_accum, d_moment2, d_samples, terms);
+            CU_TRY(cudaGetLastError());
+            prior_eval_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, r.first + r.count, n_max, threshold, params->width, params->height,
+                                                               prior->radius, prior->prior_samples, d_accum, terms, r.keep);
+            CU_TRY(cudaGetLastError());
+            *launches += 2;
+            return RT_OK;
+        }
+        adaptive_eval_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, r.first + r.count, n_max, threshold, d_accum, d_moment2,
+                                                              d_samples, r.keep);
         CU_TRY(cudaGetLastError());
         *launches += 1;
         return RT_OK;
@@ -186,13 +240,19 @@ int rt_render_moments_fixed_device(const RtScene* scene_, const RtCamera* cam, c
     return render_stats(scene, params, (uint64_t)npix * count, launches, stats);
 }
 
-int rt_render_adaptive(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, int32_t* rgb, int32_t* samples,
-                       uint64_t* accum_fixed, uint64_t* moment2_fixed, RtProgressFn cb, void* user, RtStats* stats) {
+}  // extern "C"
+
+namespace {
+
+// rt_render_adaptive (prior == nullptr) and rt_render_adaptive_prior
+int render_adaptive(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtPrior* prior, int32_t* rgb,
+                    int32_t* samples, uint64_t* accum_fixed, uint64_t* moment2_fixed, RtProgressFn cb, void* user, RtStats* stats, const char* who) {
     int rc = have_device();
     if (rc != RT_OK) return rc;
     if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
-    if (!ad) return set_error(RT_ERR_INVALID, "rt_render_adaptive: null RtAdaptive");
-    if ((rc = check_sample_range(params, ad, "rt_render_adaptive")) != RT_OK) return rc;
+    if (!ad) return set_error(RT_ERR_INVALID, "%s: null RtAdaptive", who);
+    if (prior && (rc = check_prior(prior, who)) != RT_OK) return rc;
+    if ((rc = check_sample_range(params, ad, who)) != RT_OK) return rc;
     if ((rc = check_pipeline(params)) != RT_OK) return rc;
     RtScene* scene = const_cast<RtScene*>(scene_);
     DeviceGuard g(scene->device);
@@ -211,7 +271,8 @@ int rt_render_adaptive(const RtScene* scene_, const RtCamera* cam, const RtParam
     rtb::RowProgress rows{cb, user, params->height, 0};
     int launches = 0;
     uint64_t paths = 0;
-    rc = moments_rounds(scene, cam, params, (uint32_t)ad->min_samples, ad->noise_threshold, d_accum, d_moment2, d_samples, stream, &rows, &launches, &paths);
+    rc = moments_rounds(scene, cam, params, (uint32_t)ad->min_samples, ad->noise_threshold, d_accum, d_moment2, d_samples, stream, &rows, &launches, &paths,
+                        prior);
     if (rc != RT_OK) return rc;
     tonemap_counts_kernel<<<(unsigned)((n_values + 255) / 256), 256, 0, stream>>>(d_accum, d_samples, d_rgb, (int)n_values);
     CU_TRY(cudaGetLastError());
@@ -224,6 +285,24 @@ int rt_render_adaptive(const RtScene* scene_, const RtCamera* cam, const RtParam
     CU_TRY(cudaStreamSynchronize(stream));
     rtb::row_progress(1, 1, &rows);  // whatever rows the rounds did not cover
     return render_stats(scene, params, paths, launches, stats);
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_render_adaptive(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, int32_t* rgb, int32_t* samples,
+                       uint64_t* accum_fixed, uint64_t* moment2_fixed, RtProgressFn cb, void* user, RtStats* stats) {
+    return render_adaptive(scene, cam, params, ad, nullptr, rgb, samples, accum_fixed, moment2_fixed, cb, user, stats, "rt_render_adaptive");
+}
+
+int rt_render_adaptive_prior(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtPrior* prior, int32_t* rgb,
+                             int32_t* samples, uint64_t* accum_fixed, uint64_t* moment2_fixed, RtProgressFn cb, void* user, RtStats* stats) {
+    if (!prior) {  // (render_adaptive takes a null RtPrior for the rule without a prior)
+        const int rc = have_device();
+        return rc != RT_OK ? rc : set_error(RT_ERR_INVALID, "rt_render_adaptive_prior: null RtPrior");
+    }
+    return render_adaptive(scene, cam, params, ad, prior, rgb, samples, accum_fixed, moment2_fixed, cb, user, stats, "rt_render_adaptive_prior");
 }
 
 }  // extern "C"

@@ -27,6 +27,11 @@
 // both directions.  sure_risk_kernel then writes the risk estimate s_hat of every pixel, candidate and channel, and
 // sure_select_kernel picks the candidate of least windowed risk per pixel and writes out, err and the choice.
 //
+// rt_render_denoised_sure_prior (the definition of the prior is in include/rt_b200.h): after the SURE filter of a round,
+// prior_term_dual_kernel updates the terms of both halves of the pixels rendered this round, prior_var_kernel writes v~ of both
+// halves for every pixel, sure_risk_kernel runs again with v~ in place of v (s_hat' over s_hat in the scratch) and
+// prior_sure_err_kernel writes err', the window mean of s_hat' at the stored choice, for the filtered rule.
+//
 // Every filter launch goes through with_locations (the instance of the patch radius) and launch_tiles (one block per tile).
 //
 // Both renders run the round driver of rt_adaptive.cu (adaptive_rounds); a uniform render is its single round of
@@ -369,6 +374,48 @@ __global__ void denoise_tonemap_kernel(const float* __restrict__ x, int32_t* __r
     if (i < n_values) rgb[i] = to_rgb_f64((double)x[i]);
 }
 
+// the terms (prior_term, 4 f64 per pixel) of both halves of the active pixels after a dual round that brought each half to n samples
+__global__ void prior_term_dual_kernel(const uint32_t* __restrict__ list, unsigned int n_list, uint32_t n, const AccumFx* __restrict__ s1_a,
+                                       const AccumFx* __restrict__ s2_a, const AccumFx* __restrict__ s1_b, const AccumFx* __restrict__ s2_b,
+                                       double* __restrict__ terms_a, double* __restrict__ terms_b) {
+    const unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_list) return;
+    const size_t p = list[i];
+    prior_term((const uint64_t*)s1_a + 3 * p, (const uint64_t*)s2_a + 3 * p, n, terms_a + 4 * p);
+    prior_term((const uint64_t*)s1_b + 3 * p, (const uint64_t*)s2_b + 3 * p, n, terms_b + 4 * p);
+}
+
+// v~ of both halves of every pixel (3*W*H f32 each): the pool of the (2b + 1)^2 window of the half's terms, the posterior with
+// n0 pseudo-samples and the division by the half's count
+__global__ void prior_var_kernel(const double* __restrict__ terms_a, const double* __restrict__ terms_b, const int32_t* __restrict__ half, int W, int H,
+                                 int b, double n0, float* __restrict__ vt_a, float* __restrict__ vt_b) {
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= (long long)W * H) return;
+    const int x = (int)(p % W), y = (int)(p / W);
+    const uint32_t n = (uint32_t)half[p];
+    double sum[4];
+    prior_pool(x, y, W, H, b, [&](size_t q) { return terms_a + 4 * q; }, sum);
+    const double* t = terms_a + 4 * p;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) vt_a[3 * p + c] = prior_var_of_mean(prior_posterior(t[c], t[3], sum[c], sum[3], n0), n);
+    prior_pool(x, y, W, H, b, [&](size_t q) { return terms_b + 4 * q; }, sum);
+    t = terms_b + 4 * p;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) vt_b[3 * p + c] = prior_var_of_mean(prior_posterior(t[c], t[3], sum[c], sum[3], n0), n);
+}
+
+// err' of every pixel: the window mean of s_hat' (risk, [H][W][9]) at the pixel's choice over the (2b + 1)^2 window of the
+// selection (clamped, sure_window_err)
+__global__ void prior_sure_err_kernel(const float* __restrict__ risk, const int32_t* __restrict__ choice, int W, int H, int b, float* __restrict__ err) {
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= (long long)W * H) return;
+    const int x = (int)(p % W), y = (int)(p / W), side = 2 * b + 1;
+    float e[3];
+    sure_window_err(side * side, choice[p], [&](int k) { return risk + 9 * ((size_t)clampi(y + k / side - b, H - 1) * W + clampi(x + k % side - b, W - 1)); }, e);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) err[3 * p + c] = e[c];
+}
+
 }  // namespace rtb
 
 namespace {
@@ -599,16 +646,17 @@ int check_dual_counts(const RtParams* params, const RtAdaptive* ad, const char* 
 // rt_render_denoised_dual (sure == nullptr) and rt_render_denoised_sure: the rounds of adaptive_rounds (one round of
 // samples_per_pixel for a uniform render), each rendering its two half ranges, converting both halves of every pixel,
 // filtering (the cross filter and eps, or the SURE filter and its risk estimate) and evaluating the active pixels with the
-// filtered rule
+// filtered rule.  prior (rt_render_denoised_sure_prior, with sure and ad): err' of the SURE prior rule in place of err.
 int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,
                          const RtGuide* guide, const RtSure* sure, int32_t* rgb, float* denoised_rgb, float* error_rgb, int32_t* samples,
-                         int32_t* choice, RtProgressFn cb, void* user, RtStats* stats, const char* who) {
+                         int32_t* choice, RtProgressFn cb, void* user, RtStats* stats, const char* who, const RtPrior* prior = nullptr) {
     int rc = have_device();
     if (rc != RT_OK) return rc;
     if ((rc = validate_render(scene_, cam, params)) != RT_OK) return rc;
     if ((rc = check_denoise(opt, who)) != RT_OK) return rc;
     if (guide && (rc = check_guide(guide, true, who)) != RT_OK) return rc;
     if (sure && (rc = check_sure(sure, who)) != RT_OK) return rc;
+    if (prior && (rc = check_prior(prior, who)) != RT_OK) return rc;
     if ((rc = check_sample_range(params, ad, who)) != RT_OK) return rc;
     if ((rc = check_dual_counts(params, ad, who)) != RT_OK) return rc;
     if ((rc = check_pipeline(params)) != RT_OK) return rc;
@@ -637,6 +685,12 @@ int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtPar
     }
     if (guide)
         for (float** p : {&albedo, &albedo_var, &normal, &normal_var}) CU_TRY(b.alloc(p, n_values));
+    double *terms_a = nullptr, *terms_b = nullptr;  // (prior) N_r, N_g, N_b, d of every pixel, per half
+    float *vt_a = nullptr, *vt_b = nullptr;          // (prior) v~ of both halves
+    if (prior) {
+        for (double** p : {&terms_a, &terms_b}) CU_TRY(b.alloc(p, 4 * (size_t)npix));
+        for (float** p : {&vt_a, &vt_b}) CU_TRY(b.alloc(p, n_values));
+    }
     CU_TRY(b.alloc(&half, npix));
     CU_TRY(b.alloc(&d_rgb, n_values));
     const GuideIn gi = guide ? guide_in(albedo, albedo_var, normal, normal_var, guide) : GuideIn{};
@@ -674,10 +728,24 @@ int render_denoised_dual(const RtScene* scene_, const RtCamera* cam, const RtPar
         denoise_convert_kernel<<<blocks, 256, 0, stream>>>(s1_b, s2_b, half, 0, (long long)n_values, mu_b, v_b);
         CU_TRY(cudaGetLastError());
         if (sure)
-            rc = denoise_sure(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, sure, scratch, out, err, d_choice, stream);
+            rc = denoise_sure(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, sure, scratch, out, prior ? nullptr : err, d_choice, stream);
         else
             rc = denoise_cross(mu_a, v_a, mu_b, v_b, W, H, opt, guide ? &gi : nullptr, f_a, f_b, out, err, stream);
         if (rc != RT_OK) return rc;
+        if (prior) {  // err' from s_hat' at the choice just made; F and W stay in the scratch (the layout of denoise_sure)
+            const float *fa = scratch, *fb = fa + 3 * n_values, *wa = fb + 3 * n_values, *wb = wa + 3 * (size_t)npix;
+            float* risk = scratch + 8 * n_values;
+            const unsigned pix_blocks = (npix + 255) / 256;
+            prior_term_dual_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, n / 2, s1_a, s2_a, s1_b, s2_b, terms_a, terms_b);
+            CU_TRY(cudaGetLastError());
+            prior_var_kernel<<<pix_blocks, 256, 0, stream>>>(terms_a, terms_b, half, W, H, prior->radius, prior->prior_samples, vt_a, vt_b);
+            CU_TRY(cudaGetLastError());
+            sure_risk_kernel<<<(unsigned)((3 * n_values + 255) / 256), 256, 0, stream>>>(fa, fb, wa, wb, mu_a, vt_a, mu_b, vt_b, W, H, risk);
+            CU_TRY(cudaGetLastError());
+            prior_sure_err_kernel<<<pix_blocks, 256, 0, stream>>>(risk, d_choice, W, H, sure->smooth_radius, err);
+            CU_TRY(cudaGetLastError());
+            launches += 4;
+        }
         dual_eval_kernel<<<list_blocks, 256, 0, stream>>>(r.list, r.n_list, n, n_max, threshold, out, err, r.keep);
         CU_TRY(cudaGetLastError());
         launches += sure ? 7 : 6;
@@ -835,6 +903,19 @@ int rt_render_denoised_sure(const RtScene* scene, const RtCamera* cam, const RtP
     }
     return render_denoised_dual(scene, cam, params, ad, opt, guide, sure, rgb, denoised_rgb, error_rgb, samples, choice, cb, user, stats,
                                 "rt_render_denoised_sure");
+}
+
+int rt_render_denoised_sure_prior(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,
+                                  const RtGuide* guide, const RtSure* sure, const RtPrior* prior, int32_t* rgb, float* denoised_rgb, float* error_rgb,
+                                  int32_t* samples, int32_t* choice, RtProgressFn cb, void* user, RtStats* stats) {
+    const char* who = "rt_render_denoised_sure_prior";
+    const int rc = have_device();
+    if (rc != RT_OK) return rc;
+    // (render_denoised_dual takes a null RtSure for the cross filter and a null RtPrior for the rule without a prior)
+    if (!sure) return set_error(RT_ERR_INVALID, "%s: null RtSure", who);
+    if (!prior) return set_error(RT_ERR_INVALID, "%s: null RtPrior", who);
+    if (!ad) return set_error(RT_ERR_INVALID, "%s: null RtAdaptive (a uniform render has no stop rule)", who);
+    return render_denoised_dual(scene, cam, params, ad, opt, guide, sure, rgb, denoised_rgb, error_rgb, samples, choice, cb, user, stats, who, prior);
 }
 
 int rt_render_denoised_guided(const RtScene* scene, const RtCamera* cam, const RtParams* params, const RtAdaptive* ad, const RtDenoise* opt,

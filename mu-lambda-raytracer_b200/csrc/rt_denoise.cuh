@@ -200,4 +200,87 @@ RTD_DEV int sure_select(int n, Risk risk, float err[3]) {
     return best;
 }
 
+// err_c = max(0, the window mean of s_hat_j,c) for a given j, in the order and f32 arithmetic of sure_select (with j = j* it is
+// sure_select's err bit for bit)
+template <class Risk>
+RTD_DEV void sure_window_err(int n, int j, Risk risk, float err[3]) {
+    float E[3] = {0.0f, 0.0f, 0.0f};
+    for (int k = 0; k < n; ++k) {
+        const float* s = risk(k) + 3 * j;
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+        for (int c = 0; c < 3; ++c) E[c] = RTD_FADD(E[c], s[c]);
+    }
+    const float fn = (float)n;
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int c = 0; c < 3; ++c) {
+        const float e = RTD_FDIV_RN(E[c], fn);
+        err[c] = e > 0.0f ? e : 0.0f;
+    }
+}
+
+// ---- neighbourhood variance prior (rt_render_adaptive_prior, rt_render_denoised_sure_prior)
+
+// The term of one pixel holding n >= 2 samples: N_c = max(0, S2 2^-24 - n mu^2) per channel, with mu as in adaptive_pixel_done,
+// and d = n - 1, into t[4] = (N_r, N_g, N_b, d).  f64, every operation rounded on its own.
+RTD_DEV void prior_term(const uint64_t s1[3], const uint64_t s2[3], uint32_t n, double t[4]) {
+    const double dn = (double)n;
+    for (int c = 0; c < 3; ++c) {
+        const double mu = RTD_DDIV(RTD_DMUL((double)s1[c], 2.3283064365386963e-10), dn);
+        const double m2 = RTD_DMUL((double)s2[c], 5.9604644775390625e-08);
+        const double x = RTD_DSUB(m2, RTD_DMUL(dn, RTD_DMUL(mu, mu)));
+        t[c] = x > 0.0 ? x : 0.0;
+    }
+    t[3] = RTD_DSUB(dn, 1.0);
+}
+
+// The pool of pixel (x, y) of a W x H image: sums of the terms of the (2b + 1)^2 window without (x, y), neighbours outside the
+// image skipped, in row order from the bottom left; term(q) points to the four f64 of pixel q.  sum[4] = (sum N_c, sum d).
+template <class Term>
+RTD_DEV void prior_pool(int x, int y, int W, int H, int b, Term term, double sum[4]) {
+    sum[0] = sum[1] = sum[2] = sum[3] = 0.0;
+    for (int dy = -b; dy <= b; ++dy) {
+        const int qy = y + dy;
+        if (qy < 0 || qy >= H) continue;
+        for (int dx = -b; dx <= b; ++dx) {
+            const int qx = x + dx;
+            if (qx < 0 || qx >= W || (dx | dy) == 0) continue;
+            const double* t = term((size_t)qy * W + qx);
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+            for (int k = 0; k < 4; ++k) sum[k] = RTD_DADD(sum[k], t[k]);
+        }
+    }
+}
+
+// The posterior per-sample variance of one channel from the pixel's term (N, d) and its pool (sum_n, sum_d) with n0 pseudo-samples:
+// (N + n0 P) / (d + n0), P = sum_n / sum_d; N / d (s^2, no prior) when the window holds no pixel
+RTD_DEV double prior_posterior(double N, double d, double sum_n, double sum_d, double n0) {
+    if (sum_d == 0.0) return RTD_DDIV(N, d);
+    const double P = RTD_DDIV(sum_n, sum_d);
+    return RTD_DDIV(RTD_DADD(N, RTD_DMUL(n0, P)), RTD_DADD(d, n0));
+}
+
+// The prior rule for a pixel that holds n of at most n_max samples: the rule of adaptive_pixel_done with the posterior per-sample
+// variances var[3] in place of s^2
+RTD_DEV bool prior_pixel_done(uint32_t n, uint32_t n_max, const uint64_t s1[3], const double var[3], double threshold) {
+    if (n >= n_max) return true;
+    const double dn = (double)n;
+    for (int c = 0; c < 3; ++c) {
+        const double mu = RTD_DDIV(RTD_DMUL((double)s1[c], 2.3283064365386963e-10), dn);
+        const double se = RTD_DSQRT(RTD_DDIV(var[c], dn));
+        const double e = RTD_DDIV(se, RTD_DMUL(2.0, RTD_DSQRT(mu > 1.52587890625e-05 ? mu : 1.52587890625e-05)));
+        if (!(e <= threshold || RTD_DSUB(mu, RTD_DMUL(3.0, se)) >= 1.0)) return false;
+    }
+    return true;
+}
+
+// v~ of one channel of a half holding n >= 2 samples from its posterior per-sample variance: s~^2 / n, rounded once to f32
+// (with s~^2 = s^2 it is denoise_mean_var's v bit for bit)
+RTD_DEV float prior_var_of_mean(double var, uint32_t n) { return RTD_F32(RTD_DDIV(var, (double)n)); }
+
 }  // namespace rtb

@@ -121,6 +121,8 @@ class DeviceBlocks {
 // sample_count 0), then with an RtAdaptive its min_samples and noise_threshold
 int check_pipeline(const RtParams* p);
 int check_sample_range(const RtParams* params, const RtAdaptive* ad, const char* who);
+// rt_adaptive.cu: RT_ERR_INVALID unless prior is non-null with prior_samples finite and >= 0 and radius in [1, RT_PRIOR_MAX_RADIUS]
+int check_prior(const RtPrior* prior, const char* who);
 // one round of adaptive_rounds: samples [first, first + count) of the n_list active pixels
 struct AdaptiveRound {
     uint32_t first, count;
@@ -138,9 +140,10 @@ int adaptive_rounds(unsigned int npix, uint32_t m, uint32_t n_max, cudaStream_t 
                     const std::function<int()>& start, const std::function<int(const AdaptiveRound&)>& round);
 // the rounds of rt_render_adaptive (uniform: m = n_max): zeroes d_accum / d_moment2 (3*W*H), renders every round through the
 // moments family and applies the stop rule (adaptive_pixel_done) with `threshold`; leaves each pixel's sums and its count
-// (d_samples, W*H) on the device.  Timing starts at scene->ev0, recorded before the first launch.
+// (d_samples, W*H) on the device.  Timing starts at scene->ev0, recorded before the first launch.  prior (checked): the prior
+// rule of rt_render_adaptive_prior in place of adaptive_pixel_done, with 4*W*H f64 of terms allocated before the timing starts.
 int moments_rounds(RtScene* scene, const RtCamera* cam, const RtParams* params, uint32_t m, double threshold, AccumFx* d_accum, AccumFx* d_moment2,
-                   int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths);
+                   int32_t* d_samples, cudaStream_t stream, RowProgress* rows, int* launches, uint64_t* paths, const RtPrior* prior = nullptr);
 // fills *stats (if non-null) of a persistent-pipeline render timed from scene->ev0 to scene->ev1 (both recorded)
 int render_stats(const RtScene* scene, const RtParams* params, uint64_t paths, int launches, RtStats* stats);
 // the schedule of the rounds: the new samples of the round after every active pixel holds n_done (0 before round 0) of at

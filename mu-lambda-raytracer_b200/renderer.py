@@ -240,12 +240,14 @@ class Renderer:  # raytrace.rs:137-198
         self.stats = _stats_dict(stats)
         return rgb, accum
 
-    def render_adaptive(self, noise_threshold, min_samples=16, logger=None):
+    def render_adaptive(self, noise_threshold, min_samples=16, logger=None, prior=None):
         """EXTENSION: noise-threshold adaptive sampling (rt_render_adaptive).  Every pixel gets samples until the standard
         error of its tonemapped value is at most `noise_threshold` in every channel (or the channel saturates), at least
         `min_samples` and at most parameters.samples_per_pixel.  Returns (rgb int32 [H,W,3], samples int32 [H,W],
         accum_fixed uint64 [H,W,3], moment2_fixed uint64 [H,W,3]) with row 0 at the bottom; the sums are in
-        1 / RT_ACCUM_FIXED_ONE and 1 / RT_MOMENT2_FIXED_ONE units.  logger(j, H) as in render_arrays, paced by rounds."""
+        1 / RT_ACCUM_FIXED_ONE and 1 / RT_MOMENT2_FIXED_ONE units.  logger(j, H) as in render_arrays, paced by rounds.
+        prior: None, or a dict of radius and prior_samples (each optional; defaults RT_PRIOR_DEFAULT_*): the stop rule then
+        uses each pixel's variance pooled with its neighbourhood's (rt_render_adaptive_prior, see `prior_struct`)."""
         p = self._params()
         h, w = p.height, p.width
         rgb = np.empty((h, w, 3), dtype=np.int32)
@@ -255,9 +257,14 @@ class Renderer:  # raytrace.rs:137-198
         ad = _adaptive(noise_threshold, min_samples)
         cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
         stats = abi.RtStats()
-        abi.check(abi.load().rt_render_adaptive(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad),
-                                                rgb.ctypes.data, samples.ctypes.data, accum.ctypes.data, moment2.ctypes.data,
-                                                cb, None, C.byref(stats)))
+        if prior is None:
+            abi.check(abi.load().rt_render_adaptive(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad),
+                                                    rgb.ctypes.data, samples.ctypes.data, accum.ctypes.data, moment2.ctypes.data,
+                                                    cb, None, C.byref(stats)))
+        else:
+            abi.check(abi.load().rt_render_adaptive_prior(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad),
+                                                          C.byref(prior_struct(**prior)), rgb.ctypes.data, samples.ctypes.data,
+                                                          accum.ctypes.data, moment2.ctypes.data, cb, None, C.byref(stats)))
         self.stats = _stats_dict(stats)
         return rgb, samples, accum, moment2
 
@@ -312,13 +319,16 @@ class Renderer:  # raytrace.rs:137-198
         return rgb, out, err, samples
 
     def render_denoised_sure(self, noise_threshold=None, min_samples=16, logger=None, guide=None, ratio=abi.RT_SURE_DEFAULT_RATIO,
-                             smooth_radius=abi.RT_SURE_DEFAULT_SMOOTH_RADIUS, **denoise_options):
+                             smooth_radius=abi.RT_SURE_DEFAULT_SMOOTH_RADIUS, prior=None, **denoise_options):
         """EXTENSION: render_denoised_dual with the SURE filter (rt_render_denoised_sure; the definition is in include/rt_b200.h):
         per pixel, the cross filter of strength 1, ratio^2 or ratio^-2 with the least risk estimate over a (2 smooth_radius + 1)^2
         window, and that risk estimate (bias included) as the error, which also drives the stop rule of an adaptive render.
         Arguments as in render_denoised_dual; ratio >= 1, smooth_radius in [0, RT_SURE_MAX_SMOOTH_RADIUS].  Returns (rgb int32
         [H,W,3]; denoised float32 [H,W,3]; err float32 [H,W,3], the risk estimate of each channel; samples int32 [H,W]; choice int32
-        [H,W], the candidate each pixel took: 0 strength 1, 1 blurs less, 2 blurs more), row 0 at the bottom."""
+        [H,W], the candidate each pixel took: 0 strength 1, 1 blurs less, 2 blurs more), row 0 at the bottom.
+        prior: None, or a dict of radius and prior_samples (each optional) for an adaptive render: the stop rule then judges
+        err', the risk estimate with each half's variance pooled with its neighbourhood's (rt_render_denoised_sure_prior), and
+        err returns err'; out and choice are unchanged."""
         p = self._params()
         h, w = p.height, p.width
         rgb = np.empty((h, w, 3), dtype=np.int32)
@@ -329,11 +339,15 @@ class Renderer:  # raytrace.rs:137-198
         ad = _adaptive(noise_threshold, min_samples)
         cb = abi.RtProgressFn(lambda row, total, user: logger(row, total)) if logger else abi.RtProgressFn()
         stats = abi.RtStats()
-        abi.check(abi.load().rt_render_denoised_sure(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None,
-                                                     C.byref(denoise_options_struct(**denoise_options)),
-                                                     C.byref(guide_struct(**guide)) if guide is not None else None,
-                                                     C.byref(sure_struct(ratio, smooth_radius)), rgb.ctypes.data, out.ctypes.data, err.ctypes.data,
-                                                     samples.ctypes.data, choice.ctypes.data, cb, None, C.byref(stats)))
+        args = (C.byref(denoise_options_struct(**denoise_options)), C.byref(guide_struct(**guide)) if guide is not None else None,
+                C.byref(sure_struct(ratio, smooth_radius)))
+        bufs = (rgb.ctypes.data, out.ctypes.data, err.ctypes.data, samples.ctypes.data, choice.ctypes.data, cb, None, C.byref(stats))
+        lib = abi.load()
+        if prior is None:
+            abi.check(lib.rt_render_denoised_sure(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None, *args, *bufs))
+        else:
+            abi.check(lib.rt_render_denoised_sure_prior(self.world.handle, C.byref(self.camera.c), C.byref(p), C.byref(ad) if ad else None, *args,
+                                                        C.byref(prior_struct(**prior)), *bufs))
         self.stats = _stats_dict(stats)
         return rgb, out, err, samples, choice
 
@@ -436,6 +450,13 @@ def sure_struct(ratio=abi.RT_SURE_DEFAULT_RATIO, smooth_radius=abi.RT_SURE_DEFAU
     sure = abi.RtSure()
     sure.ratio, sure.smooth_radius = float(ratio), int(smooth_radius)
     return sure
+
+
+def prior_struct(radius=abi.RT_PRIOR_DEFAULT_RADIUS, prior_samples=abi.RT_PRIOR_DEFAULT_SAMPLES):
+    """the RtPrior of the arguments (defaults: the header's RT_PRIOR_DEFAULT_*)"""
+    prior = abi.RtPrior()
+    prior.prior_samples, prior.radius = float(prior_samples), int(radius)
+    return prior
 
 
 def denoise_sure(mean_a, var_a, mean_b, var_b, features=None, k_feature=abi.RT_GUIDE_DEFAULT_K_FEATURE, tau=abi.RT_GUIDE_DEFAULT_TAU,
